@@ -2,6 +2,7 @@
 """Headline benchmark: GAT layer fwd+bwd edges/sec (BASELINE.json metric) + achieved HBM GB/s vs peak.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload powerlaw_200m|elliptic|skew] [--impl reference]
+                  [--dump-outputs DIR]
 
 A "step" is one GATConv layer (H=8, C=64, concat=False, bias, dropout off) forward + backward over the
 whole synthetic graph, CSR cached (its build is reported separately).  Default workload at N=1 is the
@@ -11,6 +12,11 @@ configuration the metric's target is quoted on: the 200M-edge / 20M-node power-l
 `--impl reference` times the reference formulation (PyG GATConv semantics: the CPU oracle port, since
 torch_geometric is not installable in this image) on the host cores, on a bounded sample of the same
 workload family.
+
+`--dump-outputs DIR` writes what the timed path computed in its last timed step -- the layer output and the parameter
+gradients (the TGN workload: loss, logits and parameter gradients) -- as DIR/<name>.npy in float32 / float64.  Of an
+output with more than 65,536 rows, a fixed seeded sample of 65,536 rows is written.  The inputs are seeded, so two builds
+run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -49,6 +55,33 @@ def env_int(name, default):
         return int(os.environ.get(name, default))
     except ValueError:
         return default
+
+
+DUMP_ROWS = 65_536
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def output_sample(arrays: dict) -> dict:
+    """Host float32 / float64 copies of ``arrays``; of a tensor with more than DUMP_ROWS rows, the rows of a fixed
+    seeded sample (the same rows in every run)."""
+    res = {}
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.dim() and t.size(0) > DUMP_ROWS:
+            rows = torch.randperm(t.size(0), generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+            t = t[rows.to(t.device)]
+        res[name] = (t if t.dtype == torch.float64 else t.float()).cpu().numpy()
+    return res
+
+
+def write_outputs(path: str, arrays: dict) -> None:
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
 
 
 def make_edges(workload: str, N: int, E: int, device):
@@ -155,7 +188,7 @@ def cpu_reference_step_fn(workload, threads):
             p.grad = None
         out = conv(x, ei)
         out.backward(d_out)
-        return float(out[0, 0].detach())
+        return {"out": out.detach(), **{f"grad.{n}": p.grad for n, p in conv.named_parameters()}}
 
     return step, kind, what + ", one GATConv fwd+bwd", E, same
 
@@ -180,7 +213,7 @@ def cpu_tgn_step_fn(threads):
         m = y != -1
         loss = crit(lg[m].squeeze(1), y[m].float())
         loss.backward()
-        return float(loss.detach())
+        return {"loss": loss.detach(), "logits": lg.detach(), **{f"grad.{n}": p.grad for n, p in ref.named_parameters()}}
 
     return step, "port", (f"Elliptic-shaped graph N={N} E={E} K={K}, 49 time steps, at FULL size: one TemporalGNN (2 layers) "
                           f"training step, fwd + loss + bwd"), E, True
@@ -200,8 +233,10 @@ def run_reference_arm(args):
         step()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step()
+        outputs = step()
     dt = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, output_sample(outputs))
     val = E / dt
     line = {
         "impl": "reference", "metric": "tgn_train_step_edges_per_sec" if args.workload == "tgn_snapshots" else METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -365,9 +400,11 @@ def run_gpu_arm(args):
     all_marks = []
     t_host = time.perf_counter()
     e_start.record()
-    for _ in range(args.steps):
-        _, _, marks = step(True)
+    for i in range(args.steps):
+        out, grads, marks = step(True)
         all_marks.append(marks)
+        if i + 1 < args.steps:
+            del out, grads          # only the last step's outputs are kept
     e_end.record()
     host_enqueue_ms = (time.perf_counter() - t_host) * 1e3 / args.steps       # host time to ENQUEUE one step
     torch.cuda.synchronize()
@@ -375,6 +412,9 @@ def run_gpu_arm(args):
         dist.barrier()
         torch.cuda.synchronize()
     launches = int(L.gnnfd_launch_count())
+    out_names = ("out", "dW", "datt_src", "datt_dst", "dbias")
+    dumped = output_sample(dict(zip(out_names, (out,) + tuple(grads)))) if args.dump_outputs and rank == 0 else None
+    del out, grads
     total_ms = e_start.elapsed_time(e_end)
     if world > 1:
         t = torch.tensor([total_ms], device=dev)
@@ -421,6 +461,8 @@ def run_gpu_arm(args):
                 g_ms = float(t.item())
             ms_per_step = g_ms / args.steps
             graph_note = "timed as K replays of ONE CUDA graph of the whole step (kernels + collectives)"
+            if dumped is not None:
+                dumped = output_sample(dict(zip(out_names, (g_out,) + tuple(g_grads))))
             del cg, g_out, g_grads
         except Exception as ex:     # capture not possible on this stack: keep the eager number
             graph_note = f"CUDA graph capture failed ({type(ex).__name__}: {str(ex)[:120]}); eager timing reported"
@@ -549,6 +591,8 @@ def run_gpu_arm(args):
             "timing": {"eager_ms_per_step": eager_ms_per_step, "host_enqueue_ms_per_step": host_enqueue_ms, "cuda_graph": graph_note},
             "selfcheck": selfcheck,
         }
+        if dumped is not None:
+            write_outputs(args.dump_outputs, dumped)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -648,10 +692,19 @@ def run_tgn_snapshots(args):
         logits, _ = model(xl, el)
         loss, stats = fused.masked_bce_with_logits(logits, yl, 50.0)
         (loss * w_lab).backward()                        # global mean over labelled nodes = share-weighted local means
+        flat = None
         if world > 1:
             flat = torch.cat([p.grad.reshape(-1) for p in params])
             dist.all_reduce(flat)
-        return loss
+        return loss, logits, flat
+
+    def outputs(res):
+        """What a caller of the step receives: the loss, the logits and the (all-reduced) parameter gradients."""
+        loss, logits, flat = res
+        names = [n for n, _ in model.named_parameters()]
+        grads = [p.grad for p in params] if flat is None else flat.split([p.numel() for p in params])
+        return output_sample({"loss": loss, "logits": logits,
+                              **{f"grad.{n}": g.view(p.shape) for n, g, p in zip(names, grads, params)}})
 
     for _ in range(max(args.warmup, 3)):
         step()
@@ -664,11 +717,13 @@ def run_tgn_snapshots(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step()
+        res = step()
     e1.record()
     torch.cuda.synchronize()
     launches = int(L.gnnfd_launch_count())
     eager_ms = e0.elapsed_time(e1) / args.steps
+    dumped = outputs(res) if args.dump_outputs and rank == 0 else None
+    del res
     ms, graph_note = eager_ms, None
     if args.graph != "off":
         try:
@@ -678,7 +733,7 @@ def run_tgn_snapshots(args):
                 step()
                 cs.synchronize()
                 with torch.cuda.graph(cg, stream=cs):
-                    step()
+                    g_res = step()
             torch.cuda.current_stream().wait_stream(cs)
             for _ in range(3):
                 cg.replay()
@@ -692,7 +747,9 @@ def run_tgn_snapshots(args):
             torch.cuda.synchronize()
             ms = e0.elapsed_time(e1) / args.steps
             graph_note = "timed as K replays of ONE CUDA graph of the whole training step (launch-bound at this size)"
-            del cg          # a live graph with captured collectives stalls destroy_process_group
+            if dumped is not None:
+                dumped = outputs(g_res)
+            del cg, g_res   # a live graph with captured collectives stalls destroy_process_group
             torch.cuda.synchronize()
         except Exception as ex:
             graph_note = f"CUDA graph capture failed ({type(ex).__name__}: {str(ex)[:120]}); eager timing reported"
@@ -735,6 +792,8 @@ def run_tgn_snapshots(args):
             "cpu_baseline": cpu, "e2e": None, "gpu_launches": launches, "clocks": clocks,
             "timing": {"eager_ms_per_step": eager_ms, "cuda_graph": graph_note},
         }
+        if dumped is not None:
+            write_outputs(args.dump_outputs, dumped)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -804,7 +863,11 @@ def main():
                     help="time the step as replays of one CUDA graph (auto: multi-GPU only)")
     ap.add_argument("--mgpu", default="input", choices=["input", "replicate", "allgather"],
                     help="multi-GPU variant of the destination-range partition (see partition.py)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference_arm(args)
     if args.workload == "tgn_snapshots":

@@ -1,16 +1,16 @@
-"""Generates the committed fixtures under tests/golden/ (run in the authoring container only).
+"""Generates the committed fixtures under tests/golden/.
 
-  python tests/golden/make_golden.py
+  python tests/golden/make_golden.py REFERENCE_CHECKOUT
 
 * ``gat_ckpt.npz`` / ``tgn_ckpt.npz``: the reference's own trained weights
-  (/root/reference/results/gat_model.pt, tgn_model.pt -- the only golden artefacts the reference ships
-  for this path), converted to numpy with the ``lin_dst.weight`` alias dropped (it is bit-identical to
-  ``lin_src.weight``; asserted below).
+  (REFERENCE_CHECKOUT/results/gat_model.pt, tgn_model.pt of aum2606/GNN-Fraud-Detection -- the only golden artefacts
+  the reference ships for this path), converted to numpy with the ``lin_dst.weight`` alias dropped (it is bit-identical
+  to ``lin_src.weight``; asserted below).
 * ``golden_small.npz``: a seeded small Elliptic-shaped input and the outputs of the ORACLE
   (oracle/pyg_gatconv.py) on it with those weights: layer-0 GATConv output + attention, full GAT and
   TemporalGNN eval-mode logits, and the CSR of the graph.  PyG itself is not installable here, so these
   are oracle outputs, not outputs of the reference running -- they pin the oracle against regressions
-  and give the GPU tests a fixed target that does not need /root/reference at run time.
+  and give the GPU tests a fixed target that does not need the reference at run time.
 """
 import os
 import sys
@@ -25,11 +25,8 @@ sys.path.insert(0, ROOT)
 from oracle import pyg_gatconv as O  # noqa: E402
 from gnn_fraud_detection_b200 import synth  # noqa: E402
 
-REF = "/root/reference/results"
-
-
 def convert(name):
-    sd = torch.load(os.path.join(REF, name), map_location="cpu", weights_only=False)
+    sd = torch.load(os.path.join(sys.argv[1], "results", name), map_location="cpu", weights_only=False)
     out = {}
     for k, v in sd.items():
         if k.endswith("lin_dst.weight"):

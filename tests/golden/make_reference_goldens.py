@@ -1,8 +1,9 @@
-"""Golden vectors produced by the reference's OWN model code (run in the authoring container only).
+"""Golden vectors produced by the reference's OWN model code.
 
-  python tests/golden/make_reference_goldens.py
+  python tests/golden/make_reference_goldens.py REFERENCE_CHECKOUT
 
-``/root/reference/src/models/gat.py`` and ``tgn.py`` are imported UNMODIFIED (importlib, from where they lie).  Their
+``REFERENCE_CHECKOUT/src/models/gat.py`` and ``tgn.py`` (a checkout of aum2606/GNN-Fraud-Detection) are imported
+UNMODIFIED (importlib, from where they lie).  Their
 only missing import is third-party ``torch_geometric.nn.GATConv`` (not installable here), which is satisfied by a stub
 module exposing the CPU oracle layer (``oracle.pyg_gatconv.OracleGATConv``).  The reference's classes -- constructor
 logic, layer loop, BatchNorm / ReLU / dropout / residual, GRUCell head, ``predict`` -- then run exactly as shipped, load the
@@ -14,8 +15,13 @@ stored in ``reference_models_golden.npz``:
     reference's loss (masked ``BCEWithLogitsLoss(pos_weight=50)``, ``src/train.py:108-139,360-361``) in fp64: loss, logits
     and the gradient of every parameter.
 
-``/root/reference`` does not exist on the GPU box, so the GPU tests compare the CUDA models with THIS file; the CPU test
-``tests/test_reference_models.py`` re-derives it from the reference sources whenever they are present.
+To keep the file under 1 MB, ``shrink`` stores every float array as float32 (its rounding is three orders of magnitude
+below the tolerances of the tests that read it) and, of each weight gradient with more than 64 rows, a fixed seeded half
+of its rows (their indices under ``<name>.rows``).  The fp32 eval outputs are not stored: they are bit-identical to
+``golden_small.npz``'s ``gat_logits`` / ``tgn_logits`` / ``tgn_hidden``.
+
+The reference is not part of this repository, so the tests compare with THIS file: the GPU tests the CUDA models, and
+``tests/test_reference_models.py`` the oracle's restated wrappers (which reproduced it bit for bit in fp64).
 """
 import importlib.util
 import os
@@ -28,10 +34,10 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-REF = "/root/reference"
+ROW_SAMPLE_MIN_ROWS = 64
 
 
-def load_reference_models(gatconv_cls):
+def load_reference_models(gatconv_cls, ref):
     """The reference's ``GAT`` / ``TemporalGNN`` classes with ``torch_geometric.nn.GATConv`` := ``gatconv_cls``."""
     saved = {k: sys.modules.get(k) for k in ("torch_geometric", "torch_geometric.nn", "src", "src.config")}
     tg, tgnn = types.ModuleType("torch_geometric"), types.ModuleType("torch_geometric.nn")
@@ -40,12 +46,12 @@ def load_reference_models(gatconv_cls):
     sys.modules["torch_geometric"], sys.modules["torch_geometric.nn"] = tg, tgnn
     # tgn.py does `from src.config import MODEL_CONFIG` (never used): load the reference's config the same way
     src_pkg = types.ModuleType("src")
-    src_pkg.__path__ = [os.path.join(REF, "src")]
+    src_pkg.__path__ = [os.path.join(ref, "src")]
     sys.modules["src"] = src_pkg
     mods = {}
     try:
         for name, rel in (("src.config", "src/config.py"), ("_ref_gat", "src/models/gat.py"), ("_ref_tgn", "src/models/tgn.py")):
-            spec = importlib.util.spec_from_file_location(name, os.path.join(REF, rel))
+            spec = importlib.util.spec_from_file_location(name, os.path.join(ref, rel))
             m = importlib.util.module_from_spec(spec)
             sys.modules[name] = m
             spec.loader.exec_module(m)
@@ -59,16 +65,16 @@ def load_reference_models(gatconv_cls):
     return mods["_ref_gat"].GAT, mods["_ref_tgn"].TemporalGNN
 
 
-def reference_outputs():
+def reference_outputs(ref):
     from oracle import pyg_gatconv as O
-    RefGAT, RefTGN = load_reference_models(O.OracleGATConv)
+    RefGAT, RefTGN = load_reference_models(O.OracleGATConv, ref)
     gold = np.load(os.path.join(HERE, "golden_small.npz"))
     x, ei = torch.from_numpy(gold["x"]), torch.from_numpy(gold["edge_index"])
     K = x.size(1)
     out = {}
     sds = {}
     for name, cls, ck in (("gat", RefGAT, "gat_model.pt"), ("tgn", RefTGN, "tgn_model.pt")):
-        sd = torch.load(os.path.join(REF, "results", ck), map_location="cpu", weights_only=False)
+        sd = torch.load(os.path.join(ref, "results", ck), map_location="cpu", weights_only=False)
         sds[name] = sd
         m = cls(K, 64, 1, num_layers=3)                         # compare_gnn_models.py:35-54
         m.load_state_dict(sd, strict=True)                      # src/evaluate.py:173-176
@@ -107,8 +113,25 @@ def reference_outputs():
     return out
 
 
+def shrink(full):
+    """What the fixture stores of ``reference_outputs()`` (see the module docstring)."""
+    out = {}
+    for k, a in full.items():
+        a = np.asarray(a)
+        if k.endswith("_f32"):
+            continue
+        if a.dtype == np.float64 and a.ndim > 0:
+            a = a.astype(np.float32)
+        if k.startswith("train_") and "_grad." in k and a.ndim == 2 and a.shape[0] > ROW_SAMPLE_MIN_ROWS:
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], a.shape[0] // 2, replace=False))
+            out[k + ".rows"] = rows
+            a = a[rows]
+        out[k] = a
+    return out
+
+
 def main():
-    out = reference_outputs()
+    out = shrink(reference_outputs(sys.argv[1]))
     path = os.path.join(HERE, "reference_models_golden.npz")
     np.savez_compressed(path, **out)
     print(path, os.path.getsize(path), "bytes;", len(out), "arrays")
