@@ -18,7 +18,7 @@ F32, BF16 = 0, 1
 ACT_NONE, ACT_RELU, ACT_ELU = 0, 1, 2
 GEMM_AUTO, GEMM_SIMT, GEMM_TC, GEMM_INPUT = 0, 1, 2, 3
 HUB_THRESHOLD, HUB_CHUNK = 512, 512
-ABI_VERSION = 18
+ABI_VERSION = 19
 
 _i32p = C.POINTER(C.c_int32)
 
@@ -118,6 +118,10 @@ SIGNATURES = {
     "gnnfd_gru_head_bwd": (_i, [_vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                 _vp, _vp, _sz, _vp]),
     "gnnfd_bce_masked": (_i, [_vp, _vp, _i64, _f, _f, _vp, _vp, _vp, _vp, _sz, _vp]),
+    # neighbour sampling
+    "gnnfd_sample_workspace_bytes": (_i, [_i64, _i64, C.c_int32, _szp]),
+    "gnnfd_neighbor_sample": (_i, [_vp, _vp, _vp, _i64, _vp, _i64, _i32p, C.c_int32, _u64, _vp, _vp, _i64, _vp, _i64, _vp,
+                                   _i64, _i64p, _vp, _sz, _vp]),
 }
 
 

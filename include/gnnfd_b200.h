@@ -37,7 +37,7 @@
 extern "C" {
 #endif
 
-#define GNNFD_ABI_VERSION 18
+#define GNNFD_ABI_VERSION 19
 
 typedef void* gnnfd_stream_t; /* cudaStream_t */
 
@@ -372,6 +372,37 @@ int gnnfd_in_logits_bcast(const float* x, int64_t ldx, int64_t N, int64_t K, con
  * (deterministic).  The reduce-scatter of the partial da_src [n_pos,H]: every rank reduces ITS OWN row range. */
 int gnnfd_peer_reduce(const gnnfd_peers_t* buf, int64_t offset, int64_t n, int op, int use_multicast, float* out,
                       gnnfd_stream_t stream);
+
+/* ---- (8) neighbour sampling (src/data/dataloader.py:42-66, NeighborLoader(num_neighbors=[10,10,10]) with PyG's defaults
+ * replace=False, directed=True) ----------------------------------------------------------------------------------------
+ * Graph: the RAW destination-sorted CSR of edge_index [2,E] (gnnfd_csr_build with flags = 0): rowptr [N+1], col [E] the
+ * source of each sorted edge, eid [E] its column in edge_index (the csr_build `perm`).  The neighbours of v are its in-edges
+ * j -> v, duplicates and self-loops included; position p is the p-th in-edge of v in edge_index order.
+ * Hop 1 expands the seeds; hop l expands exactly the nodes first discovered in hop l-1 (no node is expanded twice).
+ * Selection for a node v of in-degree d expanded with fanout k: every position 0..d-1 when k == -1 or d <= k; otherwise
+ * Floyd's algorithm -- for i = 0..k-1: j = d-k+i, t = U_i(j), add j if t is already chosen, else t -- and the chosen
+ * positions in ascending order (fanouts up to 32 resolve Floyd in registers; larger ones cost O(k^2/32) per node, serial per
+ * warp).  U_i(j) = mulhi64(w, j+1), w = splitmix64(seed + 0x9E3779B97F4A7C15 * (2*(v*2^32 + i) + 1))
+ * (mod 2^64), so a node's sample depends only on (seed, v): not on the batch, the hop or the scheduling.
+ * Outputs: n_id [node_cap] int64 global ids -- the seeds (local ids 0..B-1, input order), then the nodes new in hop 1 in
+ * order of first appearance in hop 1's edge list, then hop 2, ...; edges ordered by hop, then by local destination id, then
+ * by position: edge_index rows at [0, m) (local source) and [ld_edge, ld_edge + m) (local destination, non-decreasing),
+ * e_id [m] = column in the input edge_index.
+ * counts_host [3 + 2*n_hops]: total nodes, total edges, then num_sampled_nodes = [B, n_1..n_L], then
+ * num_sampled_edges = [m_1..m_L].  Synchronises `stream` once to return them.
+ * node_map [N] int32 must be all -1 on entry and is all -1 on return, also when the call fails after launching (the reset
+ * touches only the sampled entries: a call costs work proportional to the sample, never O(N)).
+ * Errors: seed outside [0,N) -> GNNFD_ERR_RANGE; duplicate seeds (found on the device), a fanout < -1 or more than 64 hops
+ * -> GNNFD_ERR_ARG;
+ * more nodes than node_cap or edges than edge_cap -> GNNFD_ERR_WORKSPACE (nothing is written beyond the caps).  Caps that
+ * always suffice: nodes min(N, B * prod(1 + k_l)), edges min(E, sum_l F_l * k_l) with F_1 = B, F_{l+1} = min(N, F_l * k_l),
+ * reading k = -1 as the maximum in-degree. */
+int gnnfd_sample_workspace_bytes(int64_t node_cap, int64_t edge_cap, int32_t n_hops, size_t* bytes);
+int gnnfd_neighbor_sample(const int32_t* rowptr, const int32_t* col, const int32_t* eid, int64_t N,
+                          const int64_t* seeds, int64_t n_seeds, const int32_t* fanouts_host, int32_t n_hops,
+                          uint64_t seed, int32_t* node_map, int64_t* n_id, int64_t node_cap, int64_t* edge_index,
+                          int64_t ld_edge, int64_t* e_id, int64_t edge_cap, int64_t* counts_host,
+                          void* ws, size_t ws_bytes, gnnfd_stream_t stream);
 
 #ifdef __cplusplus
 }
