@@ -1,6 +1,10 @@
 // (4a) backward, dst-major pass (autograd mirror of GATConv.forward's edge_update/aggregate, triggered by
 // loss.backward() at src/train.py:142; closed forms in SURVEY.md 8(a3)).
 //
+// For the head mean on a graph with direct edge-gradient slots, gnnfd_gat_bwd_dst runs the two-pass form of
+// gat_bwd_dalpha.cu (d_alpha source-major, then a dst pass that reads no features).  The kernels below are the
+// single-pass gather form, used for concat, for the multi-GPU receive layout and for the destination-range row view.
+//
 // Same warp-stream structure as the forward (gat_stream.cuh): one warp per edge-balanced work item, the
 // 2 KB source rows arrive through the bulk-copy ring.  Per chunk of <= 32 edges:
 //   phase A  lane = edge: recompute alpha from the saved row statistics, remember the LeakyReLU slope and
@@ -24,6 +28,11 @@
 namespace gnnfd {
 extern std::atomic<long long> g_launches;
 int check_graph(const gnnfd_graph_t* g, bool need_csc, const char* who);
+bool gat_bwd_dst_srcmajor_applies(const gnnfd_graph_t* g, int concat);       // gat_bwd_dalpha.cu
+int gat_bwd_dst_srcmajor(const gnnfd_graph_t* g, const void* xw, int xw_dtype, int H, int C, const float* a_src,
+                         const float* a_dst, const float* rowmax, const float* rowsum, const float* d_out,
+                         float negative_slope, const uint8_t* keep_mask, float p_drop, uint64_t seed, float* alpha_used,
+                         float* dz, float* da_dst, void* ws, size_t ws_bytes, cudaStream_t st);
 
 
 // dO_h slice owned by this lane (already divided by H for the head mean)
@@ -60,8 +69,7 @@ __device__ __forceinline__ void bwd_dst_stream(ChunkCursor& cur, WarpRing<GE, bw
                                                float* __restrict__ da_dst, float* __restrict__ part_t, int chunk_id,
                                                int lane)
 {
-    constexpr int H = GE::H, NS = GE::NS, VW = GE::VW, HP = GE::HP, G = GE::G;
-    const int sub = lane / G;
+    constexpr int H = GE::H, NS = GE::NS, VW = GE::VW;
     float* dal_s = reinterpret_cast<float*>(ring.extra);
     int* bits_s = reinterpret_cast<int*>(ring.extra + 32 * H * 4);
     auto on_empty = [&](int r) {
@@ -108,26 +116,7 @@ __device__ __forceinline__ void bwd_dst_stream(ChunkCursor& cur, WarpRing<GE, bw
 #pragma unroll
                 for (int k = 0; k < VW; ++k) d[q] = fmaf(g0[q][k], v[q][k], d[q]);
             }
-            if constexpr (NS == 4 && G == 16) {
-                // reduce-scatter butterfly over the 16-lane head group: 5 shuffles instead of 4 x 4.  After the
-                // xor-8 / xor-4 steps a lane keeps only slot q = 2*bit3 + bit2; xor-2 / xor-1 finish its sum.
-                const bool b3 = lane & 8, b2 = lane & 4;
-                const float k0 = b3 ? d[2] : d[0], k1 = b3 ? d[3] : d[1];
-                const float s0 = b3 ? d[0] : d[2], s1 = b3 ? d[1] : d[3];
-                const float a0 = k0 + __shfl_xor_sync(FULL, s0, 8), a1 = k1 + __shfl_xor_sync(FULL, s1, 8);
-                float b = (b2 ? a1 : a0) + __shfl_xor_sync(FULL, b2 ? a0 : a1, 4);
-                b += __shfl_xor_sync(FULL, b, 2);
-                b += __shfl_xor_sync(FULL, b, 1);
-                if ((lane & 3) == 0) dal_s[t * H + ((lane >> 2) & 3) * HP + sub] = b;
-            } else {
-#pragma unroll
-                for (int q = 0; q < NS; ++q) {
-                    float dq = d[q];
-#pragma unroll
-                    for (int o = G / 2; o > 0; o >>= 1) dq += __shfl_xor_sync(FULL, dq, o);
-                    if ((lane & (G - 1)) == 0) dal_s[t * H + q * HP + sub] = dq;
-                }
-            }
+            dalpha_reduce<GE>(d, dal_s + t * H, lane);
             ring.pop();
             if (issued0 < c0.n) ring.issue(xw, j0[issued0++], lane);
             else if (have1 && issued1 < c1.n) ring.issue(xw, j1[issued1++], lane);
@@ -241,8 +230,7 @@ __device__ __forceinline__ void bwd_dst_stream_pack(ChunkCursor& cur, WarpRing<G
                                                     float* __restrict__ alpha_used, float* __restrict__ dz, int64_t eg_ld,
                                                     float* __restrict__ da_dst, int lane)
 {
-    constexpr int H = GE::H, NS = GE::NS, VW = GE::VW, HP = GE::HP, G = GE::G;
-    const int sub = lane / G;
+    constexpr int H = GE::H, NS = GE::NS, VW = GE::VW;
     float* dal_s = reinterpret_cast<float*>(ring.extra);
     int* bits_s = reinterpret_cast<int*>(ring.extra + 32 * H * 4);
     auto on_empty = [&](int r) {
@@ -298,24 +286,7 @@ __device__ __forceinline__ void bwd_dst_stream_pack(ChunkCursor& cur, WarpRing<G
 #pragma unroll
                 for (int kk = 0; kk < VW; ++kk) d[q] = fmaf(g0[q][kk], v[q][kk], d[q]);
             }
-            if constexpr (NS == 4 && G == 16) {
-                const bool b3 = lane & 8, b2 = lane & 4;
-                const float kk0 = b3 ? d[2] : d[0], kk1 = b3 ? d[3] : d[1];
-                const float s0 = b3 ? d[0] : d[2], s1 = b3 ? d[1] : d[3];
-                const float a0 = kk0 + __shfl_xor_sync(FULL, s0, 8), a1 = kk1 + __shfl_xor_sync(FULL, s1, 8);
-                float b = (b2 ? a1 : a0) + __shfl_xor_sync(FULL, b2 ? a0 : a1, 4);
-                b += __shfl_xor_sync(FULL, b, 2);
-                b += __shfl_xor_sync(FULL, b, 1);
-                if ((lane & 3) == 0) dal_s[t * H + ((lane >> 2) & 3) * HP + sub] = b;
-            } else {
-#pragma unroll
-                for (int q = 0; q < NS; ++q) {
-                    float dq = d[q];
-#pragma unroll
-                    for (int o = G / 2; o > 0; o >>= 1) dq += __shfl_xor_sync(FULL, dq, o);
-                    if ((lane & (G - 1)) == 0) dal_s[t * H + q * HP + sub] = dq;
-                }
-            }
+            dalpha_reduce<GE>(d, dal_s + t * H, lane);
             ring.pop();
             if (issued0 < c0.n) ring.issue(xw, j0[issued0++], lane);
             else if (kind1 && issued1 < c1.n) ring.issue(xw, j1[issued1++], lane);
@@ -571,6 +542,9 @@ int gnnfd_gat_bwd_dst(const gnnfd_graph_t* g, const void* xw, int xw_dtype, cons
                   "gat_bwd_dst: csr2csc is NULL (edge gradients are emitted in source-major order)");
     GNNFD_REQUIRE(p_drop >= 0.f && p_drop < 1.f, GNNFD_ERR_ARG, "gat_bwd_dst: dropout p must be in [0,1)");
     cudaStream_t st = (cudaStream_t)stream;
+    if (gat_bwd_dst_srcmajor_applies(g, concat))
+        return gat_bwd_dst_srcmajor(g, xw, xw_dtype, H, C, a_src, a_dst, rowmax, rowsum, d_out, negative_slope, keep_mask,
+                                    p_drop, dropout_seed, alpha_used, dz, da_dst, ws, ws_bytes, st);
     if (H == 8 && C == 64 && xw_dtype == GNNFD_F32)
         return launch_bwd_dst<Geo<8, 64, float>>(g, xw, a_src, a_dst, rowmax, rowsum, d_out, negative_slope, concat,
                                                  keep_mask, p_drop, dropout_seed, alpha_used, dz, da_dst, ws, ws_bytes, st);

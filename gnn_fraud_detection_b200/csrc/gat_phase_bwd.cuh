@@ -69,6 +69,35 @@ __device__ __forceinline__ void bwd_phase_a(const BwdChunk& c, const int32_t* __
     __syncwarp();
 }
 
+// phase B's head reduction: d[q] is this lane's partial dot product for head q*HP + lane/G; the full sums
+// d_alpha[0..H) of the edge land in dal_t[0..H).
+template <class GE>
+__device__ __forceinline__ void dalpha_reduce(const float (&d)[GE::NS], float* dal_t, int lane)
+{
+    constexpr int NS = GE::NS, HP = GE::HP, G = GE::G;
+    const int sub = lane / G;
+    if constexpr (NS == 4 && G == 16) {
+        // reduce-scatter butterfly over the 16-lane head group: 5 shuffles instead of 4 x 4.  After the
+        // xor-8 / xor-4 steps a lane keeps only slot q = 2*bit3 + bit2; xor-2 / xor-1 finish its sum.
+        const bool b3 = lane & 8, b2 = lane & 4;
+        const float k0 = b3 ? d[2] : d[0], k1 = b3 ? d[3] : d[1];
+        const float s0 = b3 ? d[0] : d[2], s1 = b3 ? d[1] : d[3];
+        const float a0 = k0 + __shfl_xor_sync(FULL, s0, 8), a1 = k1 + __shfl_xor_sync(FULL, s1, 8);
+        float b = (b2 ? a1 : a0) + __shfl_xor_sync(FULL, b2 ? a0 : a1, 4);
+        b += __shfl_xor_sync(FULL, b, 2);
+        b += __shfl_xor_sync(FULL, b, 1);
+        if ((lane & 3) == 0) dal_t[((lane >> 2) & 3) * HP + sub] = b;
+    } else {
+#pragma unroll
+        for (int q = 0; q < NS; ++q) {
+            float dq = d[q];
+#pragma unroll
+            for (int o = G / 2; o > 0; o >>= 1) dq += __shfl_xor_sync(FULL, dq, o);
+            if ((lane & (G - 1)) == 0) dal_t[q * HP + sub] = dq;
+        }
+    }
+}
+
 // second sweep of a long row: dz = slope * (u - alpha * t); returns the lane-local partial of da_dst
 template <class GE>
 __device__ __forceinline__ void dst_sweep2(const RowStat<GE::H>& r, int beg, int end, const int32_t* __restrict__ col,
@@ -100,6 +129,23 @@ __device__ __forceinline__ void dst_sweep2(const RowStat<GE::H>& r, int beg, int
 // every row of the pack in registers with SEGMENTED warp sums.
 // bits layout per staged edge: [0,8) LeakyReLU-positive, [8,16) dropout keep, [16,21) first lane of the row,
 // [21,26) last lane of the row, bit 26 = this edge is the last of its row.
+//
+// The row of lane `lane`'s edge inside a pack of k rows starting at edge beg: its index lo in the pack and its first /
+// last lane sa / sb (lanes l < k hold row l's edge range in lane_a / lane_b).
+__device__ __forceinline__ void pack_lane_segment(int beg, int k, int lane_a, int lane_b, int lane, int& lo, int& sa, int& sb)
+{
+    const int e_id = beg + lane;
+    int hi = k - 1;
+    lo = 0;
+#pragma unroll
+    for (int it = 0; it < 5; ++it) {
+        const int mid = (lo + hi) >> 1;
+        const int bm = __shfl_sync(FULL, lane_b, mid);
+        if (bm > e_id) hi = mid; else lo = min(mid + 1, k - 1);
+    }
+    sa = __shfl_sync(FULL, lane_a, lo) - beg;
+    sb = __shfl_sync(FULL, lane_b, lo) - beg - 1;
+}
 template <class GE, bool CONCAT, bool DROPOUT>
 __device__ __forceinline__ void bwd_phase_a_pack(int row0, int beg, int n, int k, int lane_a, int lane_b,
                                                  const int32_t* __restrict__ col, const int32_t* __restrict__ perm,
@@ -111,15 +157,8 @@ __device__ __forceinline__ void bwd_phase_a_pack(int row0, int beg, int n, int k
     constexpr int H = GE::H;
     const bool act = lane < n;
     const int e_id = beg + lane;
-    int lo = 0, hi = k - 1;
-#pragma unroll
-    for (int it = 0; it < 5; ++it) {
-        const int mid = (lo + hi) >> 1;
-        const int bm = __shfl_sync(FULL, lane_b, mid);
-        if (bm > e_id) hi = mid; else lo = min(mid + 1, k - 1);
-    }
-    const int sa = __shfl_sync(FULL, lane_a, lo) - beg;
-    const int sb = __shfl_sync(FULL, lane_b, lo) - beg - 1;
+    int lo, sa, sb;
+    pack_lane_segment(beg, k, lane_a, lane_b, lane, lo, sa, sb);
     if (!CONCAT) {
         // the pack's dO rows are one contiguous block of k*C floats
         const char* pb = reinterpret_cast<const char*>(d_out + int64_t(row0) * GE::C);

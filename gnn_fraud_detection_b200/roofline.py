@@ -3,6 +3,8 @@
 Gather traffic is charged per edge (no credit for cache reuse); indices are int32 (i = 4 B); logits,
 row statistics, gradients are fp32; ``s`` is the storage size of a projected feature element (4 fp32 /
 2 bf16); ``Co`` = C (head mean) or H*C (concat).  ``Ep`` is E' (edges after the self-loop rewrite).
+The ``gat_bwd_dst`` term describes the backward that runs: for the head mean the two-pass form (d_alpha computed
+source-major, then a dst pass that reads no features), for ``concat`` the single gather pass.
 """
 from __future__ import annotations
 
@@ -17,9 +19,16 @@ def stage_bytes(N: int, Ep: int, K: int, H: int = 8, C: int = 64, concat: bool =
     b["project_fwd"] = N * (K * 4 + D * s + 8 * H) + K * D * 4
     # per edge: xw[src] row, col, a_src[src]; per row: a_dst, out, (max,sum), rowptr
     b["gat_fwd"] = Ep * (D * s + i + 4 * H) + N * (4 * H + 4 * Co + 8 * H + i)
-    # per edge: xw[src] row, col, a_src[src], dz write (alpha write is not charged, as in SURVEY 8(d));
-    # per row: dOut, (a_dst,max,sum), da_dst, rowptr
-    b["gat_bwd_dst"] = Ep * (D * s + i + 4 * H + 4 * H) + N * (4 * Co + 8 * H + 4 * H + i)
+    if concat:
+        # one gather pass -- per edge: xw[src] row, col, a_src[src], dz write (alpha write is not charged, as in
+        # SURVEY 8(d)); per row: dOut, (a_dst,max,sum), da_dst, rowptr
+        b["gat_bwd_dst"] = Ep * (D * s + i + 4 * H + 4 * H) + N * (4 * Co + 8 * H + 4 * H + i)
+    else:
+        # head mean, two passes (DESIGN 4.4).  Source-major d_alpha -- per edge: csc_row, dOut[dst] row,
+        # (a_dst,max,sum)[dst], (alpha, d_alpha) write; per source row: xw row, a_src, colptr.  Feature-free dst pass --
+        # per edge: csr2csc, the (alpha, d_alpha) read and the (alpha_used, dz) write; per row: da_dst, rowptr
+        b["gat_bwd_dst"] = (Ep * (i + 4 * Co + 12 * H + 8 * H) + Ns * (D * s + 4 * H + i)
+                            + Ep * (i + 8 * H + 8 * H) + N * (4 * H + i))
     # per edge: dOut[dst] row, (csc_row, csc_eid), alpha, dz; per source row: dxw write, da_src write, colptr
     b["gat_bwd_src"] = Ep * (4 * Co + 2 * i + 4 * H + 4 * H) + Ns * (D * 4 + 4 * H + i)
     # GEMM-bwd: read dxw, xw, x (+ dx write), da_src/da_dst; W read + dW write
