@@ -3,21 +3,22 @@
 // d_alpha[e,h] = <dO[i]/H, xw[j,h,:]> needs no row reduction, and with the head mean dO[i] is one C-float row
 // shared by all heads.  So d_alpha is computed SOURCE-major, where xw[j] is read once, and only the 256 B dO[i] row
 // is gathered per edge; the row reductions follow in a second pass that reads no features.
-//   pass 1 (CSC, one warp per source row j; gat_bwd_dalpha_src_rows / _hub): xw[j] is held in registers in the
-//            slot layout of gat_common.cuh.  Per chunk of <= 32 out-edges the warp copies the chunk's dO rows into
-//            shared memory (cp.async, all in flight at once) while each lane (= edge) computes alpha from the
-//            destination's saved statistics exactly as phase A does.  Then per edge 16 FMAs and phase B's butterfly
-//            give d_alpha with phase B's arithmetic.  The edge's 64 B slot of the edge-gradient buffer (its CSC
-//            position) receives the pre-dropout alpha, with the sign bit set where the logit is on the LeakyReLU's
-//            negative side, and d_alpha.  Sources above the hub threshold are split by the hub_src plan; every output
-//            is per edge, so the chunks need no merge.
+//   pass 1 (CSC; gat_bwd_dalpha_src_stream / _hub): one warp streams the out-edges of one work item in CSC order,
+//            across source-row boundaries, as tasks of <= 32 edges of one source row.  Each task's dO rows go into a
+//            per-warp ring of DA_RING row slots and, when the task starts a new source row, xw[j] into one of
+//            DA_XROWS row slots (16-byte cp.async, 16 lanes per dO row, one commit group per task), so the next
+//            tasks' rows are in flight while the current one is reduced.  Per edge 16 FMAs and phase B's butterfly
+//            give d_alpha with phase B's arithmetic; it is stored at the edge's CSR position csc_eid[p] of an
+//            [E',H] workspace buffer.  Sources above the hub threshold are split by the hub_src plan (_hub, one
+//            warp per chunk); every output is per edge, so the chunks need no merge.
 //   pass 2 (CSR; gat_bwd_dst_eg_items / _hub1 / _hub2): the chunk, pack and hub_dst schedule of the gather kernels,
-//            lane = edge, reading the slot at csr2csc[e] instead of the row xw[col[e]].  Keep bits, u = alpha *
-//            d_alpha * keep, t, dz and da_dst use the same warp sums in the same order as the gather kernels, and
-//            the slot is overwritten with (alpha_used, dz) by the thread that read it.
-// Per edge this moves ~4 + 256 + 96 + 64 B (pass 1) and ~4 + 64 + 64 B (pass 2) instead of a 2 KB row.  alpha_used
-// equals the gather kernels' bit for bit; dz and da_dst differ in the last bits on rows longer than one chunk, where
-// the gather kernels recompute alpha for the second sweep with a contracted multiply-add.
+//            lane = edge.  It reads col, d_alpha, csr2csc (and perm) contiguously, the row statistics per row and
+//            a_src[col[e]] as its one gather, recomputes alpha with edge_alpha, and forms u = alpha * d_alpha * keep,
+//            t, dz and da_dst with the same warp sums in the same order as the gather kernels.  (alpha_used, dz) go
+//            to the edge's source-major slot csr2csc[e].
+// Per edge this moves ~4 + 4 + 256 + 32 B (pass 1) and ~4 + 32 + 32 + 4 + 64 B (pass 2).  alpha_used equals the
+// gather kernels' bit for bit; dz and da_dst differ in the last bits on rows longer than one chunk, where the gather
+// kernels recompute alpha for the second sweep with a contracted multiply-add.
 #include "gat_stream.cuh"
 #include "gat_phase_bwd.cuh"
 
@@ -27,142 +28,187 @@
 namespace gnnfd {
 extern std::atomic<long long> g_launches;
 
-constexpr int DA_WARPS = 4;                  // warps per CTA in pass 1 (the dO staging fits static shared memory)
+constexpr int DA_WARPS = 4;                  // warps per CTA in pass 1
 constexpr int DA_THREADS = DA_WARPS * 32;
+constexpr int DA_RING = 32;                  // dO row slots per warp (pass 1 stream): a whole 32-edge task fits
+constexpr int DA_XROWS = 2;                  // xw row slots per warp (pass 1 stream)
+constexpr int DA_TASKS = 8;                  // tasks in flight per warp at most (cp.async groups)
 
 __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc)
 {
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(st_smem_u32(smem_dst)), "l"(gsrc) : "memory");
 }
-__device__ __forceinline__ void cp_async_wait_all()
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+// wait until at most n of this thread's commit groups are pending (n < DA_TASKS)
+__device__ __forceinline__ void cp_async_wait_pending(int n)
 {
-    asm volatile("cp.async.commit_group;\n\tcp.async.wait_group 0;" ::: "memory");
+    switch (n) {
+    case 0: asm volatile("cp.async.wait_group 0;" ::: "memory"); break;
+    case 1: asm volatile("cp.async.wait_group 1;" ::: "memory"); break;
+    case 2: asm volatile("cp.async.wait_group 2;" ::: "memory"); break;
+    case 3: asm volatile("cp.async.wait_group 3;" ::: "memory"); break;
+    case 4: asm volatile("cp.async.wait_group 4;" ::: "memory"); break;
+    case 5: asm volatile("cp.async.wait_group 5;" ::: "memory"); break;
+    case 6: asm volatile("cp.async.wait_group 6;" ::: "memory"); break;
+    default: asm volatile("cp.async.wait_group 7;" ::: "memory"); break;
+    }
 }
-constexpr uint32_t NEG_FLAG = 0x80000000u;   // sign bit of the stored alpha: LeakyReLU-negative logit
+static_assert(DA_TASKS <= 8 && DA_TASKS <= 32, "cp_async_wait_pending covers 8 groups; one lane holds each task");
+static_assert(DA_RING >= 32, "a task of 32 edges must fit the dO ring, or the stream could never issue it");
+constexpr uint32_t NEG_FLAG = 0x80000000u;   // sign bit of alpha held in registers: LeakyReLU-negative logit
 
 // ---------------------------------------------------------------------------------------------------------
 // pass 1: source-major d_alpha
 // ---------------------------------------------------------------------------------------------------------
-// out-edges [beg, end) of source row j (a whole row, or one hub chunk of it).  Per chunk the warp copies the chunk's
-// dO rows into do_s [32][C] (cp.async, all in flight at once) while the lanes compute alpha.
-template <class GE>
-__device__ __forceinline__ void dalpha_range(int64_t j, int beg, int end, const int32_t* __restrict__ csc_row,
-                                             const typename GE::XT* __restrict__ xw, const float* __restrict__ a_src,
-                                             const float* __restrict__ a_dst, const float* __restrict__ rowmax,
-                                             const float* __restrict__ rowsum, const float* __restrict__ d_out,
-                                             float slope, float* __restrict__ alpha_used, float* __restrict__ dz,
-                                             int64_t eg_ld, float* do_s, float* dal_s, int* i_s, int lane)
+// copies dO rows [i_0 .. i_{n-1}] (lane l holds i_l) into the slots (first + r) % SLOTS: C/4 lanes per row, 16 B
+// each, so every instruction moves 32/(C/4) whole rows
+template <class GE, int SLOTS>
+__device__ __forceinline__ void copy_do_rows(float* do_s, int first, int n, int i, const float* __restrict__ d_out,
+                                             int lane)
 {
-    constexpr int H = GE::H, NS = GE::NS, VW = GE::VW, C = GE::C;
-    static_assert((32 * VW) % C == 0, "every slot of a lane must see the same dO channels");
-    float v[NS][VW];
-#pragma unroll
-    for (int q = 0; q < NS; ++q) load_slot(xw + j * GE::D, q, lane, v[q]);
-    const int cm = (VW * lane) % C;          // dO channels of this lane's slots
-    const float sc = 1.f / H;
-    for (int base = beg; base < end; base += 32) {
-        const int n = min(32, end - base);
-        const int64_t i = lane < n ? csc_row[base + lane] : 0;
-        i_s[lane] = int(i);
-        __syncwarp();
-        // C/4 lanes copy one dO row (16 B each): every instruction moves 32/(C/4) whole rows
-        {
-            constexpr int LPR = C / 4, RPI = 32 / LPR;
-            const int sub = lane / LPR, c4 = 4 * (lane % LPR);
-#pragma unroll
-            for (int r = 0; r < 32; r += RPI)
-                if (r + sub < n) cp_async16(do_s + (r + sub) * C + c4, d_out + int64_t(i_s[r + sub]) * C + c4);
-        }
-        if (lane < n) {
-            // alpha as phase A computes it (load_row_stat), four heads at a time
-#pragma unroll
-            for (int k = 0; k < H / 4; ++k) {
-                const float4 as = __ldg(reinterpret_cast<const float4*>(a_src + j * H) + k);
-                const float4 ad = __ldg(reinterpret_cast<const float4*>(a_dst + i * H) + k);
-                const float4 mx = __ldg(reinterpret_cast<const float4*>(rowmax + i * H) + k);
-                const float4 sm = __ldg(reinterpret_cast<const float4*>(rowsum + i * H) + k);
-                const float zs[4] = {as.x + ad.x, as.y + ad.y, as.z + ad.z, as.w + ad.w};
-                const float ms[4] = {mx.x, mx.y, mx.z, mx.w}, ss[4] = {sm.x, sm.y, sm.z, sm.w};
-                float al[4];
-#pragma unroll
-                for (int h = 0; h < 4; ++h) {
-                    const float z = zs[h], inv = 1.f / ss[h];
-                    const bool pos = z > 0.f;
-                    const float a = expf((pos ? z : z * slope) - ms[h]) * inv;
-                    al[h] = __uint_as_float(__float_as_uint(a) | (pos ? 0u : NEG_FLAG));
-                }
-                reinterpret_cast<float4*>(alpha_used + int64_t(base + lane) * eg_ld)[k] = make_float4(al[0], al[1], al[2], al[3]);
-            }
-        }
-        cp_async_wait_all();
-        __syncwarp();
-        for (int t = 0; t < n; ++t) {
-            float g[VW];
-#pragma unroll
-            for (int k = 0; k < VW; k += 4) {
-                const float4 tv = *reinterpret_cast<const float4*>(do_s + t * C + cm + k);
-                g[k] = tv.x * sc; g[k + 1] = tv.y * sc; g[k + 2] = tv.z * sc; g[k + 3] = tv.w * sc;
-            }
-            float d[NS];
-#pragma unroll
-            for (int q = 0; q < NS; ++q) {
-                d[q] = 0.f;
-#pragma unroll
-                for (int k = 0; k < VW; ++k) d[q] = fmaf(g[k], v[q][k], d[q]);
-            }
-            dalpha_reduce<GE>(d, dal_s + t * H, lane);
-        }
-        __syncwarp();
-        if (lane < n) {
-            float dal[H];
-#pragma unroll
-            for (int k = 0; k < H / 4; ++k) {
-                const float4 d4 = *reinterpret_cast<const float4*>(dal_s + lane * H + 4 * k);
-                dal[4 * k] = d4.x; dal[4 * k + 1] = d4.y; dal[4 * k + 2] = d4.z; dal[4 * k + 3] = d4.w;
-            }
-            store_vecH<H>(dz + int64_t(base + lane) * eg_ld, dal);
-        }
-        __syncwarp();
+    constexpr int C = GE::C, LPR = C / 4, RPI = 32 / LPR;
+    const int sub = lane / LPR, c4 = 4 * (lane % LPR);
+    for (int r = 0; r < n; r += RPI) {
+        const int ir = __shfl_sync(FULL, i, (r + sub) & 31);
+        if (r + sub < n) cp_async16(do_s + ((first + r + sub) % SLOTS) * C + c4, d_out + int64_t(ir) * C + c4);
     }
 }
-
-// one warp per edge-balanced work item over colptr (a run of whole source rows); hub rows are left to _hub
+// d_alpha of one edge against the dO row staged at g_row: phase B's FMAs and butterfly, result in dal_t[0..H)
 template <class GE>
-__global__ void __launch_bounds__(DA_THREADS, 6)
-gat_bwd_dalpha_src_rows(const int32_t* __restrict__ colptr, const int32_t* __restrict__ csc_row,
-                        const typename GE::XT* __restrict__ xw, const float* __restrict__ a_src,
-                        const float* __restrict__ a_dst, const float* __restrict__ rowmax,
-                        const float* __restrict__ rowsum, const float* __restrict__ d_out, gnnfd_item_plan_t items,
-                        int hub_threshold, float slope, float* __restrict__ alpha_used, float* __restrict__ dz,
-                        int64_t eg_ld)
+__device__ __forceinline__ void dalpha_edge(const float (&v)[GE::NS][GE::VW], const float* g_row, float* dal_t, int lane)
 {
-    __shared__ __align__(16) float do_sh[DA_WARPS][32 * GE::C];
-    __shared__ __align__(16) float dal_sh[DA_WARPS][32 * GE::H];
-    __shared__ int i_sh[DA_WARPS][32];
+    constexpr int NS = GE::NS, VW = GE::VW, C = GE::C, H = GE::H;
+    static_assert((32 * VW) % C == 0, "every slot of a lane must see the same dO channels");
+    const int cm = (VW * lane) % C;          // dO channels of this lane's slots
+    const float sc = 1.f / H;
+    float g[VW];
+#pragma unroll
+    for (int k = 0; k < VW; k += 4) {
+        const float4 tv = *reinterpret_cast<const float4*>(g_row + cm + k);
+        g[k] = tv.x * sc; g[k + 1] = tv.y * sc; g[k + 2] = tv.z * sc; g[k + 3] = tv.w * sc;
+    }
+    float d[NS];
+#pragma unroll
+    for (int q = 0; q < NS; ++q) {
+        d[q] = 0.f;
+#pragma unroll
+        for (int k = 0; k < VW; ++k) d[q] = fmaf(g[k], v[q][k], d[q]);
+    }
+    dalpha_reduce<GE>(d, dal_t, lane);
+}
+
+// one edge's d_alpha from shared memory to its CSR position
+template <int H>
+__device__ __forceinline__ void store_dalpha(float* __restrict__ dst, const float* dal_t)
+{
+    float dal[H];
+#pragma unroll
+    for (int k = 0; k < H / 4; ++k) {
+        const float4 d4 = *reinterpret_cast<const float4*>(dal_t + 4 * k);
+        dal[4 * k] = d4.x; dal[4 * k + 1] = d4.y; dal[4 * k + 2] = d4.z; dal[4 * k + 3] = d4.w;
+    }
+    store_vecH<H>(dst, dal);
+}
+
+// per-warp shared memory of the pass-1 stream
+template <class GE>
+struct DaGeo {
+    static constexpr int DO_BYTES = DA_RING * GE::C * 4;
+    static constexpr int XROW_BYTES = GE::D * int(sizeof(typename GE::XT));
+    static constexpr int X_BYTES = DA_XROWS * XROW_BYTES;
+    static constexpr int DAL_BYTES = 32 * GE::H * 4;
+    static constexpr int EID_BYTES = DA_RING * 4;
+    static constexpr int WARP_BYTES = ((DO_BYTES + X_BYTES + DAL_BYTES + EID_BYTES + 127) / 128) * 128;
+    static constexpr int CTA_BYTES = DA_WARPS * WARP_BYTES;
+};
+
+// one warp per edge-balanced work item over colptr (a run of whole source rows); hub rows are left to _hub.
+// A task is a chunk of <= 32 out-edges of one source row (ChunkCursor over colptr); it is issued once its edges fit
+// the dO ring, a task slot is free and, if it starts a new source row, an xw slot is free.  Lane k % DA_TASKS holds
+// task k as (n | new-row flag | xw slot).
+template <class GE>
+__global__ void __launch_bounds__(DA_THREADS, 4)
+gat_bwd_dalpha_src_stream(const int32_t* __restrict__ colptr, const int32_t* __restrict__ csc_row,
+                          const int32_t* __restrict__ csc_eid, const typename GE::XT* __restrict__ xw,
+                          const float* __restrict__ d_out, gnnfd_item_plan_t items, int hub_threshold,
+                          float* __restrict__ d_alpha)
+{
+    using SG = DaGeo<GE>;
+    constexpr int H = GE::H, NS = GE::NS, VW = GE::VW, C = GE::C;
+    extern __shared__ __align__(128) uint8_t smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int item = blockIdx.x * DA_WARPS + warp;
     if (item >= items.n_items) return;
-    const int j_end = items.item_start[item + 1];
-    for (int64_t j = items.item_start[item]; j < j_end; ++j) {
-        const int beg = colptr[j], end = colptr[j + 1];
-        if (end == beg || end - beg > hub_threshold) continue;
-        dalpha_range<GE>(j, beg, end, csc_row, xw, a_src, a_dst, rowmax, rowsum, d_out, slope, alpha_used, dz, eg_ld,
-                         do_sh[warp], dal_sh[warp], i_sh[warp], lane);
+    uint8_t* base = smem + warp * SG::WARP_BYTES;
+    float* do_s = reinterpret_cast<float*>(base);
+    uint8_t* x_s = base + SG::DO_BYTES;
+    float* dal_s = reinterpret_cast<float*>(base + SG::DO_BYTES + SG::X_BYTES);
+    int* eid_s = reinterpret_cast<int*>(base + SG::DO_BYTES + SG::X_BYTES + SG::DAL_BYTES);
+
+    ChunkCursor cur;
+    cur.start_rows(items.item_start[item], items.item_start[item + 1], hub_threshold);
+    auto no_empty = [](int) {};
+    int nj = 0, nbeg = 0, nn = 0;              // the next task not yet issued
+    bool nfirst = false, nlast = false;
+    bool have = cur.next(colptr, nj, nbeg, nn, nfirst, nlast, no_empty);
+    int e_issued = 0, e_done = 0;              // edges through the dO ring
+    int t_issued = 0, t_done = 0;              // tasks
+    int x_issued = 0, x_done = 0;              // xw rows
+    int task = 0;                              // this lane's entry of the task queue
+    auto issue = [&]() {
+        while (have && e_issued - e_done + nn <= DA_RING && t_issued - t_done < DA_TASKS &&
+               (!nfirst || x_issued - x_done < DA_XROWS)) {
+            const bool live = lane < nn;
+            const int i = live ? csc_row[nbeg + lane] : 0;
+            if (live) eid_s[(e_issued + lane) % DA_RING] = csc_eid[nbeg + lane];
+            copy_do_rows<GE, DA_RING>(do_s, e_issued, nn, i, d_out, lane);
+            const int xs = x_issued % DA_XROWS;
+            if (nfirst) {
+                const uint8_t* src = reinterpret_cast<const uint8_t*>(xw + int64_t(nj) * GE::D);
+#pragma unroll
+                for (int q = 0; q < NS; ++q)
+                    cp_async16(x_s + xs * SG::XROW_BYTES + (lane + 32 * q) * 16, src + (lane + 32 * q) * 16);
+                ++x_issued;
+            }
+            cp_async_commit();
+            if (lane == t_issued % DA_TASKS) task = nn | (int(nfirst) << 6) | (xs << 7);
+            e_issued += nn;
+            ++t_issued;
+            have = cur.next(colptr, nj, nbeg, nn, nfirst, nlast, no_empty);
+        }
+    };
+    issue();
+    float v[NS][VW];                           // xw row of the current source, slot layout
+    while (t_done < t_issued) {
+        cp_async_wait_pending(t_issued - t_done - 1);
+        __syncwarp();
+        const int tk = __shfl_sync(FULL, task, t_done % DA_TASKS);
+        const int n = tk & 63;
+        if (tk & 64) {
+#pragma unroll
+            for (int q = 0; q < NS; ++q) lds_slot(x_s + (tk >> 7) * SG::XROW_BYTES, q, lane, v[q]);
+            ++x_done;
+        }
+        for (int t = 0; t < n; ++t) dalpha_edge<GE>(v, do_s + ((e_done + t) % DA_RING) * C, dal_s + t * H, lane);
+        __syncwarp();
+        if (lane < n) store_dalpha<H>(d_alpha + int64_t(eid_s[(e_done + lane) % DA_RING]) * H, dal_s + lane * H);
+        __syncwarp();                          // the task's slots are read before they are refilled
+        e_done += n;
+        ++t_done;
+        issue();
     }
 }
 
-// one warp per chunk of a hub source row
+// one warp per chunk of a hub source row: xw[j] in registers, per 32 edges the dO rows staged with cp.async
 template <class GE>
 __global__ void __launch_bounds__(DA_THREADS, 6)
 gat_bwd_dalpha_src_hub(const int32_t* __restrict__ colptr, const int32_t* __restrict__ csc_row,
-                       const typename GE::XT* __restrict__ xw, const float* __restrict__ a_src,
-                       const float* __restrict__ a_dst, const float* __restrict__ rowmax,
-                       const float* __restrict__ rowsum, const float* __restrict__ d_out, gnnfd_hub_plan_t plan,
-                       float slope, float* __restrict__ alpha_used, float* __restrict__ dz, int64_t eg_ld)
+                       const int32_t* __restrict__ csc_eid, const typename GE::XT* __restrict__ xw,
+                       const float* __restrict__ d_out, gnnfd_hub_plan_t plan, float* __restrict__ d_alpha)
 {
-    __shared__ __align__(16) float do_sh[DA_WARPS][32 * GE::C];
-    __shared__ __align__(16) float dal_sh[DA_WARPS][32 * GE::H];
-    __shared__ int i_sh[DA_WARPS][32];
+    constexpr int H = GE::H, NS = GE::NS, VW = GE::VW, C = GE::C;
+    __shared__ __align__(16) float do_sh[DA_WARPS][32 * C];
+    __shared__ __align__(16) float dal_sh[DA_WARPS][32 * H];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int c = blockIdx.x * DA_WARPS + warp;
     if (c >= plan.n_chunk) return;
@@ -170,40 +216,94 @@ gat_bwd_dalpha_src_hub(const int32_t* __restrict__ colptr, const int32_t* __rest
     const int64_t j = plan.hub_row[slot];
     const int beg = colptr[j] + (c - plan.hub_chunk_ptr[slot]) * plan.chunk;
     const int end = min(colptr[j + 1], beg + plan.chunk);
-    dalpha_range<GE>(j, beg, end, csc_row, xw, a_src, a_dst, rowmax, rowsum, d_out, slope, alpha_used, dz, eg_ld,
-                     do_sh[warp], dal_sh[warp], i_sh[warp], lane);
+    float* do_s = do_sh[warp];
+    float* dal_s = dal_sh[warp];
+    float v[NS][VW];
+#pragma unroll
+    for (int q = 0; q < NS; ++q) load_slot(xw + j * GE::D, q, lane, v[q]);
+    for (int base = beg; base < end; base += 32) {
+        const int n = min(32, end - base);
+        const bool live = lane < n;
+        const int i = live ? csc_row[base + lane] : 0;
+        const int eid = live ? csc_eid[base + lane] : 0;
+        copy_do_rows<GE, 32>(do_s, 0, n, i, d_out, lane);
+        cp_async_commit();
+        cp_async_wait_pending(0);
+        __syncwarp();
+        for (int t = 0; t < n; ++t) dalpha_edge<GE>(v, do_s + t * C, dal_s + t * H, lane);
+        __syncwarp();
+        if (live) store_dalpha<H>(d_alpha + int64_t(eid) * H, dal_s + lane * H);
+        __syncwarp();
+    }
 }
 
 // ---------------------------------------------------------------------------------------------------------
 // pass 2: feature-free dst-major reductions
 // ---------------------------------------------------------------------------------------------------------
-// pass 1's slot of one edge, lane = edge.  The slot is read here and overwritten later by the same thread, so
-// plain (coherent) loads are used.
+// one edge of pass 2, lane = edge
 template <int H>
 struct EgEdge {
     float a[H], d[H];      // alpha with the LeakyReLU-negative flag, d_alpha
     int pos;               // source-major slot
     unsigned keep;         // dropout keep bits
 };
+// pass 2 reads an edge in two steps so that the next chunk's contiguous loads are in flight while the current chunk
+// is reduced: eg_fetch (col, csr2csc, d_alpha, perm of dst-sorted edge e), then eg_finish (the row statistics of its
+// destination row, the one gather a_src[col[e]], alpha recomputed as phase A does, the keep bits)
+template <int H>
+struct EgRaw {
+    int j, pos, pe;
+    float d[H];
+};
 template <int H, bool DROPOUT>
-__device__ __forceinline__ void eg_load(EgEdge<H>& x, int e, bool live, const int32_t* __restrict__ perm,
-                                        const int32_t* __restrict__ csr2csc, KeepMask keep,
-                                        const float* alpha_used, const float* dz, int64_t eg_ld)
+__device__ __forceinline__ void eg_fetch(EgRaw<H>& r, int e, bool live, const int32_t* __restrict__ col,
+                                         const int32_t* __restrict__ perm, const int32_t* __restrict__ csr2csc,
+                                         const float* __restrict__ d_alpha)
 {
-    x.pos = 0;
+    r.j = r.pos = r.pe = 0;
+#pragma unroll
+    for (int h = 0; h < H; ++h) r.d[h] = 0.f;
+    if (!live) return;
+    r.j = col[e];
+    r.pos = csr2csc[e];
+    load_vecH<H>(d_alpha + int64_t(e) * H, r.d);
+    if (DROPOUT) r.pe = perm[e];
+}
+template <int H, bool DROPOUT>
+__device__ __forceinline__ void eg_finish(EgEdge<H>& x, const EgRaw<H>& r, bool live, int64_t row,
+                                          const float* __restrict__ a_src, const float* __restrict__ a_dst,
+                                          const float* __restrict__ rowmax, const float* __restrict__ rowsum,
+                                          float slope, KeepMask keep)
+{
+    x.pos = r.pos;
     x.keep = 0xffu;
 #pragma unroll
-    for (int h = 0; h < H; ++h) x.a[h] = x.d[h] = 0.f;
-    if (!live) return;
-    x.pos = csr2csc[e];
-#pragma unroll
-    for (int k = 0; k < H / 4; ++k) {
-        const float4 a4 = reinterpret_cast<const float4*>(alpha_used + int64_t(x.pos) * eg_ld)[k];
-        const float4 d4 = reinterpret_cast<const float4*>(dz + int64_t(x.pos) * eg_ld)[k];
-        x.a[4 * k] = a4.x; x.a[4 * k + 1] = a4.y; x.a[4 * k + 2] = a4.z; x.a[4 * k + 3] = a4.w;
-        x.d[4 * k] = d4.x; x.d[4 * k + 1] = d4.y; x.d[4 * k + 2] = d4.z; x.d[4 * k + 3] = d4.w;
+    for (int h = 0; h < H; ++h) {
+        x.a[h] = 0.f;
+        x.d[h] = r.d[h];
     }
-    if (DROPOUT) x.keep = keep.bits(perm[e], H);
+    if (!live) return;
+    RowStat<H> st;
+    load_row_stat<H>(st, row, a_dst, rowmax, rowsum);
+    float as[H];
+    load_vecH<H>(a_src + int64_t(r.j) * H, as);
+#pragma unroll
+    for (int h = 0; h < H; ++h) {
+        const float z = as[h] + st.adst[h];
+        x.a[h] = __uint_as_float(__float_as_uint(edge_alpha(z, slope, st.m[h], st.inv[h])) | (z > 0.f ? 0u : NEG_FLAG));
+    }
+    if (DROPOUT) x.keep = keep.bits(r.pe, H);
+}
+template <int H, bool DROPOUT>
+__device__ __forceinline__ void eg_load(EgEdge<H>& x, int e, bool live, int64_t row, const int32_t* __restrict__ col,
+                                        const int32_t* __restrict__ perm, const int32_t* __restrict__ csr2csc,
+                                        const float* __restrict__ a_src, const float* __restrict__ a_dst,
+                                        const float* __restrict__ rowmax, const float* __restrict__ rowsum, float slope,
+                                        KeepMask keep, const float* __restrict__ d_alpha)
+{
+    EgRaw<H> r;
+    eg_fetch<H, DROPOUT>(r, e, live, col, perm, csr2csc, d_alpha);
+    eg_finish<H, DROPOUT>(x, r, live, row, a_src, a_dst, rowmax, rowsum, slope, keep);
 }
 // head h of an edge, phase C's arithmetic: pre-dropout alpha, LeakyReLU slope, keep scale, u = alpha * d_alpha * keep
 struct EgHead {
@@ -232,16 +332,20 @@ __device__ __forceinline__ void eg_store(const EgEdge<H>& x, const float (&o)[H]
     store_vecH<H>(alpha_used + int64_t(x.pos) * eg_ld, au);
     store_vecH<H>(dz + int64_t(x.pos) * eg_ld, o);
 }
-// second sweep of a row (or hub chunk) whose t is known: final alpha_used and dz into the slots, lane-local da_dst
+// second sweep of a row (or hub chunk) whose t is known: the edges are loaded again, alpha_used and dz go to the
+// slots, da_dst is summed lane-locally
 template <int H, bool DROPOUT>
-__device__ __forceinline__ void eg_sweep2(int beg, int end, const int32_t* __restrict__ perm,
-                                          const int32_t* __restrict__ csr2csc, KeepMask keep, float keep_scale,
-                                          float slope, const float (&t)[H], float* alpha_used, float* dz,
+__device__ __forceinline__ void eg_sweep2(int64_t row, int beg, int end, const int32_t* __restrict__ col,
+                                          const int32_t* __restrict__ perm, const int32_t* __restrict__ csr2csc,
+                                          const float* __restrict__ a_src, const float* __restrict__ a_dst,
+                                          const float* __restrict__ rowmax, const float* __restrict__ rowsum,
+                                          KeepMask keep, float keep_scale, float slope, const float (&t)[H],
+                                          const float* __restrict__ d_alpha, float* alpha_used, float* dz,
                                           int64_t eg_ld, float (&dad)[H], int lane)
 {
     for (int e = beg + lane; e < end; e += 32) {
         EgEdge<H> x;
-        eg_load<H, DROPOUT>(x, e, true, perm, csr2csc, keep, alpha_used, dz, eg_ld);
+        eg_load<H, DROPOUT>(x, e, true, row, col, perm, csr2csc, a_src, a_dst, rowmax, rowsum, slope, keep, d_alpha);
         float o[H];
 #pragma unroll
         for (int h = 0; h < H; ++h) {
@@ -254,11 +358,14 @@ __device__ __forceinline__ void eg_sweep2(int beg, int end, const int32_t* __res
 }
 
 // one warp per edge-balanced work item over rowptr; the chunk and pack sequence of gat_bwd_dst_items_pack, with the
-// next chunk's slots loaded while the current one is reduced
+// next chunk's contiguous loads (eg_fetch) in flight while the current one is finished and reduced
 template <int H, bool DROPOUT>
 __global__ void __launch_bounds__(ROW_THREADS, 2)
-gat_bwd_dst_eg_items(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ perm,
-                     const int32_t* __restrict__ csr2csc, gnnfd_item_plan_t items, int hub_threshold, float slope,
+gat_bwd_dst_eg_items(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
+                     const int32_t* __restrict__ perm, const int32_t* __restrict__ csr2csc,
+                     const float* __restrict__ a_src, const float* __restrict__ a_dst,
+                     const float* __restrict__ rowmax, const float* __restrict__ rowsum,
+                     const float* __restrict__ d_alpha, gnnfd_item_plan_t items, int hub_threshold, float slope,
                      KeepMask keep, float keep_scale, float* alpha_used, float* dz, int64_t eg_ld,
                      float* __restrict__ da_dst)
 {
@@ -271,21 +378,24 @@ gat_bwd_dst_eg_items(const int32_t* __restrict__ rowptr, const int32_t* __restri
         if (lane < H) da_dst[int64_t(r) * H + lane] = 0.f;
     };
     BwdChunk c0, c1;
-    int k0 = 0, k1 = 0, la = 0, lb = 0, lo = 0;
+    int k0 = 0, k1 = 0, la = 0, lb = 0, lo0 = 0, lo1 = 0;
     int sa0 = 0, sb0 = 0, sa1 = 0, sb1 = 0;
     int kind0 = cur.next_any(rowptr, lane, c0.row, c0.beg, c0.n, c0.first, c0.last, k0, la, lb, on_empty);
     if (!kind0) return;
-    if (kind0 == 2) pack_lane_segment(c0.beg, k0, la, lb, lane, lo, sa0, sb0);
-    EgEdge<H> x0, x1;
-    eg_load<H, DROPOUT>(x0, c0.beg + lane, lane < c0.n, perm, csr2csc, keep, alpha_used, dz, eg_ld);
+    if (kind0 == 2) pack_lane_segment(c0.beg, k0, la, lb, lane, lo0, sa0, sb0);
+    EgRaw<H> r0, r1;
+    eg_fetch<H, DROPOUT>(r0, c0.beg + lane, lane < c0.n, col, perm, csr2csc, d_alpha);
     float trow[H];               // running t = sum alpha*d_alpha of the current (multi-chunk) row
     int row_beg = c0.beg;        // first edge of the current row
 #pragma unroll
     for (int h = 0; h < H; ++h) trow[h] = 0.f;
     while (true) {
         const int kind1 = cur.next_any(rowptr, lane, c1.row, c1.beg, c1.n, c1.first, c1.last, k1, la, lb, on_empty);
-        if (kind1 == 2) pack_lane_segment(c1.beg, k1, la, lb, lane, lo, sa1, sb1);
-        if (kind1) eg_load<H, DROPOUT>(x1, c1.beg + lane, lane < c1.n, perm, csr2csc, keep, alpha_used, dz, eg_ld);
+        lo1 = 0;
+        if (kind1 == 2) pack_lane_segment(c1.beg, k1, la, lb, lane, lo1, sa1, sb1);
+        if (kind1) eg_fetch<H, DROPOUT>(r1, c1.beg + lane, lane < c1.n, col, perm, csr2csc, d_alpha);
+        EgEdge<H> x0;
+        eg_finish<H, DROPOUT>(x0, r0, lane < c0.n, c0.row + lo0, a_src, a_dst, rowmax, rowsum, slope, keep);
         if (c0.first) {
             row_beg = c0.beg;
 #pragma unroll
@@ -327,8 +437,8 @@ gat_bwd_dst_eg_items(const int32_t* __restrict__ rowptr, const int32_t* __restri
                 float dad[H];
 #pragma unroll
                 for (int h = 0; h < H; ++h) dad[h] = 0.f;
-                eg_sweep2<H, DROPOUT>(row_beg, c0.beg + c0.n, perm, csr2csc, keep, keep_scale, slope, trow, alpha_used, dz,
-                                      eg_ld, dad, lane);
+                eg_sweep2<H, DROPOUT>(c0.row, row_beg, c0.beg + c0.n, col, perm, csr2csc, a_src, a_dst, rowmax, rowsum,
+                                      keep, keep_scale, slope, trow, d_alpha, alpha_used, dz, eg_ld, dad, lane);
 #pragma unroll
                 for (int h = 0; h < H; ++h) dad[h] = warp_sum(dad[h]);
                 if (lane == 0) store_vecH<H>(da_dst + int64_t(c0.row) * H, dad);
@@ -340,17 +450,20 @@ gat_bwd_dst_eg_items(const int32_t* __restrict__ rowptr, const int32_t* __restri
         k0 = k1;
         sa0 = sa1;
         sb0 = sb1;
-        x0 = x1;
+        lo0 = lo1;
+        r0 = r1;
     }
 }
 
 // hub rows, step 1: one warp per chunk -- partial t of the chunk
 template <int H, bool DROPOUT>
 __global__ void __launch_bounds__(ROW_THREADS)
-gat_bwd_dst_eg_hub1(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ perm,
-                    const int32_t* __restrict__ csr2csc, gnnfd_hub_plan_t plan, float slope, KeepMask keep,
-                    float keep_scale, const float* alpha_used, const float* dz, int64_t eg_ld,
-                    float* __restrict__ part_t)
+gat_bwd_dst_eg_hub1(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
+                    const int32_t* __restrict__ perm, const int32_t* __restrict__ csr2csc,
+                    const float* __restrict__ a_src, const float* __restrict__ a_dst,
+                    const float* __restrict__ rowmax, const float* __restrict__ rowsum,
+                    const float* __restrict__ d_alpha, gnnfd_hub_plan_t plan, float slope, KeepMask keep,
+                    float keep_scale, float* __restrict__ part_t)
 {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int c = blockIdx.x * ROW_WARPS + warp;
@@ -365,7 +478,8 @@ gat_bwd_dst_eg_hub1(const int32_t* __restrict__ rowptr, const int32_t* __restric
     for (int base = beg; base < end; base += 32) {
         const bool live = base + lane < end;
         EgEdge<H> x;
-        eg_load<H, DROPOUT>(x, base + lane, live, perm, csr2csc, keep, alpha_used, dz, eg_ld);
+        eg_load<H, DROPOUT>(x, base + lane, live, i, col, perm, csr2csc, a_src, a_dst, rowmax, rowsum, slope, keep,
+                            d_alpha);
 #pragma unroll
         for (int h = 0; h < H; ++h) trow[h] += warp_sum(eg_head<H>(x, h, live, slope, keep_scale).u);
     }
@@ -375,8 +489,11 @@ gat_bwd_dst_eg_hub1(const int32_t* __restrict__ rowptr, const int32_t* __restric
 // hub rows, step 2: the row's total t (chunk order), second sweep, partial da_dst
 template <int H, bool DROPOUT>
 __global__ void __launch_bounds__(ROW_THREADS)
-gat_bwd_dst_eg_hub2(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ perm,
-                    const int32_t* __restrict__ csr2csc, gnnfd_hub_plan_t plan, float slope, KeepMask keep,
+gat_bwd_dst_eg_hub2(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
+                    const int32_t* __restrict__ perm, const int32_t* __restrict__ csr2csc,
+                    const float* __restrict__ a_src, const float* __restrict__ a_dst,
+                    const float* __restrict__ rowmax, const float* __restrict__ rowsum,
+                    const float* __restrict__ d_alpha, gnnfd_hub_plan_t plan, float slope, KeepMask keep,
                     float keep_scale, const float* __restrict__ t_total, float* alpha_used, float* dz, int64_t eg_ld,
                     float* __restrict__ part_dad)
 {
@@ -391,34 +508,53 @@ gat_bwd_dst_eg_hub2(const int32_t* __restrict__ rowptr, const int32_t* __restric
     load_vecH<H>(t_total + int64_t(slot) * H, t);
 #pragma unroll
     for (int h = 0; h < H; ++h) dad[h] = 0.f;
-    eg_sweep2<H, DROPOUT>(beg, end, perm, csr2csc, keep, keep_scale, slope, t, alpha_used, dz, eg_ld, dad, lane);
+    eg_sweep2<H, DROPOUT>(i, beg, end, col, perm, csr2csc, a_src, a_dst, rowmax, rowsum, keep, keep_scale, slope, t,
+                          d_alpha, alpha_used, dz, eg_ld, dad, lane);
 #pragma unroll
     for (int h = 0; h < H; ++h) dad[h] = warp_sum(dad[h]);
     if (lane == 0) store_vecH<H>(part_dad + int64_t(c) * H, dad);
 }
 
+struct EgArgs {
+    const float *a_src, *a_dst, *rowmax, *rowsum, *d_alpha;
+};
 template <class GE, bool DROPOUT>
-static void launch_dst_eg(const gnnfd_graph_t* g, float slope, KeepMask keep, float ks, float* alpha_used, float* dz,
-                          int64_t eg_ld, float* da_dst, float* part_t, float* part_dad, float* t_total, cudaStream_t st)
+static void launch_dst_eg(const gnnfd_graph_t* g, const EgArgs& in, float slope, KeepMask keep, float ks,
+                          float* alpha_used, float* dz, int64_t eg_ld, float* da_dst, float* part_t, float* part_dad,
+                          float* t_total, cudaStream_t st)
 {
     constexpr int H = GE::H;
     const int thr = g->hub_dst.n_hub > 0 ? g->hub_dst.threshold : INT_MAX;
     const unsigned grid = (unsigned)((g->items_dst.n_items + ROW_WARPS - 1) / ROW_WARPS);
-    gat_bwd_dst_eg_items<H, DROPOUT><<<grid, ROW_THREADS, 0, st>>>(g->rowptr, g->perm, g->csr2csc, g->items_dst, thr,
-                                                                    slope, keep, ks, alpha_used, dz, eg_ld, da_dst);
+    gat_bwd_dst_eg_items<H, DROPOUT><<<grid, ROW_THREADS, 0, st>>>(g->rowptr, g->col, g->perm, g->csr2csc, in.a_src,
+                                                                    in.a_dst, in.rowmax, in.rowsum, in.d_alpha,
+                                                                    g->items_dst, thr, slope, keep, ks, alpha_used, dz,
+                                                                    eg_ld, da_dst);
     g_launches += 1;
     if (g->hub_dst.n_hub > 0) {
         const gnnfd_hub_plan_t& pl = g->hub_dst;
         const unsigned gh = (unsigned)((pl.n_hub + ROW_WARPS - 1) / ROW_WARPS);
         const unsigned gc = (unsigned)((pl.n_chunk + ROW_WARPS - 1) / ROW_WARPS);
-        gat_bwd_dst_eg_hub1<H, DROPOUT><<<gc, ROW_THREADS, 0, st>>>(g->rowptr, g->perm, g->csr2csc, pl, slope, keep, ks,
-                                                                     alpha_used, dz, eg_ld, part_t);
+        gat_bwd_dst_eg_hub1<H, DROPOUT><<<gc, ROW_THREADS, 0, st>>>(g->rowptr, g->col, g->perm, g->csr2csc, in.a_src,
+                                                                     in.a_dst, in.rowmax, in.rowsum, in.d_alpha, pl,
+                                                                     slope, keep, ks, part_t);
         gat_hub_chunk_sum<H, false><<<gh, ROW_THREADS, 0, st>>>(pl, part_t, t_total);
-        gat_bwd_dst_eg_hub2<H, DROPOUT><<<gc, ROW_THREADS, 0, st>>>(g->rowptr, g->perm, g->csr2csc, pl, slope, keep, ks,
-                                                                     t_total, alpha_used, dz, eg_ld, part_dad);
+        gat_bwd_dst_eg_hub2<H, DROPOUT><<<gc, ROW_THREADS, 0, st>>>(g->rowptr, g->col, g->perm, g->csr2csc, in.a_src,
+                                                                     in.a_dst, in.rowmax, in.rowsum, in.d_alpha, pl,
+                                                                     slope, keep, ks, t_total, alpha_used, dz, eg_ld,
+                                                                     part_dad);
         gat_hub_chunk_sum<H, true><<<gh, ROW_THREADS, 0, st>>>(pl, part_dad, da_dst);
         g_launches += 4;
     }
+}
+
+// workspace of the two-pass form: d_alpha [E',H] in CSR order, then the hub_dst partials
+size_t gat_bwd_dst_srcmajor_ws_bytes(const gnnfd_graph_t* g, int H)
+{
+    size_t b = carve_bytes(size_t(g->n_edges) * H, 4);
+    if (g->hub_dst.n_hub > 0)
+        b += 2 * carve_bytes(size_t(g->hub_dst.n_chunk) * H, 4) + carve_bytes(size_t(g->hub_dst.n_hub) * H, 4);
+    return b;
 }
 
 template <class GE>
@@ -435,44 +571,49 @@ static int launch_bwd_dst_srcmajor(const gnnfd_graph_t* g, const void* xw_, cons
                   "gat_bwd_dst: the graph has no work-item plan over rowptr (gnnfd_item_plan)");
     // two dense [E',H] arrays, or the halves of one interleaved [E',2H] buffer (dz == alpha_used + H)
     const int64_t eg_ld = (dz == alpha_used + H) ? 2 * H : H;
+    const size_t need = gat_bwd_dst_srcmajor_ws_bytes(g, H);
+    GNNFD_REQUIRE(ws && ws_bytes >= need, GNNFD_ERR_WORKSPACE, "gat_bwd_dst: workspace %zu < %zu", ws_bytes, need);
+    char* p = reinterpret_cast<char*>(ws);
+    float* d_alpha = carve<float>(p, size_t(g->n_edges) * H);
     float *part_t = nullptr, *part_dad = nullptr, *t_total = nullptr;
     if (g->hub_dst.n_hub > 0) {
         const gnnfd_hub_plan_t& pl = g->hub_dst;
-        const size_t need = 2 * carve_bytes(size_t(pl.n_chunk) * H, 4) + carve_bytes(size_t(pl.n_hub) * H, 4);
-        GNNFD_REQUIRE(ws && ws_bytes >= need, GNNFD_ERR_WORKSPACE, "gat_bwd_dst: workspace %zu < %zu", ws_bytes, need);
-        char* p = reinterpret_cast<char*>(ws);
         part_t = carve<float>(p, size_t(pl.n_chunk) * H);
         part_dad = carve<float>(p, size_t(pl.n_chunk) * H);
         t_total = carve<float>(p, size_t(pl.n_hub) * H);
     }
     if (g->n_edges > 0) {
+        constexpr int SMEM = DaGeo<GE>::CTA_BYTES;
+        GNNFD_CUDA(cudaFuncSetAttribute(gat_bwd_dalpha_src_stream<GE>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
         const int thr = g->hub_src.n_hub > 0 ? g->hub_src.threshold : INT_MAX;
         const unsigned grid = (unsigned)((g->items_src.n_items + DA_WARPS - 1) / DA_WARPS);
-        gat_bwd_dalpha_src_rows<GE><<<grid, DA_THREADS, 0, st>>>(g->colptr, g->csc_row, xw, a_src, a_dst, rowmax, rowsum,
-                                                                  d_out, g->items_src, thr, slope, alpha_used, dz, eg_ld);
+        gat_bwd_dalpha_src_stream<GE><<<grid, DA_THREADS, SMEM, st>>>(g->colptr, g->csc_row, g->csc_eid, xw, d_out,
+                                                                      g->items_src, thr, d_alpha);
         g_launches += 1;
         if (g->hub_src.n_hub > 0) {
             const unsigned gc = (unsigned)((g->hub_src.n_chunk + DA_WARPS - 1) / DA_WARPS);
-            gat_bwd_dalpha_src_hub<GE><<<gc, DA_THREADS, 0, st>>>(g->colptr, g->csc_row, xw, a_src, a_dst, rowmax,
-                                                                   rowsum, d_out, g->hub_src, slope, alpha_used, dz, eg_ld);
+            gat_bwd_dalpha_src_hub<GE><<<gc, DA_THREADS, 0, st>>>(g->colptr, g->csc_row, g->csc_eid, xw, d_out,
+                                                                   g->hub_src, d_alpha);
             g_launches += 1;
         }
     }
     float ks = 1.f;
     const KeepMask keep = make_keep(keep_mask, p_drop, seed, &ks);
+    const EgArgs in{a_src, a_dst, rowmax, rowsum, d_alpha};
     if (p_drop > 0.f)
-        launch_dst_eg<GE, true>(g, slope, keep, ks, alpha_used, dz, eg_ld, da_dst, part_t, part_dad, t_total, st);
+        launch_dst_eg<GE, true>(g, in, slope, keep, ks, alpha_used, dz, eg_ld, da_dst, part_t, part_dad, t_total, st);
     else
-        launch_dst_eg<GE, false>(g, slope, keep, ks, alpha_used, dz, eg_ld, da_dst, part_t, part_dad, t_total, st);
+        launch_dst_eg<GE, false>(g, in, slope, keep, ks, alpha_used, dz, eg_ld, da_dst, part_t, part_dad, t_total, st);
     GNNFD_LAUNCH_CHECK();
     return GNNFD_OK;
 }
 
 // The two-pass backward applies to the head mean on a graph whose CSC positions are the edge-gradient slots
-// (not the indirect multi-GPU receive layout) and whose sources and destinations are one node set.
+// (not the indirect multi-GPU receive layout), whose CSC twin is complete (csc_eid included) and whose sources and
+// destinations are one node set.
 bool gat_bwd_dst_srcmajor_applies(const gnnfd_graph_t* g, int concat)
 {
-    return !concat && !g->edge_grads_indirect && g->n_src == g->n_dst && g->colptr && g->csc_row &&
+    return !concat && !g->edge_grads_indirect && g->n_src == g->n_dst && g->colptr && g->csc_row && g->csc_eid &&
            g->items_src.n_items > 0 && g->items_src.item_start;
 }
 

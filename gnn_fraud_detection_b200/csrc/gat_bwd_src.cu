@@ -15,6 +15,8 @@
 namespace gnnfd {
 extern std::atomic<long long> g_launches;
 int check_graph(const gnnfd_graph_t* g, bool need_csc, const char* who);
+bool gat_bwd_dst_srcmajor_applies(const gnnfd_graph_t* g, int concat);       // gat_bwd_dalpha.cu
+size_t gat_bwd_dst_srcmajor_ws_bytes(const gnnfd_graph_t* g, int H);
 
 #ifndef GNNFD_SRC_MINB
 #define GNNFD_SRC_MINB 4
@@ -294,7 +296,9 @@ int gnnfd_gat_bwd_workspace_bytes(const gnnfd_graph_t* g, int H, int C, size_t* 
 {
     GNNFD_REQUIRE(g && bytes, GNNFD_ERR_ARG, "gat_bwd_workspace_bytes: NULL argument");
     const size_t nd = (size_t)g->hub_dst.n_chunk, ns = (size_t)g->hub_src.n_chunk;
-    const size_t a = 2 * carve_bytes(nd * H, 4) + carve_bytes(size_t(g->hub_dst.n_hub) * H, 4);
+    // the dst pass: its two-pass form (head mean) also keeps d_alpha [E',H] here; concat is not known at this point
+    const size_t a = gat_bwd_dst_srcmajor_applies(g, 0) ? gat_bwd_dst_srcmajor_ws_bytes(g, H)
+                                                        : 2 * carve_bytes(nd * H, 4) + carve_bytes(size_t(g->hub_dst.n_hub) * H, 4);
     const size_t b = carve_bytes(ns * size_t(H) * C, 4) + carve_bytes(ns * H, 4);
     *bytes = (a > b ? a : b) + 256;
     return GNNFD_OK;

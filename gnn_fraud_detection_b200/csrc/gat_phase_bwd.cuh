@@ -25,6 +25,12 @@ __device__ __forceinline__ void load_row_stat(RowStat<H>& r, int64_t i, const fl
 #pragma unroll
     for (int h = 0; h < H; ++h) r.inv[h] = 1.f / st[h];
 }
+// alpha of one (edge, head) from its logit z and the row's saved max m and 1/sum inv.  Every backward kernel forms alpha
+// through this one expression, so that their alpha_used agree bit for bit.
+__device__ __forceinline__ float edge_alpha(float z, float slope, float m, float inv)
+{
+    return expf((z > 0.f ? z : z * slope) - m) * inv;
+}
 struct BwdChunk {
     int row, beg, n;
     bool first, last;
@@ -50,9 +56,8 @@ __device__ __forceinline__ void bwd_phase_a(const BwdChunk& c, const int32_t* __
 #pragma unroll
         for (int h = 0; h < H; ++h) {
             const float z = as[h] + r.adst[h];
-            const bool pos = z > 0.f;
-            bits |= int(pos) << h;
-            alpha[h] = expf((pos ? z : z * slope) - r.m[h]) * r.inv[h];
+            bits |= int(z > 0.f) << h;
+            alpha[h] = edge_alpha(z, slope, r.m[h], r.inv[h]);
         }
         if (DROPOUT) {
             bits |= int(keep.bits(perm[c.beg + lane], H)) << 8;
@@ -177,9 +182,8 @@ __device__ __forceinline__ void bwd_phase_a_pack(int row0, int beg, int n, int k
 #pragma unroll
         for (int h = 0; h < H; ++h) {
             const float z = as[h] + r.adst[h];
-            const bool pos = z > 0.f;
-            bits |= int(pos) << h;
-            alpha[h] = expf((pos ? z : z * slope) - r.m[h]) * r.inv[h];
+            bits |= int(z > 0.f) << h;
+            alpha[h] = edge_alpha(z, slope, r.m[h], r.inv[h]);
         }
         if (DROPOUT) {
             bits |= int(keep.bits(perm[e_id], H)) << 8;

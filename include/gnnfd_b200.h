@@ -223,7 +223,10 @@ int gnnfd_gat_alpha(const gnnfd_graph_t* g, const float* a_src, const float* a_d
  *   across GPUs, the exchange to the source owners) reads them contiguously -- and da_dst [n_dst,H].
  *   alpha_used and dz are either two dense [E',H] arrays or the two halves of ONE interleaved [E',2H]
  *   buffer (dz == alpha_used + H: 64 contiguous bytes per edge) -- the library recognises the latter from
- *   the pointers.  Needs the CSC twin and csr2csc.
+ *   the pointers.  Needs the CSC twin and csr2csc.  For the head mean (concat = 0) on a graph with the whole CSC twin
+ *   (colptr, csc_row, csc_eid), a source work-item plan, direct edge-gradient slots and n_src == n_dst, d_alpha is
+ *   computed source-major into an [E',H] fp32 buffer carved from ws (gnnfd_gat_bwd_workspace_bytes includes it; a smaller
+ *   ws returns GNNFD_ERR_WORKSPACE).
  * src-major pass (needs the CSC twin): dxw[j] = sum_e alpha_used*dO_h[i] + da_src[j]*att_src
  *   + da_dst_full[j]*att_dst, da_src[j] = sum_e dz.  da_dst_full is indexed by SOURCE id (for a single
  *   GPU it is the da_dst the dst pass produced; NULL => the att_dst term is skipped).
