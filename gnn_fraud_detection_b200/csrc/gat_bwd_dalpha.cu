@@ -608,14 +608,16 @@ static int launch_bwd_dst_srcmajor(const gnnfd_graph_t* g, const void* xw_, cons
     return GNNFD_OK;
 }
 
-// The two-pass backward applies to the head mean on a graph whose CSC positions are the edge-gradient slots
-// (not the indirect multi-GPU receive layout), whose CSC twin is complete (csc_eid included) and whose sources and
-// destinations are one node set.
-bool gat_bwd_dst_srcmajor_applies(const gnnfd_graph_t* g, int concat)
+// The source-major head-mean passes -- this two-pass backward and the three-pass forward (gat_fwd_msg.cu) -- apply to
+// the head mean on a graph whose CSC positions are the edge-gradient slots (not the indirect multi-GPU receive layout),
+// whose CSC twin is complete (csc_eid included) with a work-item plan over colptr, and whose sources and destinations
+// are one node set.
+bool gat_srcmajor_applies(const gnnfd_graph_t* g, int concat)
 {
     return !concat && !g->edge_grads_indirect && g->n_src == g->n_dst && g->colptr && g->csc_row && g->csc_eid &&
            g->items_src.n_items > 0 && g->items_src.item_start;
 }
+bool gat_bwd_dst_srcmajor_applies(const gnnfd_graph_t* g, int concat) { return gat_srcmajor_applies(g, concat); }
 
 int gat_bwd_dst_srcmajor(const gnnfd_graph_t* g, const void* xw, int xw_dtype, int H, int C, const float* a_src,
                          const float* a_dst, const float* rowmax, const float* rowsum, const float* d_out,

@@ -21,23 +21,12 @@
 
 namespace gnnfd {
 extern std::atomic<long long> g_launches;
-
-// Fused row epilogue:  v = mean/concat + bias;  v = v*scale + shift (folded eval-mode BatchNorm, optional);
-// v = act(v);  v += residual[row] (optional).  Mirrors gat.py:80-91 in eval mode (BatchNorm -> ReLU -> residual).
-struct EpiParams {
-    const float* bias;
-    const float* scale;
-    const float* shift;
-    const float* residual;
-    int act;
-};
-
-__device__ __forceinline__ float apply_act(float v, int act)
-{
-    if (act == GNNFD_ACT_RELU) return fmaxf(v, 0.f);
-    if (act == GNNFD_ACT_ELU) return v > 0.f ? v : expm1f(v);
-    return v;
-}
+// the source-major head-mean forward (gat_fwd_msg.cu)
+bool gat_fwd_srcmajor_applies(const gnnfd_graph_t* g, int concat);
+size_t gat_fwd_srcmajor_ws_bytes(const gnnfd_graph_t* g, int H, int C);
+int gat_fwd_srcmajor(const gnnfd_graph_t* g, const void* xw, int xw_dtype, int H, int C, const float* a_src,
+                     const float* a_dst, const EpiParams& ep, float negative_slope, const uint8_t* keep_mask, float p_drop,
+                     uint64_t seed, float* out, float* rowmax, float* rowsum, void* ws, size_t ws_bytes, cudaStream_t st);
 
 // normalise by the softmax denominator, save the row statistics, head mean/concat + bias + activation
 template <class GE, bool CONCAT>
@@ -70,13 +59,7 @@ __device__ __forceinline__ void fwd_epilogue(int64_t i, const float (&m)[GE::H],
             const int c0 = VW * (lane + 32 * q);
             float r[VW];
 #pragma unroll
-            for (int k = 0; k < VW; ++k) {
-                float v = acc[q][k] + (ep.bias ? ep.bias[c0 + k] : 0.f);
-                if (ep.scale) v = fmaf(v, ep.scale[c0 + k], ep.shift[c0 + k]);
-                v = apply_act(v, ep.act);
-                if (ep.residual) v += ep.residual[i * D + c0 + k];
-                r[k] = v;
-            }
+            for (int k = 0; k < VW; ++k) r[k] = epi_value(acc[q][k], c0 + k, i, D, ep);
 #pragma unroll
             for (int k = 0; k < VW; k += 4)
                 stg_stream(reinterpret_cast<float4*>(out + i * D + c0 + k), make_float4(r[k], r[k + 1], r[k + 2], r[k + 3]));
@@ -94,13 +77,7 @@ __device__ __forceinline__ void fwd_epilogue(int64_t i, const float (&m)[GE::H],
         if (sub == 0) {
             const int c0 = VW * lane;  // lane < G here
 #pragma unroll
-            for (int k = 0; k < VW; ++k) {
-                float v = r[k] * (1.f / H) + (ep.bias ? ep.bias[c0 + k] : 0.f);
-                if (ep.scale) v = fmaf(v, ep.scale[c0 + k], ep.shift[c0 + k]);
-                v = apply_act(v, ep.act);
-                if (ep.residual) v += ep.residual[i * C + c0 + k];
-                r[k] = v;
-            }
+            for (int k = 0; k < VW; ++k) r[k] = epi_value(r[k] * (1.f / H), c0 + k, i, C, ep);   // 1/H: exact
 #pragma unroll
             for (int k = 0; k < VW; k += 4)
                 stg_stream(reinterpret_cast<float4*>(out + i * C + c0 + k), make_float4(r[k], r[k + 1], r[k + 2], r[k + 3]));
@@ -647,6 +624,8 @@ int gnnfd_gat_fwd_workspace_bytes(const gnnfd_graph_t* g, int H, int C, size_t* 
     GNNFD_REQUIRE(g && bytes, GNNFD_ERR_ARG, "gat_fwd_workspace_bytes: NULL argument");
     const size_t nc = (size_t)g->hub_dst.n_chunk;
     *bytes = carve_bytes(nc * 2 * H, 4) + carve_bytes(nc * size_t(H) * C, 4) + 256;
+    // the source-major head-mean form also keeps alpha_used [E',H] and the messages [E',C] here; concat is not known
+    if (gat_fwd_srcmajor_applies(g, 0)) *bytes += gat_fwd_srcmajor_ws_bytes(g, H, C);
     return GNNFD_OK;
 }
 
@@ -668,6 +647,9 @@ int gnnfd_gat_fwd_fused(const gnnfd_graph_t* g, const void* xw, int xw_dtype, co
                   "gat_fwd: post_scale and post_shift must be given together");
     cudaStream_t st = (cudaStream_t)stream;
     const EpiParams ep{bias, post_scale, post_shift, residual, act};
+    if (gat_fwd_srcmajor_applies(g, concat))
+        return gat_fwd_srcmajor(g, xw, xw_dtype, H, C, a_src, a_dst, ep, negative_slope, keep_mask, p_drop, dropout_seed, out,
+                                rowmax, rowsum, ws, ws_bytes, st);
     if (H == 8 && C == 64 && xw_dtype == GNNFD_F32)
         return launch_fwd<Geo<8, 64, float>>(g, xw, a_src, a_dst, ep, negative_slope, concat, keep_mask, p_drop, dropout_seed, out, rowmax,
                                              rowsum, ws, ws_bytes, st);

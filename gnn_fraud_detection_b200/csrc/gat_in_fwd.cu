@@ -13,6 +13,7 @@
 // chunks whose partial sums are added in chunk order (deterministic).
 #include "in_common.cuh"
 #include "gat_stream.cuh"
+#include "gat_alpha.cuh"
 
 #ifndef GNNFD_IN_UNROLL_FWD
 #define GNNFD_IN_UNROLL_FWD 1     // the row epilogue (image write) sits inside the edge loop: unrolling it 4x thrashes the i-cache
@@ -272,163 +273,22 @@ __device__ __forceinline__ void acc_zero(float2 (&acc)[NA])
 // that the logit was in LeakyReLU's negative region (the backward needs that and nothing else of the logits), and
 // jflag[e] = col[e] | (e is the last edge of its row) << 31.  The feature passes (forward and backward) then stream
 // edges without any softmax state: no logit gathers, no exp, no scans, no row statistics in their registers.
-// Warp per work item as everywhere; lane = edge.  Rows of <= 32 edges (alone or in packs) are finished from registers;
-// longer rows make a statistics sweep and a write sweep (the re-gathered logits are L2-warm); hub rows get the same
-// two sweeps chunk-parallel (in_alpha_hub_*).
+// The kernels run the attention pass of gat_alpha.cuh (PROJ = false) at H = 8, without dropout: the feature passes apply it.
 // =====================================================================================================================
-__device__ __forceinline__ float with_sign(float a, bool neg) { return __uint_as_float(__float_as_uint(a) | (neg ? 0x80000000u : 0u)); }
-
-// the write sweep of <= 32 edges of ONE row whose statistics (m, 1/s) are known
-__device__ __forceinline__ void alpha_write_chunk(int beg, int n, bool ends_row, const float (&adst)[H], const float (&m)[H],
-                                                  const float (&sinv)[H], const int32_t* __restrict__ col,
-                                                  const float* __restrict__ a_src, float slope, float* __restrict__ alpha,
-                                                  int32_t* __restrict__ jflag, int lane)
-{
-    if (lane < n) {
-        const int e = beg + lane, j = col[e];
-        float as[H], o[H];
-        load_vecH<H>(a_src + int64_t(j) * H, as);
-#pragma unroll
-        for (int h = 0; h < H; ++h) {
-            const float z = as[h] + adst[h];
-            o[h] = with_sign(expf(leaky(z, slope) - m[h]) * sinv[h], !(z > 0.f));
-        }
-        store_vecH<H>(alpha + int64_t(e) * H, o);
-        jflag[e] = j | ((ends_row && lane == n - 1) ? int(0x80000000u) : 0);
-    }
-}
-
-// statistics of <= 32 edges of one row folded into the running (m, s) of the row (all lanes hold the result)
-__device__ __forceinline__ void alpha_stat_chunk(int beg, int n, const float (&adst)[H], const int32_t* __restrict__ col,
-                                                 const float* __restrict__ a_src, float slope, float (&m)[H], float (&s)[H], int lane)
-{
-    float e[H];
-    if (lane < n) {
-        const int j = col[beg + lane];
-        float as[H];
-        load_vecH<H>(a_src + int64_t(j) * H, as);
-#pragma unroll
-        for (int h = 0; h < H; ++h) e[h] = leaky(as[h] + adst[h], slope);
-    } else {
-#pragma unroll
-        for (int h = 0; h < H; ++h) e[h] = -INFINITY;
-    }
-#pragma unroll
-    for (int h = 0; h < H; ++h) {
-        const float cm = warp_max(e[h]);
-        const float cs = warp_sum(lane < n ? expf(e[h] - cm) : 0.f);
-        const float mn = fmaxf(m[h], cm);
-        s[h] = s[h] * expf(m[h] - mn) + cs * expf(cm - mn);       // expf(-inf) = 0 on the first chunk
-        m[h] = mn;
-    }
-}
-
 template <bool PACK>
 __global__ void __launch_bounds__(IN_THREADS)
 in_alpha_items(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col, const float* __restrict__ a_src,
                const float* __restrict__ a_dst, gnnfd_item_plan_t items, int hub_threshold, float slope,
-               float* __restrict__ alpha, int32_t* __restrict__ jflag, float* __restrict__ rowmax, float* __restrict__ rowsum)
+               AlphaOut out, float* __restrict__ rowmax, float* __restrict__ rowsum)
 {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int item = blockIdx.x * IN_WARPS + warp;
     if (item >= items.n_items) return;
-    ChunkCursor cur;
-    cur.start_rows(items.item_start[item], items.item_start[item + 1], hub_threshold);
-    auto on_empty = [&](int r) {
-        if (lane < H) {
-            rowmax[int64_t(r) * H + lane] = 0.f;
-            rowsum[int64_t(r) * H + lane] = 1e-16f;
-        }
-    };
-    int row = 0, beg = 0, n = 0, k = 0, la = 0, lb = 0;
-    bool first = false, last = false;
-    while (true) {
-        const int kind = PACK ? cur.next_any(rowptr, lane, row, beg, n, first, last, k, la, lb, on_empty)
-                              : (cur.next(rowptr, row, beg, n, first, last, on_empty) ? 1 : 0);
-        if (!kind) break;
-        if (PACK && kind == 2) {
-            // pack of k whole rows: segmented scans over the lanes of each row (as fwd_phase_a_pack)
-            const bool act = lane < n;
-            const int e_id = beg + lane;
-            int lo = 0, hi = k - 1;
-#pragma unroll
-            for (int it = 0; it < 5; ++it) {
-                const int mid = (lo + hi) >> 1;
-                const int bm = __shfl_sync(FULL, lb, mid);
-                if (bm > e_id) hi = mid; else lo = min(mid + 1, k - 1);
-            }
-            const int sa = __shfl_sync(FULL, la, lo) - beg, sb = __shfl_sync(FULL, lb, lo) - beg - 1;
-            const int r = row + lo;
-            float z[H];
-            int j = 0;
-            if (act) {
-                j = col[e_id];
-                float as[H], ad[H];
-                load_vecH<H>(a_src + int64_t(j) * H, as);
-                load_vecH<H>(a_dst + int64_t(r) * H, ad);
-#pragma unroll
-                for (int h = 0; h < H; ++h) z[h] = as[h] + ad[h];
-            } else {
-#pragma unroll
-                for (int h = 0; h < H; ++h) z[h] = -INFINITY;
-            }
-            float o[H], mrow[H], srow[H];
-#pragma unroll
-            for (int h = 0; h < H; ++h) {
-                const float e = act ? leaky(z[h], slope) : -INFINITY;
-                float mx = e;
-#pragma unroll
-                for (int d = 1; d < 32; d <<= 1) {
-                    const float t = __shfl_up_sync(FULL, mx, d);
-                    if (lane - d >= sa) mx = fmaxf(mx, t);
-                }
-                mrow[h] = __shfl_sync(FULL, mx, sb);
-                const float pexp = act ? expf(e - mrow[h]) : 0.f;
-                float sm = pexp;
-#pragma unroll
-                for (int d = 1; d < 32; d <<= 1) {
-                    const float t = __shfl_up_sync(FULL, sm, d);
-                    if (lane - d >= sa) sm += t;
-                }
-                srow[h] = __shfl_sync(FULL, sm, sb) + 1e-16f;       // PyG softmax: out / (sum + 1e-16)
-                o[h] = with_sign(pexp / srow[h], !(z[h] > 0.f));
-            }
-            if (act) {
-                store_vecH<H>(alpha + int64_t(e_id) * H, o);
-                jflag[e_id] = j | (lane == sb ? int(0x80000000u) : 0);
-                if (lane == sb) {
-                    store_vecH<H>(rowmax + int64_t(r) * H, mrow);
-                    store_vecH<H>(rowsum + int64_t(r) * H, srow);
-                }
-            }
-            continue;
-        }
-        // a single row (kind 1, first chunk of it): statistics sweep over all of its chunks, then the write sweep
-        float adst[H], m[H], sv[H];
-        load_vecH<H>(a_dst + int64_t(row) * H, adst);
-#pragma unroll
-        for (int h = 0; h < H; ++h) { m[h] = -INFINITY; sv[h] = 0.f; }
-        const int row_beg = beg, r = row;
-        alpha_stat_chunk(beg, n, adst, col, a_src, slope, m, sv, lane);
-        int row_end = beg + n;
-        while (!last) {
-            cur.next(rowptr, row, beg, n, first, last, on_empty);     // stays inside the row until last
-            alpha_stat_chunk(beg, n, adst, col, a_src, slope, m, sv, lane);
-            row_end = beg + n;
-        }
-        float sinv[H];
-#pragma unroll
-        for (int h = 0; h < H; ++h) { sv[h] += 1e-16f; sinv[h] = 1.f / sv[h]; }
-        if (lane == 0) {
-            store_vecH<H>(rowmax + int64_t(r) * H, m);
-            store_vecH<H>(rowsum + int64_t(r) * H, sv);
-        }
-        for (int b = row_beg; b < row_end; b += 32)
-            alpha_write_chunk(b, min(32, row_end - b), b + 32 >= row_end, adst, m, sinv, col, a_src, slope, alpha, jflag, lane);
-    }
+    alpha_items_body<H, false, false, PACK>(rowptr, col, a_src, a_dst, items.item_start[item], items.item_start[item + 1],
+                                            hub_threshold, slope, out, rowmax, rowsum, lane);
 }
 
-// hub rows: (1) statistics of every 512-edge chunk, (2) one warp per hub row folds them in chunk order, (3) write sweep
+// hub rows: (1) statistics of every 512-edge chunk, (2) one thread per (hub row, head) folds them in chunk order, (3) write sweep
 __global__ void __launch_bounds__(IN_THREADS)
 in_alpha_hub_stats(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col, const float* __restrict__ a_src,
                    const float* __restrict__ a_dst, gnnfd_hub_plan_t plan, float slope, float* __restrict__ part_ms)
@@ -436,54 +296,23 @@ in_alpha_hub_stats(const int32_t* __restrict__ rowptr, const int32_t* __restrict
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int c = blockIdx.x * IN_WARPS + warp;
     if (c >= plan.n_chunk) return;
-    const int slot = plan.chunk_hub[c], i = plan.hub_row[slot];
-    const int beg = rowptr[i] + (c - plan.hub_chunk_ptr[slot]) * plan.chunk;
-    const int end = min(rowptr[i + 1], beg + plan.chunk);
-    float adst[H], m[H], sv[H];
-    load_vecH<H>(a_dst + int64_t(i) * H, adst);
-#pragma unroll
-    for (int h = 0; h < H; ++h) { m[h] = -INFINITY; sv[h] = 0.f; }
-    for (int b = beg; b < end; b += 32) alpha_stat_chunk(b, min(32, end - b), adst, col, a_src, slope, m, sv, lane);
-    if (lane == 0) {
-        store_vecH<H>(part_ms + int64_t(c) * 2 * H, m);
-        store_vecH<H>(part_ms + int64_t(c) * 2 * H + H, sv);
-    }
+    alpha_hub_stats_body<H>(rowptr, col, a_src, a_dst, plan, c, slope, part_ms, lane);
 }
 __global__ void in_alpha_hub_merge(gnnfd_hub_plan_t plan, const float* __restrict__ part_ms, float* __restrict__ rowmax,
                                    float* __restrict__ rowsum)
 {
-    const int slot = blockIdx.x, h = threadIdx.x;          // one thread per head: the chunk order is the summation order
-    if (h >= H) return;
-    const int i = plan.hub_row[slot];
-    float m = -INFINITY, s = 0.f;
-    for (int c = plan.hub_chunk_ptr[slot]; c < plan.hub_chunk_ptr[slot + 1]; ++c) {
-        const float cm = part_ms[int64_t(c) * 2 * H + h], cs = part_ms[int64_t(c) * 2 * H + H + h];
-        const float mn = fmaxf(m, cm);
-        s = s * expf(m - mn) + cs * expf(cm - mn);
-        m = mn;
-    }
-    rowmax[int64_t(i) * H + h] = m;
-    rowsum[int64_t(i) * H + h] = s + 1e-16f;
+    if (threadIdx.x >= H) return;
+    alpha_hub_merge_body<H>(plan, blockIdx.x, threadIdx.x, part_ms, rowmax, rowsum);
 }
 __global__ void __launch_bounds__(IN_THREADS)
 in_alpha_hub_write(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col, const float* __restrict__ a_src,
                    const float* __restrict__ a_dst, gnnfd_hub_plan_t plan, float slope, const float* __restrict__ rowmax,
-                   const float* __restrict__ rowsum, float* __restrict__ alpha, int32_t* __restrict__ jflag)
+                   const float* __restrict__ rowsum, AlphaOut out)
 {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int c = blockIdx.x * IN_WARPS + warp;
     if (c >= plan.n_chunk) return;
-    const int slot = plan.chunk_hub[c], i = plan.hub_row[slot];
-    const int beg = rowptr[i] + (c - plan.hub_chunk_ptr[slot]) * plan.chunk;
-    const int row_end = rowptr[i + 1], end = min(row_end, beg + plan.chunk);
-    float adst[H], m[H], sinv[H];
-    load_vecH<H>(a_dst + int64_t(i) * H, adst);
-    load_vecH<H>(rowmax + int64_t(i) * H, m);
-    load_vecH<H>(rowsum + int64_t(i) * H, sinv);
-#pragma unroll
-    for (int h = 0; h < H; ++h) sinv[h] = 1.f / sinv[h];
-    for (int b = beg; b < end; b += 32)
-        alpha_write_chunk(b, min(32, end - b), b + 32 >= row_end, adst, m, sinv, col, a_src, slope, alpha, jflag, lane);
+    alpha_hub_write_body<H, false, false>(rowptr, col, a_src, a_dst, plan, c, slope, rowmax, rowsum, out, lane);
 }
 
 // =====================================================================================================================
@@ -695,10 +524,11 @@ static int launch_in_alpha(const gnnfd_graph_t* g, const float* a_src, const flo
         const char* e = getenv("GNNFD_FWD_PACK");
         return e ? atoi(e) != 0 : true;
     }();
+    const AlphaOut out{alpha, jflag, nullptr, KeepMask(), 1.f};
     if (pack)
-        in_alpha_items<true><<<grid, IN_THREADS, 0, st>>>(g->rowptr, g->col, a_src, a_dst, g->items_dst, thr, slope, alpha, jflag, rowmax, rowsum);
+        in_alpha_items<true><<<grid, IN_THREADS, 0, st>>>(g->rowptr, g->col, a_src, a_dst, g->items_dst, thr, slope, out, rowmax, rowsum);
     else
-        in_alpha_items<false><<<grid, IN_THREADS, 0, st>>>(g->rowptr, g->col, a_src, a_dst, g->items_dst, thr, slope, alpha, jflag, rowmax, rowsum);
+        in_alpha_items<false><<<grid, IN_THREADS, 0, st>>>(g->rowptr, g->col, a_src, a_dst, g->items_dst, thr, slope, out, rowmax, rowsum);
     g_launches += 1;
     if (g->hub_dst.n_hub > 0) {
         const gnnfd_hub_plan_t& pl = g->hub_dst;
@@ -709,7 +539,7 @@ static int launch_in_alpha(const gnnfd_graph_t* g, const float* a_src, const flo
         const unsigned gc = (unsigned)((pl.n_chunk + IN_WARPS - 1) / IN_WARPS);
         in_alpha_hub_stats<<<gc, IN_THREADS, 0, st>>>(g->rowptr, g->col, a_src, a_dst, pl, slope, part_ms);
         in_alpha_hub_merge<<<(unsigned)pl.n_hub, 32, 0, st>>>(pl, part_ms, rowmax, rowsum);
-        in_alpha_hub_write<<<gc, IN_THREADS, 0, st>>>(g->rowptr, g->col, a_src, a_dst, pl, slope, rowmax, rowsum, alpha, jflag);
+        in_alpha_hub_write<<<gc, IN_THREADS, 0, st>>>(g->rowptr, g->col, a_src, a_dst, pl, slope, rowmax, rowsum, out);
         g_launches += 3;
     }
     GNNFD_LAUNCH_CHECK();

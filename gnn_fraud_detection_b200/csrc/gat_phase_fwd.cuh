@@ -6,6 +6,32 @@
 
 namespace gnnfd {
 
+// Fused row epilogue:  v = mean/concat + bias;  v = v*scale + shift (folded eval-mode BatchNorm, optional);
+// v = act(v);  v += residual[row] (optional).  Mirrors gat.py:80-91 in eval mode (BatchNorm -> ReLU -> residual).
+struct EpiParams {
+    const float* bias;
+    const float* scale;
+    const float* shift;
+    const float* residual;
+    int act;
+};
+
+__device__ __forceinline__ float apply_act(float v, int act)
+{
+    if (act == GNNFD_ACT_RELU) return fmaxf(v, 0.f);
+    if (act == GNNFD_ACT_ELU) return v > 0.f ? v : expm1f(v);
+    return v;
+}
+// the epilogue of output channel c of row i (ld = output row length), v = the head mean / concat value
+__device__ __forceinline__ float epi_value(float v, int c, int64_t i, int ld, const EpiParams& ep)
+{
+    v = v + (ep.bias ? ep.bias[c] : 0.f);
+    if (ep.scale) v = fmaf(v, ep.scale[c], ep.shift[c]);
+    v = apply_act(v, ep.act);
+    if (ep.residual) v += ep.residual[i * ld + c];
+    return v;
+}
+
 // statistics of one chunk, relative to its own maximum (all lanes hold the same values)
 template <int H>
 struct ChunkStat {

@@ -3,8 +3,10 @@
 Gather traffic is charged per edge (no credit for cache reuse); indices are int32 (i = 4 B); logits,
 row statistics, gradients are fp32; ``s`` is the storage size of a projected feature element (4 fp32 /
 2 bf16); ``Co`` = C (head mean) or H*C (concat).  ``Ep`` is E' (edges after the self-loop rewrite).
-The ``gat_bwd_dst`` term describes the backward that runs: for the head mean the two-pass form (d_alpha computed
-source-major, then a dst pass that reads no features), for ``concat`` the single gather pass.
+The ``gat_fwd`` and ``gat_bwd_dst`` terms describe the kernels that run: for the head mean on one node set
+(``n_src`` not given) the source-major forms (forward: attention pass, source-major messages, row sums; backward:
+d_alpha computed source-major, then a dst pass that reads no features), otherwise the gather passes (the backward's
+two-pass form also runs for a head-mean partition with ``n_src``).
 """
 from __future__ import annotations
 
@@ -17,8 +19,16 @@ def stage_bytes(N: int, Ep: int, K: int, H: int = 8, C: int = 64, concat: bool =
     b = {}
     # x read, xw write, a_src/a_dst write, W read
     b["project_fwd"] = N * (K * 4 + D * s + 8 * H) + K * D * 4
-    # per edge: xw[src] row, col, a_src[src]; per row: a_dst, out, (max,sum), rowptr
-    b["gat_fwd"] = Ep * (D * s + i + 4 * H) + N * (4 * H + 4 * Co + 8 * H + i)
+    if concat or n_src is not None:
+        # gather pass -- per edge: xw[src] row, col, a_src[src]; per row: a_dst, out, (max,sum), rowptr
+        b["gat_fwd"] = Ep * (D * s + i + 4 * H) + N * (4 * H + 4 * Co + 8 * H + i)
+    else:
+        # head mean, three passes (DESIGN 4.3).  Attention -- per edge: col, a_src[src], alpha_used write; per row:
+        # a_dst, (max,sum), rowptr.  Messages -- per edge: csc_eid, alpha_used[eid], v write; per source row: xw row,
+        # colptr.  Sums -- per edge: v read; per row: out, rowptr
+        b["gat_fwd"] = (Ep * (i + 4 * H + 4 * H) + N * (4 * H + 8 * H + i)
+                        + Ep * (i + 4 * H + 4 * C) + Ns * (D * s + i)
+                        + Ep * 4 * C + N * (4 * Co + i))
     if concat:
         # one gather pass -- per edge: xw[src] row, col, a_src[src], dz write (alpha write is not charged, as in
         # SURVEY 8(d)); per row: dOut, (a_dst,max,sum), da_dst, rowptr

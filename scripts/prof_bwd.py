@@ -1,11 +1,13 @@
-"""Per-kernel device time of the layer backward on the headline graph (20M nodes / 200M edges, H=8, C=64, head mean).
+"""Per-kernel device time of the layer backward (or, with --stage fwd, of the layer's gat_fwd) on the headline graph
+(20M nodes / 200M edges, H=8, C=64, head mean).
 
 Runs warm-up steps of the single-GPU layer as bench.py does (project_fwd, gat_fwd, gat_bwd, project_bwd), one step for
-max_memory_allocated, then one step whose gat_bwd call (the dst and src passes) runs under torch.profiler with CUDA
-activity, and prints one JSON line: the device time of every kernel gat_bwd launched, by kernel name.  Run it in a process of its own
-(tracing slows the host; the times are device times of single launches).
+max_memory_allocated / max_memory_reserved, then one step whose gat_bwd call (the dst and src passes) or gat_fwd call
+runs under torch.profiler with CUDA activity, and prints one JSON line: the device time of every kernel that call
+launched, by kernel name.  Run it in a process of its own (tracing slows the host; the times are device times of single
+launches).
 
-  python scripts/prof_bwd.py [--workload powerlaw_200m] [--out profiles/prof_bwd_TAG.json]
+  python scripts/prof_bwd.py [--stage bwd|fwd] [--workload powerlaw_200m] [--out profiles/prof_bwd_TAG.json]
 
 GNNFD_B200_LIB selects the library build, as for bench.py."""
 import argparse
@@ -33,6 +35,7 @@ def short(name: str) -> str:
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--workload", default="powerlaw_200m", choices=["powerlaw_200m", "powerlaw_20m"])
+    ap.add_argument("--stage", default="bwd", choices=["bwd", "fwd"], help="the call that runs under the profiler")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--out", default=None, help="also write the JSON line to this file")
     args = ap.parse_args()
@@ -50,19 +53,29 @@ def main():
     x = torch.randn(N, K, device=dev, generator=torch.Generator(device=dev).manual_seed(0))
     d_out = torch.full((N, C), 1.0 / N, device=dev)
 
-    def step(prof_bwd: bool = False):
-        xw, a_src, a_dst = Fn.project_fwd(x, W, a_s, a_d, H, C)
-        out, rowmax, rowsum = Fn.gat_fwd(g, xw, a_src, a_dst, conv.bias.detach(), H, C, 0.2, False)
-        del out
-        torch.cuda.synchronize()
+    def step(prof_stage: str = ""):
         prof = None
-        if prof_bwd:                   # only gat_bwd runs inside the profiled window
-            prof = profile(activities=[ProfilerActivity.CUDA])
-            prof.__enter__()
+
+        def window(stage):             # only the profiled call runs inside the window
+            nonlocal prof
+            torch.cuda.synchronize()
+            if prof_stage == stage:
+                prof = profile(activities=[ProfilerActivity.CUDA])
+                prof.__enter__()
+
+        def close(stage):
+            torch.cuda.synchronize()
+            if prof_stage == stage:
+                prof.__exit__(None, None, None)
+
+        xw, a_src, a_dst = Fn.project_fwd(x, W, a_s, a_d, H, C)
+        window("fwd")
+        out, rowmax, rowsum = Fn.gat_fwd(g, xw, a_src, a_dst, conv.bias.detach(), H, C, 0.2, False)
+        close("fwd")
+        del out
+        window("bwd")
         dxw, da_src, da_dst = Fn.gat_bwd(g, xw, a_src, a_dst, rowmax, rowsum, d_out, a_s, a_d, H, C, 0.2, False)
-        torch.cuda.synchronize()
-        if prof_bwd:
-            prof.__exit__(None, None, None)
+        close("bwd")
         Fn.project_bwd(x, W, dxw, xw, da_src, da_dst, d_out, H, C, C, False)
         torch.cuda.synchronize()
         return prof
@@ -72,19 +85,20 @@ def main():
     torch.cuda.reset_peak_memory_stats(dev)
     step()
     peak = torch.cuda.max_memory_allocated(dev)
-    prof = step(prof_bwd=True)
+    peak_reserved = torch.cuda.max_memory_reserved(dev)
+    prof = step(prof_stage=args.stage)
     kern = {}
     for e in prof.events():
         if e.device_type.name != "CUDA" or e.name.startswith(("Memcpy", "Memset")):
             continue
         k = short(e.name)
         kern[k] = kern.get(k, 0.0) + e.time_range.elapsed_us() / 1e3
-    bwd = {k: round(v, 3) for k, v in sorted(kern.items(), key=lambda kv: -kv[1])}
+    per = {k: round(v, 3) for k, v in sorted(kern.items(), key=lambda kv: -kv[1])}
     line = {
         "workload": args.workload, "gpu": torch.cuda.get_device_name(dev),
         "lib": os.environ.get("GNNFD_B200_LIB", "gnn_fraud_detection_b200/libgnnfd_b200.so"),
-        "bwd_kernel_ms": bwd, "bwd_total_ms": round(sum(bwd.values()), 3),
-        "max_memory_allocated_gb": round(peak / 1e9, 2),
+        f"{args.stage}_kernel_ms": per, f"{args.stage}_total_ms": round(sum(per.values()), 3),
+        "max_memory_allocated_gb": round(peak / 1e9, 2), "max_memory_reserved_gb": round(peak_reserved / 1e9, 2),
     }
     s = json.dumps(line)
     print(s)
