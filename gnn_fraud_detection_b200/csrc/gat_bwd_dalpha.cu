@@ -7,18 +7,21 @@
 //            across source-row boundaries, as tasks of <= 32 edges of one source row.  Each task's dO rows go into a
 //            per-warp ring of DA_RING row slots and, when the task starts a new source row, xw[j] into one of
 //            DA_XROWS row slots (16-byte cp.async, 16 lanes per dO row, one commit group per task), so the next
-//            tasks' rows are in flight while the current one is reduced.  Per edge 16 FMAs and phase B's butterfly
-//            give d_alpha with phase B's arithmetic; it is stored at the edge's CSR position csc_eid[p] of an
-//            [E',H] workspace buffer.  Sources above the hub threshold are split by the hub_src plan (_hub, one
-//            warp per chunk); every output is per edge, so the chunks need no merge.
+//            tasks' rows are in flight while the current one is reduced; a_src[j] rides in the xw row slot.  Per
+//            edge 16 FMAs and phase B's butterfly give d_alpha with phase B's arithmetic; the record
+//            {d_alpha, a_src[j]} is stored at the edge's CSR position csc_eid[p] of an [E',2H] workspace buffer.
+//            Sources above the hub threshold are split by the hub_src plan (_hub, one warp per chunk); every output
+//            is per edge, so the chunks need no merge.
 //   pass 2 (CSR; gat_bwd_dst_eg_items / _hub1 / _hub2): the chunk, pack and hub_dst schedule of the gather kernels,
-//            lane = edge.  It reads col, d_alpha, csr2csc (and perm) contiguously, the row statistics per row and
-//            a_src[col[e]] as its one gather, recomputes alpha with edge_alpha, and forms u = alpha * d_alpha * keep,
-//            t, dz and da_dst with the same warp sums in the same order as the gather kernels.  (alpha_used, dz) go
-//            to the edge's source-major slot csr2csc[e].
-// Per edge this moves ~4 + 4 + 256 + 32 B (pass 1) and ~4 + 32 + 32 + 4 + 64 B (pass 2).  alpha_used equals the
-// gather kernels' bit for bit; dz and da_dst differ in the last bits on rows longer than one chunk, where the gather
-// kernels recompute alpha for the second sweep with a contracted multiply-add.
+//            lane = edge.  It reads only contiguous streams -- the record, csr2csc (and perm) over the edge range, the
+//            row statistics over the row range -- with the next chunk in flight, recomputes alpha with edge_alpha from
+//            the record's a_src, and forms u = alpha * d_alpha * keep, t, dz and da_dst with the same warp sums in the
+//            same order as the gather kernels.  (alpha_used, dz) go to the edge's source-major slot csr2csc[e], each
+//            32-B vector (H = 8) as one 256-bit store, so that a lane writes whole sectors at its random address.
+// Per edge this moves ~4 + 4 + 256 + 64 B (pass 1) and ~64 + 4 + 64 B (pass 2).  The record is 4H B wider than a bare
+// d_alpha so that pass 2 has no dependent gather (col[e] -> a_src[col[e]]).  alpha_used equals the gather kernels' bit
+// for bit; dz and da_dst differ in the last bits on rows longer than one chunk, where the gather kernels recompute
+// alpha for the second sweep with a contracted multiply-add.
 #include "gat_stream.cuh"
 #include "gat_phase_bwd.cuh"
 
@@ -39,6 +42,18 @@ __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc)
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(st_smem_u32(smem_dst)), "l"(gsrc) : "memory");
 }
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+// H floats to a 32-byte-aligned address: one 256-bit store for H = 8 (a whole sector per lane), else store_vecH
+template <int H>
+__device__ __forceinline__ void store_vecH_wide(float* __restrict__ p, const float (&v)[H])
+{
+    if constexpr (H == 8) {
+        asm volatile("st.global.v8.f32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(p), "f"(v[0]), "f"(v[1]),
+                     "f"(v[2]), "f"(v[3]), "f"(v[4]), "f"(v[5]), "f"(v[6]), "f"(v[7])
+                     : "memory");
+    } else {
+        store_vecH<H>(p, v);
+    }
+}
 // wait until at most n of this thread's commit groups are pending (n < DA_TASKS)
 __device__ __forceinline__ void cp_async_wait_pending(int n)
 {
@@ -97,9 +112,9 @@ __device__ __forceinline__ void dalpha_edge(const float (&v)[GE::NS][GE::VW], co
     dalpha_reduce<GE>(d, dal_t, lane);
 }
 
-// one edge's d_alpha from shared memory to its CSR position
+// one edge's record {d_alpha[0..H) from shared memory, a_src[j][0..H) of its source} to its CSR position
 template <int H>
-__device__ __forceinline__ void store_dalpha(float* __restrict__ dst, const float* dal_t)
+__device__ __forceinline__ void store_record(float* __restrict__ dst, const float* dal_t, const float (&as)[H])
 {
     float dal[H];
 #pragma unroll
@@ -107,7 +122,8 @@ __device__ __forceinline__ void store_dalpha(float* __restrict__ dst, const floa
         const float4 d4 = *reinterpret_cast<const float4*>(dal_t + 4 * k);
         dal[4 * k] = d4.x; dal[4 * k + 1] = d4.y; dal[4 * k + 2] = d4.z; dal[4 * k + 3] = d4.w;
     }
-    store_vecH<H>(dst, dal);
+    store_vecH_wide<H>(dst, dal);
+    store_vecH_wide<H>(dst + H, as);
 }
 
 // per-warp shared memory of the pass-1 stream
@@ -115,7 +131,8 @@ template <class GE>
 struct DaGeo {
     static constexpr int DO_BYTES = DA_RING * GE::C * 4;
     static constexpr int XROW_BYTES = GE::D * int(sizeof(typename GE::XT));
-    static constexpr int X_BYTES = DA_XROWS * XROW_BYTES;
+    static constexpr int XSLOT_BYTES = XROW_BYTES + GE::H * 4;    // xw[j], then a_src[j]
+    static constexpr int X_BYTES = DA_XROWS * XSLOT_BYTES;
     static constexpr int DAL_BYTES = 32 * GE::H * 4;
     static constexpr int EID_BYTES = DA_RING * 4;
     static constexpr int WARP_BYTES = ((DO_BYTES + X_BYTES + DAL_BYTES + EID_BYTES + 127) / 128) * 128;
@@ -130,8 +147,8 @@ template <class GE>
 __global__ void __launch_bounds__(DA_THREADS, 4)
 gat_bwd_dalpha_src_stream(const int32_t* __restrict__ colptr, const int32_t* __restrict__ csc_row,
                           const int32_t* __restrict__ csc_eid, const typename GE::XT* __restrict__ xw,
-                          const float* __restrict__ d_out, gnnfd_item_plan_t items, int hub_threshold,
-                          float* __restrict__ d_alpha)
+                          const float* __restrict__ a_src, const float* __restrict__ d_out, gnnfd_item_plan_t items,
+                          int hub_threshold, float* __restrict__ rec)
 {
     using SG = DaGeo<GE>;
     constexpr int H = GE::H, NS = GE::NS, VW = GE::VW, C = GE::C;
@@ -167,7 +184,10 @@ gat_bwd_dalpha_src_stream(const int32_t* __restrict__ colptr, const int32_t* __r
                 const uint8_t* src = reinterpret_cast<const uint8_t*>(xw + int64_t(nj) * GE::D);
 #pragma unroll
                 for (int q = 0; q < NS; ++q)
-                    cp_async16(x_s + xs * SG::XROW_BYTES + (lane + 32 * q) * 16, src + (lane + 32 * q) * 16);
+                    cp_async16(x_s + xs * SG::XSLOT_BYTES + (lane + 32 * q) * 16, src + (lane + 32 * q) * 16);
+                if (lane < H / 4)
+                    cp_async16(x_s + xs * SG::XSLOT_BYTES + SG::XROW_BYTES + lane * 16,
+                               a_src + int64_t(nj) * H + 4 * lane);
                 ++x_issued;
             }
             cp_async_commit();
@@ -179,6 +199,7 @@ gat_bwd_dalpha_src_stream(const int32_t* __restrict__ colptr, const int32_t* __r
     };
     issue();
     float v[NS][VW];                           // xw row of the current source, slot layout
+    float as[H];                               // a_src of the current source
     while (t_done < t_issued) {
         cp_async_wait_pending(t_issued - t_done - 1);
         __syncwarp();
@@ -186,12 +207,15 @@ gat_bwd_dalpha_src_stream(const int32_t* __restrict__ colptr, const int32_t* __r
         const int n = tk & 63;
         if (tk & 64) {
 #pragma unroll
-            for (int q = 0; q < NS; ++q) lds_slot(x_s + (tk >> 7) * SG::XROW_BYTES, q, lane, v[q]);
+            for (int q = 0; q < NS; ++q) lds_slot(x_s + (tk >> 7) * SG::XSLOT_BYTES, q, lane, v[q]);
+            const float* as_s = reinterpret_cast<const float*>(x_s + (tk >> 7) * SG::XSLOT_BYTES + SG::XROW_BYTES);
+#pragma unroll
+            for (int h = 0; h < H; ++h) as[h] = as_s[h];
             ++x_done;
         }
         for (int t = 0; t < n; ++t) dalpha_edge<GE>(v, do_s + ((e_done + t) % DA_RING) * C, dal_s + t * H, lane);
         __syncwarp();
-        if (lane < n) store_dalpha<H>(d_alpha + int64_t(eid_s[(e_done + lane) % DA_RING]) * H, dal_s + lane * H);
+        if (lane < n) store_record<H>(rec + int64_t(eid_s[(e_done + lane) % DA_RING]) * 2 * H, dal_s + lane * H, as);
         __syncwarp();                          // the task's slots are read before they are refilled
         e_done += n;
         ++t_done;
@@ -204,7 +228,8 @@ template <class GE>
 __global__ void __launch_bounds__(DA_THREADS, 6)
 gat_bwd_dalpha_src_hub(const int32_t* __restrict__ colptr, const int32_t* __restrict__ csc_row,
                        const int32_t* __restrict__ csc_eid, const typename GE::XT* __restrict__ xw,
-                       const float* __restrict__ d_out, gnnfd_hub_plan_t plan, float* __restrict__ d_alpha)
+                       const float* __restrict__ a_src, const float* __restrict__ d_out, gnnfd_hub_plan_t plan,
+                       float* __restrict__ rec)
 {
     constexpr int H = GE::H, NS = GE::NS, VW = GE::VW, C = GE::C;
     __shared__ __align__(16) float do_sh[DA_WARPS][32 * C];
@@ -218,9 +243,10 @@ gat_bwd_dalpha_src_hub(const int32_t* __restrict__ colptr, const int32_t* __rest
     const int end = min(colptr[j + 1], beg + plan.chunk);
     float* do_s = do_sh[warp];
     float* dal_s = dal_sh[warp];
-    float v[NS][VW];
+    float v[NS][VW], as[H];
 #pragma unroll
     for (int q = 0; q < NS; ++q) load_slot(xw + j * GE::D, q, lane, v[q]);
+    load_vecH<H>(a_src + j * H, as);
     for (int base = beg; base < end; base += 32) {
         const int n = min(32, end - base);
         const bool live = lane < n;
@@ -232,7 +258,7 @@ gat_bwd_dalpha_src_hub(const int32_t* __restrict__ colptr, const int32_t* __rest
         __syncwarp();
         for (int t = 0; t < n; ++t) dalpha_edge<GE>(v, do_s + t * C, dal_s + t * H, lane);
         __syncwarp();
-        if (live) store_dalpha<H>(d_alpha + int64_t(eid) * H, dal_s + lane * H);
+        if (live) store_record<H>(rec + int64_t(eid) * 2 * H, dal_s + lane * H, as);
         __syncwarp();
     }
 }
@@ -247,33 +273,81 @@ struct EgEdge {
     int pos;               // source-major slot
     unsigned keep;         // dropout keep bits
 };
-// pass 2 reads an edge in two steps so that the next chunk's contiguous loads are in flight while the current chunk
-// is reduced: eg_fetch (col, csr2csc, d_alpha, perm of dst-sorted edge e), then eg_finish (the row statistics of its
-// destination row, the one gather a_src[col[e]], alpha recomputed as phase A does, the keep bits)
+// pass 2 reads an edge in two steps so that the next chunk's loads are in flight while the current chunk is reduced:
+// eg_fetch (the record {d_alpha, a_src[j]}, csr2csc and perm of dst-sorted edge e -- all contiguous over a chunk),
+// then eg_finish (the row statistics of its destination row, alpha recomputed as phase A does, the keep bits)
 template <int H>
 struct EgRaw {
-    int j, pos, pe;
-    float d[H];
+    int pos, pe;
+    float d[H], as[H];
 };
 template <int H, bool DROPOUT>
-__device__ __forceinline__ void eg_fetch(EgRaw<H>& r, int e, bool live, const int32_t* __restrict__ col,
-                                         const int32_t* __restrict__ perm, const int32_t* __restrict__ csr2csc,
-                                         const float* __restrict__ d_alpha)
+__device__ __forceinline__ void eg_fetch(EgRaw<H>& r, int e, bool live, const int32_t* __restrict__ perm,
+                                         const int32_t* __restrict__ csr2csc, const float* __restrict__ rec)
 {
-    r.j = r.pos = r.pe = 0;
+    r.pos = r.pe = 0;
 #pragma unroll
-    for (int h = 0; h < H; ++h) r.d[h] = 0.f;
+    for (int h = 0; h < H; ++h) r.d[h] = r.as[h] = 0.f;
     if (!live) return;
-    r.j = col[e];
     r.pos = csr2csc[e];
-    load_vecH<H>(d_alpha + int64_t(e) * H, r.d);
+    load_vecH<H>(rec + int64_t(e) * 2 * H, r.d);
+    load_vecH<H>(rec + int64_t(e) * 2 * H + H, r.as);
     if (DROPOUT) r.pe = perm[e];
+}
+// the items kernel holds the next chunk in shared memory rather than in registers: eg_fetch_async copies it (lane =
+// edge, every lane copies and later reads only its own entries, one commit group per chunk), eg_take reads it back
+template <int H>
+struct EgStage {
+    float rec[32][2 * H];
+    int pos[32], pe[32];
+};
+__device__ __forceinline__ void cp_async4(void* smem_dst, const void* gsrc)
+{
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(st_smem_u32(smem_dst)), "l"(gsrc) : "memory");
+}
+template <int H, bool DROPOUT>
+__device__ __forceinline__ void eg_fetch_async(EgStage<H>& s, int e, bool live, const int32_t* __restrict__ perm,
+                                               const int32_t* __restrict__ csr2csc, const float* __restrict__ rec,
+                                               int lane)
+{
+    if (live) {
+#pragma unroll
+        for (int k = 0; k < H / 2; ++k) cp_async16(&s.rec[lane][4 * k], rec + int64_t(e) * 2 * H + 4 * k);
+        cp_async4(&s.pos[lane], csr2csc + e);
+        if (DROPOUT) cp_async4(&s.pe[lane], perm + e);
+    }
+    cp_async_commit();
+}
+template <int H, bool DROPOUT>
+__device__ __forceinline__ void eg_take(EgRaw<H>& r, const EgStage<H>& s, bool live, int lane)
+{
+    r.pos = r.pe = 0;
+#pragma unroll
+    for (int h = 0; h < H; ++h) r.d[h] = r.as[h] = 0.f;
+    if (!live) return;
+#pragma unroll
+    for (int k = 0; k < H / 4; ++k) {
+        const float4 d4 = *reinterpret_cast<const float4*>(&s.rec[lane][4 * k]);
+        const float4 a4 = *reinterpret_cast<const float4*>(&s.rec[lane][H + 4 * k]);
+        r.d[4 * k] = d4.x; r.d[4 * k + 1] = d4.y; r.d[4 * k + 2] = d4.z; r.d[4 * k + 3] = d4.w;
+        r.as[4 * k] = a4.x; r.as[4 * k + 1] = a4.y; r.as[4 * k + 2] = a4.z; r.as[4 * k + 3] = a4.w;
+    }
+    r.pos = s.pos[lane];
+    if (DROPOUT) r.pe = s.pe[lane];
+}
+// the row statistics of destination row i into L1, so that eg_finish of the next chunk does not wait on DRAM for them
+template <int H>
+__device__ __forceinline__ void eg_prefetch_row(int64_t i, const float* __restrict__ a_dst,
+                                                const float* __restrict__ rowmax, const float* __restrict__ rowsum)
+{
+    asm volatile("prefetch.global.L1 [%0];" ::"l"(a_dst + i * H));
+    asm volatile("prefetch.global.L1 [%0];" ::"l"(rowmax + i * H));
+    asm volatile("prefetch.global.L1 [%0];" ::"l"(rowsum + i * H));
 }
 template <int H, bool DROPOUT>
 __device__ __forceinline__ void eg_finish(EgEdge<H>& x, const EgRaw<H>& r, bool live, int64_t row,
-                                          const float* __restrict__ a_src, const float* __restrict__ a_dst,
-                                          const float* __restrict__ rowmax, const float* __restrict__ rowsum,
-                                          float slope, KeepMask keep)
+                                          const float* __restrict__ a_dst, const float* __restrict__ rowmax,
+                                          const float* __restrict__ rowsum, float slope, KeepMask keep)
 {
     x.pos = r.pos;
     x.keep = 0xffu;
@@ -285,25 +359,12 @@ __device__ __forceinline__ void eg_finish(EgEdge<H>& x, const EgRaw<H>& r, bool 
     if (!live) return;
     RowStat<H> st;
     load_row_stat<H>(st, row, a_dst, rowmax, rowsum);
-    float as[H];
-    load_vecH<H>(a_src + int64_t(r.j) * H, as);
 #pragma unroll
     for (int h = 0; h < H; ++h) {
-        const float z = as[h] + st.adst[h];
+        const float z = r.as[h] + st.adst[h];
         x.a[h] = __uint_as_float(__float_as_uint(edge_alpha(z, slope, st.m[h], st.inv[h])) | (z > 0.f ? 0u : NEG_FLAG));
     }
     if (DROPOUT) x.keep = keep.bits(r.pe, H);
-}
-template <int H, bool DROPOUT>
-__device__ __forceinline__ void eg_load(EgEdge<H>& x, int e, bool live, int64_t row, const int32_t* __restrict__ col,
-                                        const int32_t* __restrict__ perm, const int32_t* __restrict__ csr2csc,
-                                        const float* __restrict__ a_src, const float* __restrict__ a_dst,
-                                        const float* __restrict__ rowmax, const float* __restrict__ rowsum, float slope,
-                                        KeepMask keep, const float* __restrict__ d_alpha)
-{
-    EgRaw<H> r;
-    eg_fetch<H, DROPOUT>(r, e, live, col, perm, csr2csc, d_alpha);
-    eg_finish<H, DROPOUT>(x, r, live, row, a_src, a_dst, rowmax, rowsum, slope, keep);
 }
 // head h of an edge, phase C's arithmetic: pre-dropout alpha, LeakyReLU slope, keep scale, u = alpha * d_alpha * keep
 struct EgHead {
@@ -320,7 +381,8 @@ __device__ __forceinline__ EgHead eg_head(const EgEdge<H>& x, int h, bool live, 
     r.u = live ? r.alpha * x.d[h] * r.ks : 0.f;
     return r;
 }
-// the final slot: alpha_used = alpha * keep, dz
+// the final slot: alpha_used = alpha * keep, dz.  eg_ld < 0 marks 32-byte-aligned slots (stored with store_vecH_wide)
+// of stride -eg_ld
 template <int H>
 __device__ __forceinline__ void eg_store(const EgEdge<H>& x, const float (&o)[H], float keep_scale, float* alpha_used,
                                          float* dz, int64_t eg_ld)
@@ -329,49 +391,61 @@ __device__ __forceinline__ void eg_store(const EgEdge<H>& x, const float (&o)[H]
 #pragma unroll
     for (int h = 0; h < H; ++h)
         au[h] = __uint_as_float(__float_as_uint(x.a[h]) & ~NEG_FLAG) * ((x.keep >> h) & 1 ? keep_scale : 0.f);
-    store_vecH<H>(alpha_used + int64_t(x.pos) * eg_ld, au);
-    store_vecH<H>(dz + int64_t(x.pos) * eg_ld, o);
+    if (eg_ld < 0) {
+        store_vecH_wide<H>(alpha_used - int64_t(x.pos) * eg_ld, au);
+        store_vecH_wide<H>(dz - int64_t(x.pos) * eg_ld, o);
+    } else {
+        store_vecH<H>(alpha_used + int64_t(x.pos) * eg_ld, au);
+        store_vecH<H>(dz + int64_t(x.pos) * eg_ld, o);
+    }
 }
-// second sweep of a row (or hub chunk) whose t is known: the edges are loaded again, alpha_used and dz go to the
-// slots, da_dst is summed lane-locally
+// second sweep of a row (or hub chunk) whose t is known: the edges are read again, one chunk ahead as in the first
+// sweep; alpha_used and dz go to the slots, da_dst is summed lane-locally
 template <int H, bool DROPOUT>
-__device__ __forceinline__ void eg_sweep2(int64_t row, int beg, int end, const int32_t* __restrict__ col,
-                                          const int32_t* __restrict__ perm, const int32_t* __restrict__ csr2csc,
-                                          const float* __restrict__ a_src, const float* __restrict__ a_dst,
+__device__ __forceinline__ void eg_sweep2(int64_t row, int beg, int end, const int32_t* __restrict__ perm,
+                                          const int32_t* __restrict__ csr2csc, const float* __restrict__ a_dst,
                                           const float* __restrict__ rowmax, const float* __restrict__ rowsum,
                                           KeepMask keep, float keep_scale, float slope, const float (&t)[H],
-                                          const float* __restrict__ d_alpha, float* alpha_used, float* dz,
-                                          int64_t eg_ld, float (&dad)[H], int lane)
+                                          const float* __restrict__ rec, float* alpha_used, float* dz, int64_t eg_ld,
+                                          float (&dad)[H], int lane)
 {
-    for (int e = beg + lane; e < end; e += 32) {
-        EgEdge<H> x;
-        eg_load<H, DROPOUT>(x, e, true, row, col, perm, csr2csc, a_src, a_dst, rowmax, rowsum, slope, keep, d_alpha);
-        float o[H];
+    EgRaw<H> r0, r1;
+    eg_fetch<H, DROPOUT>(r0, beg + lane, beg + lane < end, perm, csr2csc, rec);
+    for (int base = beg; base < end; base += 32) {
+        const bool more = base + 32 < end;
+        if (more) eg_fetch<H, DROPOUT>(r1, base + 32 + lane, base + 32 + lane < end, perm, csr2csc, rec);
+        if (base + lane < end) {
+            EgEdge<H> x;
+            eg_finish<H, DROPOUT>(x, r0, true, row, a_dst, rowmax, rowsum, slope, keep);
+            float o[H];
 #pragma unroll
-        for (int h = 0; h < H; ++h) {
-            const EgHead v = eg_head<H>(x, h, true, slope, keep_scale);
-            o[h] = v.sl * (v.u - v.alpha * t[h]);
-            dad[h] += o[h];
+            for (int h = 0; h < H; ++h) {
+                const EgHead v = eg_head<H>(x, h, true, slope, keep_scale);
+                o[h] = v.sl * (v.u - v.alpha * t[h]);
+                dad[h] += o[h];
+            }
+            eg_store<H>(x, o, keep_scale, alpha_used, dz, eg_ld);
         }
-        eg_store<H>(x, o, keep_scale, alpha_used, dz, eg_ld);
+        if (more) r0 = r1;
     }
 }
 
 // one warp per edge-balanced work item over rowptr; the chunk and pack sequence of gat_bwd_dst_items_pack, with the
-// next chunk's contiguous loads (eg_fetch) in flight while the current one is finished and reduced
+// next chunk's records (eg_fetch_async, into a per-warp shared-memory stage) and row statistics in flight while the
+// current one is finished and reduced
 template <int H, bool DROPOUT>
 __global__ void __launch_bounds__(ROW_THREADS, 2)
-gat_bwd_dst_eg_items(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
-                     const int32_t* __restrict__ perm, const int32_t* __restrict__ csr2csc,
-                     const float* __restrict__ a_src, const float* __restrict__ a_dst,
-                     const float* __restrict__ rowmax, const float* __restrict__ rowsum,
-                     const float* __restrict__ d_alpha, gnnfd_item_plan_t items, int hub_threshold, float slope,
-                     KeepMask keep, float keep_scale, float* alpha_used, float* dz, int64_t eg_ld,
-                     float* __restrict__ da_dst)
+gat_bwd_dst_eg_items(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ perm,
+                     const int32_t* __restrict__ csr2csc, const float* __restrict__ a_dst,
+                     const float* __restrict__ rowmax, const float* __restrict__ rowsum, const float* __restrict__ rec,
+                     gnnfd_item_plan_t items, int hub_threshold, float slope, KeepMask keep, float keep_scale,
+                     float* alpha_used, float* dz, int64_t eg_ld, float* __restrict__ da_dst)
 {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int item = blockIdx.x * ROW_WARPS + warp;
+    __shared__ __align__(16) EgStage<H> stage_sh[ROW_WARPS][2];
     if (item >= items.n_items) return;
+    EgStage<H>* stage = stage_sh[warp];
     ChunkCursor cur;
     cur.start_rows(items.item_start[item], items.item_start[item + 1], hub_threshold);
     auto on_empty = [&](int r) {
@@ -383,8 +457,8 @@ gat_bwd_dst_eg_items(const int32_t* __restrict__ rowptr, const int32_t* __restri
     int kind0 = cur.next_any(rowptr, lane, c0.row, c0.beg, c0.n, c0.first, c0.last, k0, la, lb, on_empty);
     if (!kind0) return;
     if (kind0 == 2) pack_lane_segment(c0.beg, k0, la, lb, lane, lo0, sa0, sb0);
-    EgRaw<H> r0, r1;
-    eg_fetch<H, DROPOUT>(r0, c0.beg + lane, lane < c0.n, col, perm, csr2csc, d_alpha);
+    int b = 0;                   // stage of c0
+    eg_fetch_async<H, DROPOUT>(stage[0], c0.beg + lane, lane < c0.n, perm, csr2csc, rec, lane);
     float trow[H];               // running t = sum alpha*d_alpha of the current (multi-chunk) row
     int row_beg = c0.beg;        // first edge of the current row
 #pragma unroll
@@ -393,9 +467,19 @@ gat_bwd_dst_eg_items(const int32_t* __restrict__ rowptr, const int32_t* __restri
         const int kind1 = cur.next_any(rowptr, lane, c1.row, c1.beg, c1.n, c1.first, c1.last, k1, la, lb, on_empty);
         lo1 = 0;
         if (kind1 == 2) pack_lane_segment(c1.beg, k1, la, lb, lane, lo1, sa1, sb1);
-        if (kind1) eg_fetch<H, DROPOUT>(r1, c1.beg + lane, lane < c1.n, col, perm, csr2csc, d_alpha);
+        if (kind1) {
+            if (lane < c1.n) eg_prefetch_row<H>(c1.row + lo1, a_dst, rowmax, rowsum);
+            eg_fetch_async<H, DROPOUT>(stage[b ^ 1], c1.beg + lane, lane < c1.n, perm, csr2csc, rec, lane);
+        } else {
+            cp_async_commit();   // an empty group, so that c0's group is always the one before the newest
+        }
+        cp_async_wait_pending(1);
         EgEdge<H> x0;
-        eg_finish<H, DROPOUT>(x0, r0, lane < c0.n, c0.row + lo0, a_src, a_dst, rowmax, rowsum, slope, keep);
+        {
+            EgRaw<H> r0;
+            eg_take<H, DROPOUT>(r0, stage[b], lane < c0.n, lane);
+            eg_finish<H, DROPOUT>(x0, r0, lane < c0.n, c0.row + lo0, a_dst, rowmax, rowsum, slope, keep);
+        }
         if (c0.first) {
             row_beg = c0.beg;
 #pragma unroll
@@ -437,33 +521,31 @@ gat_bwd_dst_eg_items(const int32_t* __restrict__ rowptr, const int32_t* __restri
                 float dad[H];
 #pragma unroll
                 for (int h = 0; h < H; ++h) dad[h] = 0.f;
-                eg_sweep2<H, DROPOUT>(c0.row, row_beg, c0.beg + c0.n, col, perm, csr2csc, a_src, a_dst, rowmax, rowsum,
-                                      keep, keep_scale, slope, trow, d_alpha, alpha_used, dz, eg_ld, dad, lane);
+                eg_sweep2<H, DROPOUT>(c0.row, row_beg, c0.beg + c0.n, perm, csr2csc, a_dst, rowmax, rowsum, keep,
+                                      keep_scale, slope, trow, rec, alpha_used, dz, eg_ld, dad, lane);
 #pragma unroll
                 for (int h = 0; h < H; ++h) dad[h] = warp_sum(dad[h]);
                 if (lane == 0) store_vecH<H>(da_dst + int64_t(c0.row) * H, dad);
             }
         }
         if (!kind1) break;
+        b ^= 1;
         c0 = c1;
         kind0 = kind1;
         k0 = k1;
         sa0 = sa1;
         sb0 = sb1;
         lo0 = lo1;
-        r0 = r1;
     }
 }
 
 // hub rows, step 1: one warp per chunk -- partial t of the chunk
 template <int H, bool DROPOUT>
 __global__ void __launch_bounds__(ROW_THREADS)
-gat_bwd_dst_eg_hub1(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
-                    const int32_t* __restrict__ perm, const int32_t* __restrict__ csr2csc,
-                    const float* __restrict__ a_src, const float* __restrict__ a_dst,
-                    const float* __restrict__ rowmax, const float* __restrict__ rowsum,
-                    const float* __restrict__ d_alpha, gnnfd_hub_plan_t plan, float slope, KeepMask keep,
-                    float keep_scale, float* __restrict__ part_t)
+gat_bwd_dst_eg_hub1(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ perm,
+                    const int32_t* __restrict__ csr2csc, const float* __restrict__ a_dst,
+                    const float* __restrict__ rowmax, const float* __restrict__ rowsum, const float* __restrict__ rec,
+                    gnnfd_hub_plan_t plan, float slope, KeepMask keep, float keep_scale, float* __restrict__ part_t)
 {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int c = blockIdx.x * ROW_WARPS + warp;
@@ -475,13 +557,17 @@ gat_bwd_dst_eg_hub1(const int32_t* __restrict__ rowptr, const int32_t* __restric
     float trow[H];
 #pragma unroll
     for (int h = 0; h < H; ++h) trow[h] = 0.f;
+    EgRaw<H> r0, r1;
+    eg_fetch<H, DROPOUT>(r0, beg + lane, beg + lane < end, perm, csr2csc, rec);
     for (int base = beg; base < end; base += 32) {
+        const bool more = base + 32 < end;
+        if (more) eg_fetch<H, DROPOUT>(r1, base + 32 + lane, base + 32 + lane < end, perm, csr2csc, rec);
         const bool live = base + lane < end;
         EgEdge<H> x;
-        eg_load<H, DROPOUT>(x, base + lane, live, i, col, perm, csr2csc, a_src, a_dst, rowmax, rowsum, slope, keep,
-                            d_alpha);
+        eg_finish<H, DROPOUT>(x, r0, live, i, a_dst, rowmax, rowsum, slope, keep);
 #pragma unroll
         for (int h = 0; h < H; ++h) trow[h] += warp_sum(eg_head<H>(x, h, live, slope, keep_scale).u);
+        if (more) r0 = r1;
     }
     if (lane == 0) store_vecH<H>(part_t + int64_t(c) * H, trow);
 }
@@ -489,12 +575,11 @@ gat_bwd_dst_eg_hub1(const int32_t* __restrict__ rowptr, const int32_t* __restric
 // hub rows, step 2: the row's total t (chunk order), second sweep, partial da_dst
 template <int H, bool DROPOUT>
 __global__ void __launch_bounds__(ROW_THREADS)
-gat_bwd_dst_eg_hub2(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
-                    const int32_t* __restrict__ perm, const int32_t* __restrict__ csr2csc,
-                    const float* __restrict__ a_src, const float* __restrict__ a_dst,
-                    const float* __restrict__ rowmax, const float* __restrict__ rowsum,
-                    const float* __restrict__ d_alpha, gnnfd_hub_plan_t plan, float slope, KeepMask keep,
-                    float keep_scale, const float* __restrict__ t_total, float* alpha_used, float* dz, int64_t eg_ld,
+gat_bwd_dst_eg_hub2(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ perm,
+                    const int32_t* __restrict__ csr2csc, const float* __restrict__ a_dst,
+                    const float* __restrict__ rowmax, const float* __restrict__ rowsum, const float* __restrict__ rec,
+                    gnnfd_hub_plan_t plan, float slope, KeepMask keep, float keep_scale,
+                    const float* __restrict__ t_total, float* alpha_used, float* dz, int64_t eg_ld,
                     float* __restrict__ part_dad)
 {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -508,15 +593,15 @@ gat_bwd_dst_eg_hub2(const int32_t* __restrict__ rowptr, const int32_t* __restric
     load_vecH<H>(t_total + int64_t(slot) * H, t);
 #pragma unroll
     for (int h = 0; h < H; ++h) dad[h] = 0.f;
-    eg_sweep2<H, DROPOUT>(i, beg, end, col, perm, csr2csc, a_src, a_dst, rowmax, rowsum, keep, keep_scale, slope, t,
-                          d_alpha, alpha_used, dz, eg_ld, dad, lane);
+    eg_sweep2<H, DROPOUT>(i, beg, end, perm, csr2csc, a_dst, rowmax, rowsum, keep, keep_scale, slope, t, rec,
+                          alpha_used, dz, eg_ld, dad, lane);
 #pragma unroll
     for (int h = 0; h < H; ++h) dad[h] = warp_sum(dad[h]);
     if (lane == 0) store_vecH<H>(part_dad + int64_t(c) * H, dad);
 }
 
 struct EgArgs {
-    const float *a_src, *a_dst, *rowmax, *rowsum, *d_alpha;
+    const float *a_dst, *rowmax, *rowsum, *rec;
 };
 template <class GE, bool DROPOUT>
 static void launch_dst_eg(const gnnfd_graph_t* g, const EgArgs& in, float slope, KeepMask keep, float ks,
@@ -526,32 +611,30 @@ static void launch_dst_eg(const gnnfd_graph_t* g, const EgArgs& in, float slope,
     constexpr int H = GE::H;
     const int thr = g->hub_dst.n_hub > 0 ? g->hub_dst.threshold : INT_MAX;
     const unsigned grid = (unsigned)((g->items_dst.n_items + ROW_WARPS - 1) / ROW_WARPS);
-    gat_bwd_dst_eg_items<H, DROPOUT><<<grid, ROW_THREADS, 0, st>>>(g->rowptr, g->col, g->perm, g->csr2csc, in.a_src,
-                                                                    in.a_dst, in.rowmax, in.rowsum, in.d_alpha,
-                                                                    g->items_dst, thr, slope, keep, ks, alpha_used, dz,
-                                                                    eg_ld, da_dst);
+    gat_bwd_dst_eg_items<H, DROPOUT><<<grid, ROW_THREADS, 0, st>>>(g->rowptr, g->perm, g->csr2csc, in.a_dst, in.rowmax,
+                                                                    in.rowsum, in.rec, g->items_dst, thr, slope, keep,
+                                                                    ks, alpha_used, dz, eg_ld, da_dst);
     g_launches += 1;
     if (g->hub_dst.n_hub > 0) {
         const gnnfd_hub_plan_t& pl = g->hub_dst;
         const unsigned gh = (unsigned)((pl.n_hub + ROW_WARPS - 1) / ROW_WARPS);
         const unsigned gc = (unsigned)((pl.n_chunk + ROW_WARPS - 1) / ROW_WARPS);
-        gat_bwd_dst_eg_hub1<H, DROPOUT><<<gc, ROW_THREADS, 0, st>>>(g->rowptr, g->col, g->perm, g->csr2csc, in.a_src,
-                                                                     in.a_dst, in.rowmax, in.rowsum, in.d_alpha, pl,
-                                                                     slope, keep, ks, part_t);
+        gat_bwd_dst_eg_hub1<H, DROPOUT><<<gc, ROW_THREADS, 0, st>>>(g->rowptr, g->perm, g->csr2csc, in.a_dst,
+                                                                     in.rowmax, in.rowsum, in.rec, pl, slope, keep, ks,
+                                                                     part_t);
         gat_hub_chunk_sum<H, false><<<gh, ROW_THREADS, 0, st>>>(pl, part_t, t_total);
-        gat_bwd_dst_eg_hub2<H, DROPOUT><<<gc, ROW_THREADS, 0, st>>>(g->rowptr, g->col, g->perm, g->csr2csc, in.a_src,
-                                                                     in.a_dst, in.rowmax, in.rowsum, in.d_alpha, pl,
-                                                                     slope, keep, ks, t_total, alpha_used, dz, eg_ld,
-                                                                     part_dad);
+        gat_bwd_dst_eg_hub2<H, DROPOUT><<<gc, ROW_THREADS, 0, st>>>(g->rowptr, g->perm, g->csr2csc, in.a_dst,
+                                                                     in.rowmax, in.rowsum, in.rec, pl, slope, keep, ks,
+                                                                     t_total, alpha_used, dz, eg_ld, part_dad);
         gat_hub_chunk_sum<H, true><<<gh, ROW_THREADS, 0, st>>>(pl, part_dad, da_dst);
         g_launches += 4;
     }
 }
 
-// workspace of the two-pass form: d_alpha [E',H] in CSR order, then the hub_dst partials
+// workspace of the two-pass form: the records {d_alpha, a_src[j]} [E',2H] in CSR order, then the hub_dst partials
 size_t gat_bwd_dst_srcmajor_ws_bytes(const gnnfd_graph_t* g, int H)
 {
-    size_t b = carve_bytes(size_t(g->n_edges) * H, 4);
+    size_t b = carve_bytes(size_t(g->n_edges) * 2 * H, 4);
     if (g->hub_dst.n_hub > 0)
         b += 2 * carve_bytes(size_t(g->hub_dst.n_chunk) * H, 4) + carve_bytes(size_t(g->hub_dst.n_hub) * H, 4);
     return b;
@@ -570,11 +653,14 @@ static int launch_bwd_dst_srcmajor(const gnnfd_graph_t* g, const void* xw_, cons
     GNNFD_REQUIRE(g->items_dst.n_items > 0 && g->items_dst.item_start, GNNFD_ERR_ARG,
                   "gat_bwd_dst: the graph has no work-item plan over rowptr (gnnfd_item_plan)");
     // two dense [E',H] arrays, or the halves of one interleaved [E',2H] buffer (dz == alpha_used + H)
-    const int64_t eg_ld = (dz == alpha_used + H) ? 2 * H : H;
+    const int64_t ld = (dz == alpha_used + H) ? 2 * H : H;
+    // 32-byte-aligned slots take one 256-bit store per vector; eg_store reads that from the sign of eg_ld
+    const bool wide = ((reinterpret_cast<uintptr_t>(alpha_used) | reinterpret_cast<uintptr_t>(dz)) & 31) == 0;
+    const int64_t eg_ld = wide ? -ld : ld;
     const size_t need = gat_bwd_dst_srcmajor_ws_bytes(g, H);
     GNNFD_REQUIRE(ws && ws_bytes >= need, GNNFD_ERR_WORKSPACE, "gat_bwd_dst: workspace %zu < %zu", ws_bytes, need);
     char* p = reinterpret_cast<char*>(ws);
-    float* d_alpha = carve<float>(p, size_t(g->n_edges) * H);
+    float* rec = carve<float>(p, size_t(g->n_edges) * 2 * H);
     float *part_t = nullptr, *part_dad = nullptr, *t_total = nullptr;
     if (g->hub_dst.n_hub > 0) {
         const gnnfd_hub_plan_t& pl = g->hub_dst;
@@ -587,19 +673,19 @@ static int launch_bwd_dst_srcmajor(const gnnfd_graph_t* g, const void* xw_, cons
         GNNFD_CUDA(cudaFuncSetAttribute(gat_bwd_dalpha_src_stream<GE>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
         const int thr = g->hub_src.n_hub > 0 ? g->hub_src.threshold : INT_MAX;
         const unsigned grid = (unsigned)((g->items_src.n_items + DA_WARPS - 1) / DA_WARPS);
-        gat_bwd_dalpha_src_stream<GE><<<grid, DA_THREADS, SMEM, st>>>(g->colptr, g->csc_row, g->csc_eid, xw, d_out,
-                                                                      g->items_src, thr, d_alpha);
+        gat_bwd_dalpha_src_stream<GE><<<grid, DA_THREADS, SMEM, st>>>(g->colptr, g->csc_row, g->csc_eid, xw, a_src,
+                                                                      d_out, g->items_src, thr, rec);
         g_launches += 1;
         if (g->hub_src.n_hub > 0) {
             const unsigned gc = (unsigned)((g->hub_src.n_chunk + DA_WARPS - 1) / DA_WARPS);
-            gat_bwd_dalpha_src_hub<GE><<<gc, DA_THREADS, 0, st>>>(g->colptr, g->csc_row, g->csc_eid, xw, d_out,
-                                                                   g->hub_src, d_alpha);
+            gat_bwd_dalpha_src_hub<GE><<<gc, DA_THREADS, 0, st>>>(g->colptr, g->csc_row, g->csc_eid, xw, a_src, d_out,
+                                                                   g->hub_src, rec);
             g_launches += 1;
         }
     }
     float ks = 1.f;
     const KeepMask keep = make_keep(keep_mask, p_drop, seed, &ks);
-    const EgArgs in{a_src, a_dst, rowmax, rowsum, d_alpha};
+    const EgArgs in{a_dst, rowmax, rowsum, rec};
     if (p_drop > 0.f)
         launch_dst_eg<GE, true>(g, in, slope, keep, ks, alpha_used, dz, eg_ld, da_dst, part_t, part_dad, t_total, st);
     else

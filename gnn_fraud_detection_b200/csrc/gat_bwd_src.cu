@@ -296,7 +296,7 @@ int gnnfd_gat_bwd_workspace_bytes(const gnnfd_graph_t* g, int H, int C, size_t* 
 {
     GNNFD_REQUIRE(g && bytes, GNNFD_ERR_ARG, "gat_bwd_workspace_bytes: NULL argument");
     const size_t nd = (size_t)g->hub_dst.n_chunk, ns = (size_t)g->hub_src.n_chunk;
-    // the dst pass: its two-pass form (head mean) also keeps d_alpha [E',H] here; concat is not known at this point
+    // the dst pass: its two-pass form (head mean) also keeps the [E',2H] records here; concat is not known at this point
     const size_t a = gat_bwd_dst_srcmajor_applies(g, 0) ? gat_bwd_dst_srcmajor_ws_bytes(g, H)
                                                         : 2 * carve_bytes(nd * H, 4) + carve_bytes(size_t(g->hub_dst.n_hub) * H, 4);
     const size_t b = carve_bytes(ns * size_t(H) * C, 4) + carve_bytes(ns * H, 4);

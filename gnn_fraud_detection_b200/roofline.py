@@ -35,10 +35,12 @@ def stage_bytes(N: int, Ep: int, K: int, H: int = 8, C: int = 64, concat: bool =
         b["gat_bwd_dst"] = Ep * (D * s + i + 4 * H + 4 * H) + N * (4 * Co + 8 * H + 4 * H + i)
     else:
         # head mean, two passes (DESIGN 4.4).  Source-major d_alpha stream -- per edge: csc_row, csc_eid, dOut[dst]
-        # row, d_alpha write (CSR position); per source row: xw row, colptr.  Dst pass -- per edge: col, a_src[src],
-        # d_alpha read, csr2csc, (alpha_used, dz) write; per row: (a_dst,max,sum), da_dst, rowptr
-        b["gat_bwd_dst"] = (Ep * (2 * i + 4 * Co + 4 * H) + Ns * (D * s + i)
-                            + Ep * (i + 4 * H + 4 * H + i + 8 * H) + N * (12 * H + 4 * H + i))
+        # row, record {d_alpha, a_src[src]} write (CSR position); per source row: xw row, a_src, colptr.  Dst pass --
+        # per edge: record read, csr2csc, (alpha_used, dz) write; per row: (a_dst,max,sum), da_dst, rowptr.  The record
+        # costs 4H B more per edge than a bare d_alpha and saves the col read, but it turns the dst pass's one random
+        # gather (a_src[col[e]]) into a contiguous stream
+        b["gat_bwd_dst"] = (Ep * (2 * i + 4 * Co + 8 * H) + Ns * (D * s + 4 * H + i)
+                            + Ep * (8 * H + i + 8 * H) + N * (12 * H + 4 * H + i))
     # per edge: dOut[dst] row, (csc_row, csc_eid), alpha, dz; per source row: dxw write, da_src write, colptr
     b["gat_bwd_src"] = Ep * (4 * Co + 2 * i + 4 * H + 4 * H) + Ns * (D * 4 + 4 * H + i)
     # GEMM-bwd: read dxw, xw, x (+ dx write), da_src/da_dst; W read + dW write
