@@ -36,6 +36,13 @@ constexpr int DA_THREADS = DA_WARPS * 32;
 constexpr int DA_RING = 32;                  // dO row slots per warp (pass 1 stream): a whole 32-edge task fits
 constexpr int DA_XROWS = 2;                  // xw row slots per warp (pass 1 stream)
 constexpr int DA_TASKS = 8;                  // tasks in flight per warp at most (cp.async groups)
+// warps per CTA of the hub kernel, which stages 32 dO rows per warp in static shared memory: 8 KB per warp at C = 64;
+// at C = 128 two warps keep the 16 KB per warp under the 48 KB static limit
+template <class GE>
+constexpr int da_hub_warps()
+{
+    return GE::C > 64 ? 2 : DA_WARPS;
+}
 
 __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc)
 {
@@ -225,17 +232,18 @@ gat_bwd_dalpha_src_stream(const int32_t* __restrict__ colptr, const int32_t* __r
 
 // one warp per chunk of a hub source row: xw[j] in registers, per 32 edges the dO rows staged with cp.async
 template <class GE>
-__global__ void __launch_bounds__(DA_THREADS, 6)
+__global__ void __launch_bounds__(32 * da_hub_warps<GE>(), 6)
 gat_bwd_dalpha_src_hub(const int32_t* __restrict__ colptr, const int32_t* __restrict__ csc_row,
                        const int32_t* __restrict__ csc_eid, const typename GE::XT* __restrict__ xw,
                        const float* __restrict__ a_src, const float* __restrict__ d_out, gnnfd_hub_plan_t plan,
                        float* __restrict__ rec)
 {
     constexpr int H = GE::H, NS = GE::NS, VW = GE::VW, C = GE::C;
-    __shared__ __align__(16) float do_sh[DA_WARPS][32 * C];
-    __shared__ __align__(16) float dal_sh[DA_WARPS][32 * H];
+    constexpr int W = da_hub_warps<GE>();
+    __shared__ __align__(16) float do_sh[W][32 * C];
+    __shared__ __align__(16) float dal_sh[W][32 * H];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int c = blockIdx.x * DA_WARPS + warp;
+    const int c = blockIdx.x * W + warp;
     if (c >= plan.n_chunk) return;
     const int slot = plan.chunk_hub[c];
     const int64_t j = plan.hub_row[slot];
@@ -677,8 +685,9 @@ static int launch_bwd_dst_srcmajor(const gnnfd_graph_t* g, const void* xw_, cons
                                                                       d_out, g->items_src, thr, rec);
         g_launches += 1;
         if (g->hub_src.n_hub > 0) {
-            const unsigned gc = (unsigned)((g->hub_src.n_chunk + DA_WARPS - 1) / DA_WARPS);
-            gat_bwd_dalpha_src_hub<GE><<<gc, DA_THREADS, 0, st>>>(g->colptr, g->csc_row, g->csc_eid, xw, a_src, d_out,
+            constexpr int HW = da_hub_warps<GE>();
+            const unsigned gc = (unsigned)((g->hub_src.n_chunk + HW - 1) / HW);
+            gat_bwd_dalpha_src_hub<GE><<<gc, 32 * HW, 0, st>>>(g->colptr, g->csc_row, g->csc_eid, xw, a_src, d_out,
                                                                    g->hub_src, rec);
             g_launches += 1;
         }
@@ -720,8 +729,14 @@ int gat_bwd_dst_srcmajor(const gnnfd_graph_t* g, const void* xw, int xw_dtype, i
     if (H == 4 && C == 32 && xw_dtype == GNNFD_F32)
         return launch_bwd_dst_srcmajor<Geo<4, 32, float>>(g, xw, a_src, a_dst, rowmax, rowsum, d_out, negative_slope,
                                                           keep_mask, p_drop, seed, alpha_used, dz, da_dst, ws, ws_bytes, st);
-    GNNFD_REQUIRE(false, GNNFD_ERR_UNSUPPORTED, "gat_bwd_dst: (heads=%d, out_channels=%d, dtype=%d) is not built", H, C,
-                  xw_dtype);
+    if (H == 8 && C == 32 && xw_dtype == GNNFD_F32)
+        return launch_bwd_dst_srcmajor<Geo<8, 32, float>>(g, xw, a_src, a_dst, rowmax, rowsum, d_out, negative_slope,
+                                                          keep_mask, p_drop, seed, alpha_used, dz, da_dst, ws, ws_bytes, st);
+    if (H == 8 && C == 128 && xw_dtype == GNNFD_F32)
+        return launch_bwd_dst_srcmajor<Geo<8, 128, float>>(g, xw, a_src, a_dst, rowmax, rowsum, d_out, negative_slope,
+                                                           keep_mask, p_drop, seed, alpha_used, dz, da_dst, ws, ws_bytes, st);
+    GNNFD_REQUIRE(false, GNNFD_ERR_UNSUPPORTED, "gat_bwd_dst: (heads=%d, out_channels=%d, dtype=%d) is not built; "
+                  "available: (8,64,f32), (8,64,bf16), (8,32,f32), (8,128,f32), (4,32,f32)", H, C, xw_dtype);
     return GNNFD_ERR_UNSUPPORTED;
 }
 

@@ -197,7 +197,7 @@ __device__ __forceinline__ void bwd_dst_stream(ChunkCursor& cur, WarpRing<GE, bw
 }
 
 template <class GE, bool CONCAT, bool DROPOUT>
-__global__ void __launch_bounds__(ST_THREADS, 4)
+__global__ void __launch_bounds__(ST_THREADS, st_min_ctas<GE>())
 gat_bwd_dst_items(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col, const int32_t* __restrict__ perm,
                   const int32_t* __restrict__ csr2csc, const typename GE::XT* __restrict__ xw, const float* __restrict__ a_src,
                   const float* __restrict__ a_dst, const float* __restrict__ rowmax, const float* __restrict__ rowsum,
@@ -393,7 +393,7 @@ __device__ __forceinline__ void bwd_dst_stream_pack(ChunkCursor& cur, WarpRing<G
 }
 
 template <class GE, bool CONCAT, bool DROPOUT>
-__global__ void __launch_bounds__(ST_THREADS, 4)
+__global__ void __launch_bounds__(ST_THREADS, st_min_ctas<GE>())
 gat_bwd_dst_items_pack(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col, const int32_t* __restrict__ perm,
                        const int32_t* __restrict__ csr2csc, const typename GE::XT* __restrict__ xw, const float* __restrict__ a_src,
                        const float* __restrict__ a_dst, const float* __restrict__ rowmax, const float* __restrict__ rowsum,
@@ -415,7 +415,7 @@ gat_bwd_dst_items_pack(const int32_t* __restrict__ rowptr, const int32_t* __rest
 
 // hub rows, step 1: one warp per chunk -- first sweep, partial t
 template <class GE, bool CONCAT, bool DROPOUT>
-__global__ void __launch_bounds__(ST_THREADS, 4)
+__global__ void __launch_bounds__(ST_THREADS, st_min_ctas<GE>())
 gat_bwd_dst_hub1(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col, const int32_t* __restrict__ perm,
                  const int32_t* __restrict__ csr2csc, const typename GE::XT* __restrict__ xw, const float* __restrict__ a_src,
                  const float* __restrict__ a_dst, const float* __restrict__ rowmax, const float* __restrict__ rowsum,
@@ -554,8 +554,14 @@ int gnnfd_gat_bwd_dst(const gnnfd_graph_t* g, const void* xw, int xw_dtype, cons
     if (H == 4 && C == 32 && xw_dtype == GNNFD_F32)
         return launch_bwd_dst<Geo<4, 32, float>>(g, xw, a_src, a_dst, rowmax, rowsum, d_out, negative_slope, concat,
                                                  keep_mask, p_drop, dropout_seed, alpha_used, dz, da_dst, ws, ws_bytes, st);
-    GNNFD_REQUIRE(false, GNNFD_ERR_UNSUPPORTED, "gat_bwd_dst: (heads=%d, out_channels=%d, dtype=%d) is not built", H, C,
-                  xw_dtype);
+    if (H == 8 && C == 32 && xw_dtype == GNNFD_F32)
+        return launch_bwd_dst<Geo<8, 32, float>>(g, xw, a_src, a_dst, rowmax, rowsum, d_out, negative_slope, concat,
+                                                 keep_mask, p_drop, dropout_seed, alpha_used, dz, da_dst, ws, ws_bytes, st);
+    if (H == 8 && C == 128 && xw_dtype == GNNFD_F32)
+        return launch_bwd_dst<Geo<8, 128, float>>(g, xw, a_src, a_dst, rowmax, rowsum, d_out, negative_slope, concat,
+                                                  keep_mask, p_drop, dropout_seed, alpha_used, dz, da_dst, ws, ws_bytes, st);
+    GNNFD_REQUIRE(false, GNNFD_ERR_UNSUPPORTED, "gat_bwd_dst: (heads=%d, out_channels=%d, dtype=%d) is not built; "
+                  "available: (8,64,f32), (8,64,bf16), (8,32,f32), (8,128,f32), (4,32,f32)", H, C, xw_dtype);
     return GNNFD_ERR_UNSUPPORTED;
 }
 

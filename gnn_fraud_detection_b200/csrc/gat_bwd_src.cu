@@ -25,6 +25,18 @@ size_t gat_bwd_dst_srcmajor_ws_bytes(const gnnfd_graph_t* g, int H);
 #define GNNFD_SRC_U 4
 #endif
 constexpr int BWD_U = GNNFD_SRC_U;
+// The rows kernel at 8 x 128 channels (32 accumulators per lane): two CTAs per SM instead of GNNFD_SRC_MINB, and
+// with concat one dO row in flight per lane instead of BWD_U (each is 32 more registers), so that nothing spills.
+template <class GE>
+constexpr int src_minb()
+{
+    return GE::D > 512 ? 2 : GNNFD_SRC_MINB;
+}
+template <class GE, bool CONCAT>
+constexpr int src_unroll()
+{
+    return (GE::D > 512 && CONCAT) ? 1 : BWD_U;
+}
 
 // ---------------------------------------------------------------------------------------------------------
 // src-major pass
@@ -35,7 +47,7 @@ __device__ __forceinline__ void src_range(int beg, int end, const int32_t* __res
                                           const float* __restrict__ dz, int64_t eg_ld, const float* __restrict__ d_out,
                                           float (&acc)[GE::NS][4], float (&das)[GE::H], float* p_s, int* i_s, int lane)
 {
-    constexpr int H = GE::H, NS = GE::NS, HP = GE::HP, D = GE::D, C = GE::C;
+    constexpr int H = GE::H, NS = GE::NS, HP = GE::HP, D = GE::D, C = GE::C, U = src_unroll<GE, CONCAT>();
     const int sub = lane / GE::G;
     const int cm = (4 * lane) % C;   // C divides 128, so every slot of this lane has the same channel offset
     for (int base = beg; base < end; base += 32) {
@@ -54,10 +66,10 @@ __device__ __forceinline__ void src_range(int beg, int end, const int32_t* __res
         }
         i_s[lane] = i;
         __syncwarp();
-        for (int t = 0; t < n; t += BWD_U) {
-            float g[BWD_U][CONCAT ? NS : 1][4], wq[BWD_U][NS];
+        for (int t = 0; t < n; t += U) {
+            float g[U][CONCAT ? NS : 1][4], wq[U][NS];
 #pragma unroll
-            for (int uu = 0; uu < BWD_U; ++uu) {
+            for (int uu = 0; uu < U; ++uu) {
                 const bool ok = t + uu < n;
                 const int tt = ok ? t + uu : t;
                 const int64_t ii = i_s[tt];
@@ -72,7 +84,7 @@ __device__ __forceinline__ void src_range(int beg, int end, const int32_t* __res
                 for (int q = 0; q < NS; ++q) wq[uu][q] = ok ? p_s[tt * H + q * HP + sub] : 0.f;
             }
 #pragma unroll
-            for (int uu = 0; uu < BWD_U; ++uu)
+            for (int uu = 0; uu < U; ++uu)
 #pragma unroll
                 for (int q = 0; q < NS; ++q)
 #pragma unroll
@@ -114,7 +126,7 @@ __device__ __forceinline__ void src_epilogue(int64_t j, float (&acc)[GE::NS][4],
 }
 
 template <class GE, bool CONCAT>
-__global__ void __launch_bounds__(ROW_THREADS, GNNFD_SRC_MINB)
+__global__ void __launch_bounds__(ROW_THREADS, src_minb<GE>())
 gat_bwd_src_rows(const int32_t* __restrict__ colptr, const int32_t* __restrict__ csc_row,
                  const int32_t* __restrict__ csc_eid, const float* __restrict__ alpha_used,
                  const float* __restrict__ dz, int64_t eg_ld, const float* __restrict__ d_out, const float* __restrict__ att_src,
@@ -319,7 +331,14 @@ int gnnfd_gat_bwd_src(const gnnfd_graph_t* g, const float* alpha_used, const flo
     if (H == 4 && C == 32)
         return launch_bwd_src<Geo<4, 32, float>>(g, alpha_used, dz, d_out, att_src, att_dst, da_dst_full, concat, dxw,
                                                  da_src, ws, ws_bytes, st);
-    GNNFD_REQUIRE(false, GNNFD_ERR_UNSUPPORTED, "gat_bwd_src: (heads=%d, out_channels=%d) is not built", H, C);
+    if (H == 8 && C == 32)
+        return launch_bwd_src<Geo<8, 32, float>>(g, alpha_used, dz, d_out, att_src, att_dst, da_dst_full, concat, dxw,
+                                                 da_src, ws, ws_bytes, st);
+    if (H == 8 && C == 128)
+        return launch_bwd_src<Geo<8, 128, float>>(g, alpha_used, dz, d_out, att_src, att_dst, da_dst_full, concat, dxw,
+                                                  da_src, ws, ws_bytes, st);
+    GNNFD_REQUIRE(false, GNNFD_ERR_UNSUPPORTED, "gat_bwd_src: (heads=%d, out_channels=%d) is not built; "
+                  "available: (8,64), (8,32), (8,128), (4,32)", H, C);
     return GNNFD_ERR_UNSUPPORTED;
 }
 

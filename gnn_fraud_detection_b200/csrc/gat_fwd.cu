@@ -224,7 +224,7 @@ __device__ __forceinline__ void fwd_stream(ChunkCursor& cur, WarpRing<GE>& ring,
 }
 
 template <class GE, bool CONCAT, bool DROPOUT>
-__global__ void __launch_bounds__(ST_THREADS, 4)
+__global__ void __launch_bounds__(ST_THREADS, st_min_ctas<GE>())
 gat_fwd_items(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col, const int32_t* __restrict__ perm,
               const typename GE::XT* __restrict__ xw, const float* __restrict__ a_src,
               const float* __restrict__ a_dst, EpiParams ep, gnnfd_item_plan_t items,
@@ -351,7 +351,7 @@ __device__ __forceinline__ void fwd_stream_pack(ChunkCursor& cur, WarpRing<GE, 2
 }
 
 template <class GE, bool CONCAT, bool DROPOUT>
-__global__ void __launch_bounds__(ST_THREADS, 4)
+__global__ void __launch_bounds__(ST_THREADS, st_min_ctas<GE>())
 gat_fwd_items_pack(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col, const int32_t* __restrict__ perm,
                    const typename GE::XT* __restrict__ xw, const float* __restrict__ a_src,
                    const float* __restrict__ a_dst, EpiParams ep, gnnfd_item_plan_t items,
@@ -372,7 +372,7 @@ gat_fwd_items_pack(const int32_t* __restrict__ rowptr, const int32_t* __restrict
 
 // one warp per (hub row, chunk): partial (m, s, unnormalised acc)
 template <class GE, bool DROPOUT>
-__global__ void __launch_bounds__(ST_THREADS, 4)
+__global__ void __launch_bounds__(ST_THREADS, st_min_ctas<GE>())
 gat_fwd_hub_chunks(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col, const int32_t* __restrict__ perm,
                    const typename GE::XT* __restrict__ xw, const float* __restrict__ a_src,
                    const float* __restrict__ a_dst, gnnfd_hub_plan_t plan, float slope,
@@ -659,8 +659,14 @@ int gnnfd_gat_fwd_fused(const gnnfd_graph_t* g, const void* xw, int xw_dtype, co
     if (H == 4 && C == 32 && xw_dtype == GNNFD_F32)
         return launch_fwd<Geo<4, 32, float>>(g, xw, a_src, a_dst, ep, negative_slope, concat, keep_mask, p_drop, dropout_seed, out, rowmax,
                                              rowsum, ws, ws_bytes, st);
+    if (H == 8 && C == 32 && xw_dtype == GNNFD_F32)
+        return launch_fwd<Geo<8, 32, float>>(g, xw, a_src, a_dst, ep, negative_slope, concat, keep_mask, p_drop, dropout_seed, out, rowmax,
+                                             rowsum, ws, ws_bytes, st);
+    if (H == 8 && C == 128 && xw_dtype == GNNFD_F32)
+        return launch_fwd<Geo<8, 128, float>>(g, xw, a_src, a_dst, ep, negative_slope, concat, keep_mask, p_drop, dropout_seed, out,
+                                              rowmax, rowsum, ws, ws_bytes, st);
     GNNFD_REQUIRE(false, GNNFD_ERR_UNSUPPORTED, "gat_fwd: (heads=%d, out_channels=%d, dtype=%d) is not built; "
-                  "available: (8,64,f32), (8,64,bf16), (4,32,f32)", H, C, xw_dtype);
+                  "available: (8,64,f32), (8,64,bf16), (8,32,f32), (8,128,f32), (4,32,f32)", H, C, xw_dtype);
     return GNNFD_ERR_UNSUPPORTED;
 }
 

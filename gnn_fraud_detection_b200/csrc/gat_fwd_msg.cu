@@ -473,8 +473,14 @@ int gat_fwd_srcmajor(const gnnfd_graph_t* g, const void* xw, int xw_dtype, int H
     if (H == 4 && C == 32 && xw_dtype == GNNFD_F32)
         return launch_fwd_srcmajor<Geo<4, 32, float>>(g, xw, a_src, a_dst, ep, negative_slope, keep_mask, p_drop, seed, out,
                                                       rowmax, rowsum, ws, ws_bytes, st);
+    if (H == 8 && C == 32 && xw_dtype == GNNFD_F32)
+        return launch_fwd_srcmajor<Geo<8, 32, float>>(g, xw, a_src, a_dst, ep, negative_slope, keep_mask, p_drop, seed, out,
+                                                      rowmax, rowsum, ws, ws_bytes, st);
+    if (H == 8 && C == 128 && xw_dtype == GNNFD_F32)
+        return launch_fwd_srcmajor<Geo<8, 128, float>>(g, xw, a_src, a_dst, ep, negative_slope, keep_mask, p_drop, seed, out,
+                                                       rowmax, rowsum, ws, ws_bytes, st);
     GNNFD_REQUIRE(false, GNNFD_ERR_UNSUPPORTED, "gat_fwd: (heads=%d, out_channels=%d, dtype=%d) is not built; "
-                  "available: (8,64,f32), (8,64,bf16), (4,32,f32)", H, C, xw_dtype);
+                  "available: (8,64,f32), (8,64,bf16), (8,32,f32), (8,128,f32), (4,32,f32)", H, C, xw_dtype);
     return GNNFD_ERR_UNSUPPORTED;
 }
 

@@ -61,6 +61,15 @@ struct StreamGeo {
     static constexpr int CTA_BYTES = ST_WARPS * WARP_BYTES;
 };
 
+// CTAs per SM the stream kernels are compiled for (their __launch_bounds__).  Up to 2 KB rows four 4-warp CTAs share
+// an SM; a 4 KB row (8 heads x 128 fp32) makes the ring alone 20 KB per warp, so at most two CTAs fit and each thread
+// may use twice the registers -- which its 32 accumulators per lane need.
+template <class GE>
+constexpr int st_min_ctas()
+{
+    return GE::D * int(sizeof(typename GE::XT)) > 2048 ? 2 : 4;
+}
+
 // per-warp view of the dynamic shared memory
 template <class GE, int EXTRA = 0>
 struct WarpRing {

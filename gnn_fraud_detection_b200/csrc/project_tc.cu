@@ -195,9 +195,10 @@ __global__ void build_b_images(const float* __restrict__ src, int64_t s_row, int
 }
 
 // ---- C[M, NT*BN] = A[M, Kd] * B^T, A fp32 row-major (lda), B as prebuilt images ----------------------
-// EPI 1: forward epilogue -- store xw (fp32 / bf16) and the per-head logits; BN must be a multiple of C=64.
+// EPI 1: forward epilogue -- store xw (fp32 / bf16) and the per-head logits of heads HC columns wide; BN must be a
+//        multiple of HC.
 // EPI 0: plain fp32 store of the first n_valid columns (ldc).
-template <int BN, int EPI, bool OUT_BF16>
+template <int BN, int EPI, bool OUT_BF16, int HC = 64>
 __global__ void __launch_bounds__(THREADS)
 gemm_tc(const float* __restrict__ A, int64_t lda, int64_t M, int Kd, const float* __restrict__ b_img, int n_kb,
         float* __restrict__ Cf, __nv_bfloat16* __restrict__ Cb, int64_t ldc, int n_valid,
@@ -209,6 +210,8 @@ gemm_tc(const float* __restrict__ A, int64_t lda, int64_t M, int Kd, const float
     constexpr uint32_t TMEM_COLS = BN <= 32 ? 32 : BN <= 64 ? 64 : BN <= 128 ? 128 : 256;
     constexpr uint32_t IDESC = make_idesc(BM, BN, 0, 0);
     constexpr int STG_LD = 36;                    // staging row stride (floats): conflict-free float4 both ways
+    static_assert(HC == 32 || HC == 64 || HC == 128, "the logits epilogue covers heads of 32, 64 or 128 columns");
+    static_assert(EPI == 0 || BN % HC == 0, "a column tile holds whole heads");
 
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -305,9 +308,9 @@ gemm_tc(const float* __restrict__ A, int64_t lda, int64_t M, int Kd, const float
                 ps = fmaf(f, att_s[0][ch * 32 + c], ps);
                 pd = fmaf(f, att_s[1][ch * 32 + c], pd);
             }
-            if (ch & 1) {                                   // two 32-column chunks per 64-wide head
+            if ((ch & (HC / 32 - 1)) == HC / 32 - 1) {      // HC/32 32-column chunks per head
                 if (row < M) {
-                    const int h = (nt * BN + ch * 32) / 64;
+                    const int h = (nt * BN + ch * 32) / HC;
                     a_src[row * H + h] = ps;
                     a_dst[row * H + h] = pd;
                 }
@@ -590,7 +593,7 @@ static bool tc_device_ok()
 bool tc_supported(int64_t N, int64_t K, int H, int C)
 {
     (void)N;
-    return tc_device_ok() && C == 64 && (H * C) % 256 == 0 && K >= 1 && K <= 4096;
+    return tc_device_ok() && (C == 32 || C == 64 || C == 128) && (H * C) % 256 == 0 && K >= 1 && K <= 4096;
 }
 
 // images for the forward (W: D rows x K) + for dx (W^T: K rows x D, one tile of <= 256 rows)
@@ -605,67 +608,59 @@ size_t tc_ws_bytes(int64_t N, int64_t K, int H, int C)
     return fwd + bwd + dwp + 4096;
 }
 
-int project_fwd_tc(const float* x, int64_t ldx, const float* W, const float* att_src, const float* att_dst, int64_t N,
-                   int64_t K, int H, int C, int xw_dtype, void* xw, float* a_src, float* a_dst, void* ws, size_t ws_bytes,
-                   cudaStream_t st)
+// the forward GEMM with the logits epilogue for heads of HC columns.  bf16 feature storage (2e-2 relative tolerance)
+// takes one TF32 pass (FAST) instead of the compensated three.
+template <int HC, bool BF16>
+static int launch_fwd_tc(const float* x, int64_t ldx, const float* W, const float* att_src, const float* att_dst, int64_t N,
+                         int64_t K, int H, int D, void* xw, float* a_src, float* a_dst, void* ws, cudaStream_t st)
 {
-    const int D = H * C;
-    GNNFD_REQUIRE(tc_supported(N, K, H, C), GNNFD_ERR_UNSUPPORTED, "project_fwd_tc: unsupported shape");
-    GNNFD_REQUIRE(ws && ws_bytes >= tc_ws_bytes(N, K, H, C), GNNFD_ERR_WORKSPACE, "project_fwd_tc: workspace too small");
-    if (N == 0) return GNNFD_OK;
     constexpr int BN = 256;
     const int n_kb = tc::kblocks(K), n_tiles = D / BN;
     float* img = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(ws) + 1023) & ~uintptr_t(1023));
+    float* xf = BF16 ? nullptr : reinterpret_cast<float*>(xw);
+    __nv_bfloat16* xb = BF16 ? reinterpret_cast<__nv_bfloat16*>(xw) : nullptr;
     tc::build_b_images<<<dim3(8, n_kb, n_tiles), 256, 0, st>>>(W, K, 1, D, (int)K, BN, n_kb, img);
     if (ws_mode() == 2) {
         const int64_t tiles = int64_t(n_tiles) * ((N + 2 * tc::BM - 1) / (2 * tc::BM));
         int64_t clusters = sm_count() / 2;
         if (tiles < clusters) clusters = tiles;
         const unsigned grid = (unsigned)(2 * clusters);
-        if (xw_dtype == GNNFD_BF16) {
-            GNNFD_CUDA(cudaFuncSetAttribute(tc::gemm_tc_ws2<1, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::WS2_SMEM));
-            tc::gemm_tc_ws2<1, true, true><<<grid, tc::WS2_THREADS, tc::WS2_SMEM, st>>>(x, ldx, N, (int)K, img, n_kb, n_tiles, nullptr,
-                                                                                (__nv_bfloat16*)xw, D, D, att_src, att_dst, a_src, a_dst, H);
-        } else {
-            GNNFD_CUDA(cudaFuncSetAttribute(tc::gemm_tc_ws2<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::WS2_SMEM));
-            tc::gemm_tc_ws2<1, false><<<grid, tc::WS2_THREADS, tc::WS2_SMEM, st>>>(x, ldx, N, (int)K, img, n_kb, n_tiles, (float*)xw,
-                                                                                 nullptr, D, D, att_src, att_dst, a_src, a_dst, H);
-        }
-        g_launches += 2;
-        GNNFD_LAUNCH_CHECK();
-        return GNNFD_OK;
-    }
-    if (use_ws()) {
+        GNNFD_CUDA(cudaFuncSetAttribute(tc::gemm_tc_ws2<1, BF16, BF16, HC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        (int)tc::WS2_SMEM));
+        tc::gemm_tc_ws2<1, BF16, BF16, HC><<<grid, tc::WS2_THREADS, tc::WS2_SMEM, st>>>(
+            x, ldx, N, (int)K, img, n_kb, n_tiles, xf, xb, D, D, att_src, att_dst, a_src, a_dst, H);
+    } else if (use_ws()) {
         const int64_t tiles = int64_t(n_tiles) * ((N + tc::BM - 1) / tc::BM);
         const unsigned grid = (unsigned)(tiles < sm_count() ? tiles : sm_count());
-        if (xw_dtype == GNNFD_BF16) {
-            // bf16 feature storage (2e-2 relative tolerance): one TF32 pass instead of the compensated three
-            GNNFD_CUDA(cudaFuncSetAttribute(tc::gemm_tc_ws<1, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::WS_SMEM));
-            tc::gemm_tc_ws<1, true, true><<<grid, tc::WS_THREADS, tc::WS_SMEM, st>>>(x, ldx, N, (int)K, img, n_kb, n_tiles, nullptr,
-                                                                             (__nv_bfloat16*)xw, D, D, att_src, att_dst, a_src, a_dst, H);
-        } else {
-            GNNFD_CUDA(cudaFuncSetAttribute(tc::gemm_tc_ws<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::WS_SMEM));
-            tc::gemm_tc_ws<1, false><<<grid, tc::WS_THREADS, tc::WS_SMEM, st>>>(x, ldx, N, (int)K, img, n_kb, n_tiles, (float*)xw,
-                                                                              nullptr, D, D, att_src, att_dst, a_src, a_dst, H);
-        }
-        g_launches += 2;
-        GNNFD_LAUNCH_CHECK();
-        return GNNFD_OK;
-    }
-    const size_t smem = tc::gemm_smem_bytes<BN>();
-    dim3 grid((unsigned)(int64_t(n_tiles) * ((N + tc::BM - 1) / tc::BM)));
-    if (xw_dtype == GNNFD_BF16) {
-        GNNFD_CUDA(cudaFuncSetAttribute(tc::gemm_tc<BN, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        tc::gemm_tc<BN, 1, true><<<grid, tc::THREADS, smem, st>>>(x, ldx, N, (int)K, img, n_kb, nullptr, (__nv_bfloat16*)xw, D,
-                                                                 D, att_src, att_dst, a_src, a_dst, H);
+        GNNFD_CUDA(cudaFuncSetAttribute(tc::gemm_tc_ws<1, BF16, BF16, HC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        (int)tc::WS_SMEM));
+        tc::gemm_tc_ws<1, BF16, BF16, HC><<<grid, tc::WS_THREADS, tc::WS_SMEM, st>>>(
+            x, ldx, N, (int)K, img, n_kb, n_tiles, xf, xb, D, D, att_src, att_dst, a_src, a_dst, H);
     } else {
-        GNNFD_CUDA(cudaFuncSetAttribute(tc::gemm_tc<BN, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        tc::gemm_tc<BN, 1, false><<<grid, tc::THREADS, smem, st>>>(x, ldx, N, (int)K, img, n_kb, (float*)xw, nullptr, D, D,
-                                                                  att_src, att_dst, a_src, a_dst, H);
+        const size_t smem = tc::gemm_smem_bytes<BN>();
+        dim3 grid((unsigned)(int64_t(n_tiles) * ((N + tc::BM - 1) / tc::BM)));
+        GNNFD_CUDA(cudaFuncSetAttribute(tc::gemm_tc<BN, 1, BF16, HC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        tc::gemm_tc<BN, 1, BF16, HC><<<grid, tc::THREADS, smem, st>>>(x, ldx, N, (int)K, img, n_kb, xf, xb, D, D, att_src,
+                                                                      att_dst, a_src, a_dst, H);
     }
     g_launches += 2;
     GNNFD_LAUNCH_CHECK();
     return GNNFD_OK;
+}
+
+int project_fwd_tc(const float* x, int64_t ldx, const float* W, const float* att_src, const float* att_dst, int64_t N,
+                   int64_t K, int H, int C, int xw_dtype, void* xw, float* a_src, float* a_dst, void* ws, size_t ws_bytes,
+                   cudaStream_t st)
+{
+    GNNFD_REQUIRE(tc_supported(N, K, H, C), GNNFD_ERR_UNSUPPORTED, "project_fwd_tc: unsupported shape");
+    GNNFD_REQUIRE(xw_dtype == GNNFD_F32 || C == 64, GNNFD_ERR_UNSUPPORTED, "project_fwd: bf16 xw needs C == 64");
+    GNNFD_REQUIRE(ws && ws_bytes >= tc_ws_bytes(N, K, H, C), GNNFD_ERR_WORKSPACE, "project_fwd_tc: workspace too small");
+    if (N == 0) return GNNFD_OK;
+    const int D = H * C;
+    if (xw_dtype == GNNFD_BF16) return launch_fwd_tc<64, true>(x, ldx, W, att_src, att_dst, N, K, H, D, xw, a_src, a_dst, ws, st);
+    if (C == 32) return launch_fwd_tc<32, false>(x, ldx, W, att_src, att_dst, N, K, H, D, xw, a_src, a_dst, ws, st);
+    if (C == 128) return launch_fwd_tc<128, false>(x, ldx, W, att_src, att_dst, N, K, H, D, xw, a_src, a_dst, ws, st);
+    return launch_fwd_tc<64, false>(x, ldx, W, att_src, att_dst, N, K, H, D, xw, a_src, a_dst, ws, st);
 }
 
 // dx[N,K] = dxw[N,D] @ W[D,K]:  A = dxw (K-major in D), B rows = k (W^T), reduction over D

@@ -95,13 +95,14 @@ __device__ __forceinline__ void umma2_commit_both(uint64_t* bar)
                  : "memory");
 }
 
-template <int EPI, bool OUT_BF16, bool FAST = false>
+template <int EPI, bool OUT_BF16, bool FAST = false, int HC = 64>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WS2_THREADS, 1)
 gemm_tc_ws2(const float* __restrict__ A, int64_t lda, int64_t M, int Kd, const float* __restrict__ b_img, int n_kb,
             int n_col_tiles, float* __restrict__ Cf, __nv_bfloat16* __restrict__ Cb, int64_t ldc, int n_valid,
             const float* __restrict__ att_src, const float* __restrict__ att_dst, float* __restrict__ a_src,
             float* __restrict__ a_dst, int H)
 {
+    static_assert(HC == 32 || HC == 64 || HC == 128, "the logits epilogue covers heads of 32, 64 or 128 columns");
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     __shared__ uint64_t full_a[WS2_STAGES], full_b[WS2_STAGES], empty[WS2_STAGES], acc_full[2], acc_empty[2];
@@ -304,9 +305,9 @@ gemm_tc_ws2(const float* __restrict__ A, int64_t lda, int64_t M, int Kd, const f
                         ps = fmaf(__uint_as_float(v[c + 2]), as4.z, ps); pd = fmaf(__uint_as_float(v[c + 2]), ad4.z, pd);
                         ps = fmaf(__uint_as_float(v[c + 3]), as4.w, ps); pd = fmaf(__uint_as_float(v[c + 3]), ad4.w, pd);
                     }
-                    if (ch & 1) {
+                    if ((ch & (HC / 32 - 1)) == HC / 32 - 1) {      // HC/32 32-column chunks per head
                         if (row < M) {
-                            const int h = col0 / 64;
+                            const int h = col0 / HC;
                             a_src[row * H + h] = ps;
                             a_dst[row * H + h] = pd;
                         }

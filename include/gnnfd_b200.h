@@ -189,7 +189,9 @@ int gnnfd_project_fwd_image(const void* ximg, const float* row_scale, int64_t N,
  * either keep_mask is an explicit [E',H] uint8 keep mask in edge_index' (PyG) order, applied as alpha*keep/(1-p) (parity
  * tests inject one), or keep_mask is NULL and the kernels draw the bits from a counter-based RNG keyed on (dropout_seed,
  * position in edge_index', head) -- no [E',H] tensor exists; forward and backward must be given the same seed.
- * gnnfd_dropout_mask writes those bits out (test hook) and returns the survivor scale. */
+ * gnnfd_dropout_mask writes those bits out (test hook) and returns the survivor scale.
+ * Built geometries (heads, out_channels, xw dtype): (8,32,f32), (8,64,f32), (8,64,bf16), (8,128,f32), (4,32,f32); any other
+ * returns GNNFD_ERR_UNSUPPORTED ("... is not built; available: ...").  The same set holds for (4). */
 int gnnfd_dropout_mask(uint64_t dropout_seed, float p_drop, int64_t n_edges, int H, uint8_t* keep_mask,
                        float* scale_host, gnnfd_stream_t stream);
 /* Process-wide: when device_word is not NULL every kernel that draws dropout bits adds *device_word to its seed.  A training
@@ -230,7 +232,7 @@ int gnnfd_gat_alpha(const gnnfd_graph_t* g, const float* a_src, const float* a_d
  * src-major pass (needs the CSC twin): dxw[j] = sum_e alpha_used*dO_h[i] + da_src[j]*att_src
  *   + da_dst_full[j]*att_dst, da_src[j] = sum_e dz.  da_dst_full is indexed by SOURCE id (for a single
  *   GPU it is the da_dst the dst pass produced; NULL => the att_dst term is skipped).
- * d_out [n_dst, concat ? H*C : C]. */
+ * d_out [n_dst, concat ? H*C : C].  Geometries as in (3); gnnfd_gat_bwd_src takes fp32 only. */
 int gnnfd_gat_bwd_workspace_bytes(const gnnfd_graph_t* g, int H, int C, size_t* bytes);
 int gnnfd_gat_bwd_dst(const gnnfd_graph_t* g, const void* xw, int xw_dtype, const float* a_src,
                       const float* a_dst, const float* rowmax, const float* rowsum, const float* d_out,
