@@ -18,7 +18,7 @@ F32, BF16 = 0, 1
 ACT_NONE, ACT_RELU, ACT_ELU = 0, 1, 2
 GEMM_AUTO, GEMM_SIMT, GEMM_TC, GEMM_INPUT = 0, 1, 2, 3
 HUB_THRESHOLD, HUB_CHUNK = 512, 512
-ABI_VERSION = 19
+ABI_VERSION = 20
 
 _i32p = C.POINTER(C.c_int32)
 
@@ -98,6 +98,7 @@ SIGNATURES = {
     "gnnfd_in_fwd_workspace_bytes": (_i, [_gp, _szp]),
     "gnnfd_in_fwd": (_i, [_gp, _vp, _i64, _i64, _vp, _vp, _f, _vp, _f, _u64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "gnnfd_in_out": (_i, [_vp, _i64, _i64, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp]),
+    "gnnfd_in_out_bcast": (_i, [_vp, _i64, _i64, _vp, _vp, _i, _vp, _vp, _vp, C.POINTER(Peers), _i64, _i, _vp, _vp]),
     "gnnfd_in_bwd_gd_workspace_bytes": (_i, [_i64, _szp]),
     "gnnfd_in_bwd_gd": (_i, [_vp, _i64, _i64, _vp, _vp, _vp, _sz, _vp]),
     "gnnfd_in_bwd_edges_workspace_bytes": (_i, [_gp, _szp]),

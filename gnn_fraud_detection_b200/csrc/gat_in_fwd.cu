@@ -50,23 +50,11 @@ __global__ void in_u_kernel(const float* __restrict__ W, const float* __restrict
 // shared memory (ONE bulk copy per tile, double-buffered); lane = (head h, quarter q) as in the edge kernels: 44 + 44
 // u values in registers, per row 11 shared loads, 88 FMAs and two 2-step quad reductions.  Also max |x|.
 constexpr int LG_ROWS = 64, LG_WARPS = 8;
-// where the a_src rows go: mode 0 = a_src (local); 1 = row (row_off + r) of the same buffer on every peer (one 16-byte
-// store per peer over NVLink); 2 = one multimem.st to the multicast mapping (the NVSwitch replicates it to every rank)
-struct LogitPeers {
-    int mode, n;
-    int64_t row_off;
-    float* ptr[GNNFD_MAX_PEERS];
-    float* mc;
-};
-__device__ __forceinline__ void multimem_st_v4(float* p, float4 v)
-{
-    asm volatile("multimem.st.relaxed.sys.global.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w)
-                 : "memory");
-}
+// the a_src rows go to a_src (peers.mode 0) or into the same rows of a buffer on every rank (PeerRows, in_common.cuh)
 template <int N4>
 __global__ void __launch_bounds__(LG_WARPS * 32, 2)
 in_logits_kernel(const float* __restrict__ x, int64_t ldx, int64_t N, int KP, const float* __restrict__ u,
-                 float* __restrict__ a_src, float* __restrict__ a_dst, unsigned* __restrict__ xmax_bits, LogitPeers peers)
+                 float* __restrict__ a_src, float* __restrict__ a_dst, unsigned* __restrict__ xmax_bits, PeerRows peers)
 {
     using RG = RowGeo<N4>;
     extern __shared__ __align__(128) uint8_t lsm[];
@@ -643,7 +631,7 @@ int gnnfd_in_pad_x(const float* x, int64_t ldx, int64_t N, int64_t K, float* x16
 /* a_src / a_dst [N,H] for rows [0,N) of x, and xmax[0] = max(xmax[0], max |x|) (caller zeroes xmax before the first call;
  * across GPUs the per-rank maxima are max-reduced before gnnfd_in_prepare).  x: padded rows (gnnfd_in_pad_x layout). */
 static int in_logits_launch(const float* x, int64_t ldx, int64_t N, int64_t K, const float* W, const float* att_src,
-                            const float* att_dst, float* a_src, float* a_dst, float* xmax, void* prep, const LogitPeers& peers,
+                            const float* att_dst, float* a_src, float* a_dst, float* xmax, void* prep, const PeerRows& peers,
                             cudaStream_t st)
 {
     const Dims d((int)K);
@@ -684,7 +672,7 @@ int gnnfd_in_logits(const float* x, int64_t ldx, int64_t N, int64_t K, const flo
     GNNFD_REQUIRE(K >= 1 && K <= MAX_K && N >= 0, GNNFD_ERR_ARG, "in_logits: bad shape (K <= %d)", MAX_K);
     GNNFD_REQUIRE(W && att_src && att_dst && xmax && prep, GNNFD_ERR_ARG, "in_logits: NULL argument");
     GNNFD_REQUIRE(N == 0 || (x && a_src && a_dst), GNNFD_ERR_ARG, "in_logits: NULL tensor");
-    LogitPeers peers{};
+    PeerRows peers{};
     return in_logits_launch(x, ldx, N, K, W, att_src, att_dst, a_src, a_dst, xmax, prep, peers, (cudaStream_t)stream);
 }
 
@@ -695,19 +683,9 @@ int gnnfd_in_logits_bcast(const float* x, int64_t ldx, int64_t N, int64_t K, con
     GNNFD_REQUIRE(K >= 1 && K <= MAX_K && N >= 0 && row_offset >= 0, GNNFD_ERR_ARG, "in_logits_bcast: bad shape (K <= %d)", MAX_K);
     GNNFD_REQUIRE(W && att_src && att_dst && xmax && prep && a_src_all, GNNFD_ERR_ARG, "in_logits_bcast: NULL argument");
     GNNFD_REQUIRE(N == 0 || (x && a_dst), GNNFD_ERR_ARG, "in_logits_bcast: NULL tensor");
-    GNNFD_REQUIRE(a_src_all->n_peers >= 1 && a_src_all->n_peers <= GNNFD_MAX_PEERS, GNNFD_ERR_ARG, "in_logits_bcast: 1..%d peers",
-                  GNNFD_MAX_PEERS);
-    GNNFD_REQUIRE(!use_multicast || a_src_all->multicast, GNNFD_ERR_ARG, "in_logits_bcast: no multicast mapping given");
-    LogitPeers peers{};
-    peers.mode = use_multicast ? 2 : 1;
-    peers.n = a_src_all->n_peers;
-    peers.row_off = row_offset;
-    peers.mc = reinterpret_cast<float*>(a_src_all->multicast);
-    for (int g = 0; g < peers.n; ++g) {
-        GNNFD_REQUIRE(a_src_all->ptr[g] && (reinterpret_cast<uintptr_t>(a_src_all->ptr[g]) & 15) == 0, GNNFD_ERR_ARG,
-                      "in_logits_bcast: peer buffer %d NULL or not 16-byte aligned", g);
-        peers.ptr[g] = reinterpret_cast<float*>(a_src_all->ptr[g]);
-    }
+    PeerRows peers;
+    const int rc = peer_rows_from(a_src_all, row_offset, use_multicast, "in_logits_bcast", peers);
+    if (rc) return rc;
     return in_logits_launch(x, ldx, N, K, W, att_src, att_dst, nullptr, a_dst, xmax, prep, peers, (cudaStream_t)stream);
 }
 

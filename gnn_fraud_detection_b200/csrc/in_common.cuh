@@ -90,6 +90,39 @@ __host__ __device__ inline size_t prep_bytes(const Dims& d) { return prep_off_u(
 
 inline size_t zimg_bytes(int64_t n_rows, const Dims& d) { return size_t((n_rows + TILE - 1) / TILE) * d.NKB * KBLOCK; }
 
+// Where a kernel's finished rows also go (header section 7): mode 0 = nowhere else; 1 = row (row_off + r) of the same buffer
+// on every peer (one 16-byte store per peer over NVLink); 2 = one multimem.st to the multicast mapping (the NVSwitch
+// replicates it to every rank)
+struct PeerRows {
+    int mode, n;
+    int64_t row_off;
+    float* ptr[GNNFD_MAX_PEERS];
+    float* mc;
+};
+__device__ __forceinline__ void multimem_st_v4(float* p, float4 v)
+{
+    asm volatile("multimem.st.relaxed.sys.global.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w)
+                 : "memory");
+}
+// checks the caller's peer table before anything is launched and fills `pr` (mode 1 or 2)
+inline int peer_rows_from(const gnnfd_peers_t* p, int64_t row_offset, int use_multicast, const char* who, PeerRows& pr)
+{
+    GNNFD_REQUIRE(p && row_offset >= 0, GNNFD_ERR_ARG, "%s: NULL peer table or negative row offset", who);
+    GNNFD_REQUIRE(p->n_peers >= 1 && p->n_peers <= GNNFD_MAX_PEERS, GNNFD_ERR_ARG, "%s: 1..%d peers", who, GNNFD_MAX_PEERS);
+    GNNFD_REQUIRE(!use_multicast || p->multicast, GNNFD_ERR_ARG, "%s: no multicast mapping given", who);
+    pr = PeerRows{};
+    pr.mode = use_multicast ? 2 : 1;
+    pr.n = p->n_peers;
+    pr.row_off = row_offset;
+    pr.mc = reinterpret_cast<float*>(p->multicast);
+    for (int g = 0; g < pr.n; ++g) {
+        GNNFD_REQUIRE(p->ptr[g] && (reinterpret_cast<uintptr_t>(p->ptr[g]) & 15) == 0, GNNFD_ERR_ARG,
+                      "%s: peer buffer %d NULL or not 16-byte aligned", who, g);
+        pr.ptr[g] = reinterpret_cast<float*>(p->ptr[g]);
+    }
+    return GNNFD_OK;
+}
+
 }  // namespace in
 }  // namespace gnnfd
 

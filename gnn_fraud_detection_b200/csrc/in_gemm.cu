@@ -127,9 +127,12 @@ __device__ __forceinline__ float out_act(float v, int act)
     return v;
 }
 
+// PM: where the finished rows go besides `out` (PeerRows::mode; 0: `out` only, 1 / 2: also row (row_off + r) on every rank,
+// `out` optional)
+template <int PM>
 __global__ void __launch_bounds__(G1_THREADS, 1)
 in_out_gemm(const uint8_t* __restrict__ zimg, const uint8_t* __restrict__ wimg, const float* __restrict__ scal, int64_t n,
-            int NKB, OutEpi ep, float* __restrict__ out)
+            int NKB, OutEpi ep, float* __restrict__ out, PeerRows peers)
 {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -249,7 +252,13 @@ in_out_gemm(const uint8_t* __restrict__ zimg, const uint8_t* __restrict__ wimg, 
                             if (ep.residual) v += ep.residual[gm * C + cq + k];
                             ov[k] = v;
                         }
-                        *reinterpret_cast<float4*>(out + gm * C + cq) = make_float4(ov[0], ov[1], ov[2], ov[3]);
+                        const float4 o4 = make_float4(ov[0], ov[1], ov[2], ov[3]);
+                        if (PM == 0 || out) *reinterpret_cast<float4*>(out + gm * C + cq) = o4;
+                        const int64_t po = (peers.row_off + gm) * C + cq;
+                        if (PM == 1)
+                            for (int g = 0; g < peers.n; ++g) *reinterpret_cast<float4*>(peers.ptr[g] + po) = o4;
+                        else if (PM == 2)
+                            multimem_st_v4(peers.mc + po, o4);
                     }
                 }
             }
@@ -780,6 +789,23 @@ static size_t dw_partial_floats(const Dims& d) { return size_t((d.NKB + 1) / 2) 
 using namespace gnnfd;
 using namespace gnnfd::in;
 
+template <int PM>
+static int in_out_launch(const void* zimg, int64_t n, int64_t K, const void* prep, const OutEpi& ep, float* out,
+                         const PeerRows& peers, cudaStream_t st)
+{
+    const Dims d((int)K);
+    const char* p = reinterpret_cast<const char*>(prep);
+    const int64_t n_tiles = (n + TILE - 1) / TILE;
+    const unsigned grid = (unsigned)(n_tiles < sm_count() ? n_tiles : sm_count());
+    GNNFD_CUDA(cudaFuncSetAttribute(in_out_gemm<PM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G1_SMEM));
+    in_out_gemm<PM><<<grid, G1_THREADS, G1_SMEM, st>>>(reinterpret_cast<const uint8_t*>(zimg),
+                                                       reinterpret_cast<const uint8_t*>(p + prep_off_wout(d)),
+                                                       reinterpret_cast<const float*>(p), n, d.NKB, ep, out, peers);
+    g_launches += 1;
+    GNNFD_LAUNCH_CHECK();
+    return GNNFD_OK;
+}
+
 extern "C" {
 
 /* out [n, C] = act((Z W_r / H + bias) * post_scale + post_shift) + residual   (cf. gnnfd_gat_fwd_fused) */
@@ -794,19 +820,32 @@ int gnnfd_in_out(const void* zimg, int64_t n, int64_t K, const void* prep, const
                   "in_out: post_scale and post_shift must be given together");
     GNNFD_REQUIRE((reinterpret_cast<uintptr_t>(zimg) & 1023) == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0, GNNFD_ERR_ARG,
                   "in_out: zimg must be 1024-byte and out 16-byte aligned");
-    cudaStream_t st = (cudaStream_t)stream;
-    const Dims d((int)K);
-    const char* p = reinterpret_cast<const char*>(prep);
-    const int64_t n_tiles = (n + TILE - 1) / TILE;
-    const unsigned grid = (unsigned)(n_tiles < sm_count() ? n_tiles : sm_count());
-    GNNFD_CUDA(cudaFuncSetAttribute(in_out_gemm, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G1_SMEM));
     const OutEpi ep{bias, post_scale, post_shift, residual, act};
-    in_out_gemm<<<grid, G1_THREADS, G1_SMEM, st>>>(reinterpret_cast<const uint8_t*>(zimg),
-                                                   reinterpret_cast<const uint8_t*>(p + prep_off_wout(d)),
-                                                   reinterpret_cast<const float*>(p), n, d.NKB, ep, out);
-    g_launches += 1;
-    GNNFD_LAUNCH_CHECK();
-    return GNNFD_OK;
+    return in_out_launch<0>(zimg, n, K, prep, ep, out, PeerRows{}, (cudaStream_t)stream);
+}
+
+/* gnnfd_in_out fused with the all-gather of the output rows: every finished 16-byte piece of row r also goes to row
+ * (row_offset + r) of h_all [n_pos, C] on every rank (one multimem.st, or one store per peer).  out (own rows) may be NULL. */
+int gnnfd_in_out_bcast(const void* zimg, int64_t n, int64_t K, const void* prep, const float* bias, int act,
+                       const float* post_scale, const float* post_shift, const float* residual,
+                       const gnnfd_peers_t* h_all, int64_t row_offset, int use_multicast, float* out,
+                       gnnfd_stream_t stream)
+{
+    GNNFD_REQUIRE(K >= 1 && K <= MAX_K && n >= 0, GNNFD_ERR_ARG, "in_out_bcast: bad shape");
+    PeerRows peers;
+    const int rc = peer_rows_from(h_all, row_offset, use_multicast, "in_out_bcast", peers);
+    if (rc) return rc;
+    if (n == 0) return GNNFD_OK;
+    GNNFD_REQUIRE(zimg && prep, GNNFD_ERR_ARG, "in_out_bcast: NULL tensor");
+    GNNFD_REQUIRE((post_scale == nullptr) == (post_shift == nullptr), GNNFD_ERR_ARG,
+                  "in_out_bcast: post_scale and post_shift must be given together");
+    GNNFD_REQUIRE((reinterpret_cast<uintptr_t>(zimg) & 1023) == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0, GNNFD_ERR_ARG,
+                  "in_out_bcast: zimg must be 1024-byte and out 16-byte aligned");
+    GNNFD_REQUIRE(!use_multicast || (reinterpret_cast<uintptr_t>(h_all->multicast) & 15) == 0, GNNFD_ERR_ARG,
+                  "in_out_bcast: the multicast address must be 16-byte aligned");
+    const OutEpi ep{bias, post_scale, post_shift, residual, act};
+    cudaStream_t st = (cudaStream_t)stream;
+    return use_multicast ? in_out_launch<2>(zimg, n, K, prep, ep, out, peers, st) : in_out_launch<1>(zimg, n, K, prep, ep, out, peers, st);
 }
 
 /* gd [n, F] = d_out [n, C] @ W_r^T / H  (F = gnnfd_in_sizes' gd_ld): the per-destination vectors whose dot product with

@@ -339,11 +339,23 @@ def in_fwd(g: GraphCSR, x, a_src, a_dst, negative_slope, prep, keep_mask=None, p
     return zimg, InAttention(alpha, jflag, rowmax, rowsum)
 
 
-def in_out(zimg, n, K, prep, bias, act=_abi.ACT_NONE, post_scale=None, post_shift=None, residual=None):
-    out = torch.empty(n, 64, dtype=torch.float32, device=zimg.device)
+def in_out(zimg, n, K, prep, bias, act=_abi.ACT_NONE, post_scale=None, post_shift=None, residual=None, out=None):
+    if out is None:
+        out = torch.empty(n, 64, dtype=torch.float32, device=zimg.device)
     _abi.check(_abi.lib().gnnfd_in_out(zimg.data_ptr(), int(n), int(K), prep.data_ptr(), _abi.ptr(bias), int(act),
                                        _abi.ptr(post_scale), _abi.ptr(post_shift), _abi.ptr(residual), out.data_ptr(),
                                        _stream()))
+    return out
+
+
+def in_out_bcast(zimg, n, K, prep, bias, peers, row_offset, use_multicast=False, act=_abi.ACT_NONE, post_scale=None,
+                 post_shift=None, residual=None, out=None):
+    """``in_out`` fused with the all-gather of its rows: row ``r`` also goes to row ``row_offset + r`` of the symmetric
+    ``[n_pos, 64]`` buffer described by ``peers`` (``_abi.Peers``) on EVERY rank.  ``out`` (the own rows) is optional;
+    returns it."""
+    _abi.check(_abi.lib().gnnfd_in_out_bcast(zimg.data_ptr(), int(n), int(K), prep.data_ptr(), _abi.ptr(bias), int(act),
+                                             _abi.ptr(post_scale), _abi.ptr(post_shift), _abi.ptr(residual), C.byref(peers),
+                                             int(row_offset), int(use_multicast), _abi.ptr(out), _stream()))
     return out
 
 

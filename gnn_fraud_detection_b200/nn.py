@@ -26,6 +26,16 @@ def glorot_(t: torch.Tensor) -> torch.Tensor:
         return t.uniform_(-a, a)
 
 
+def fold_batch_norm(batch_norm: Optional[nn.BatchNorm1d]):
+    """Eval-mode BatchNorm as the per-channel affine ``(scale, shift)`` the fused epilogues take; ``(None, None)`` for none."""
+    if batch_norm is None:
+        return None, None
+    inv = torch.rsqrt(batch_norm.running_var + batch_norm.eps)
+    w = batch_norm.weight if batch_norm.weight is not None else torch.ones_like(inv)
+    b = batch_norm.bias if batch_norm.bias is not None else torch.zeros_like(inv)
+    return (w * inv).contiguous(), (b - batch_norm.running_mean * w * inv).contiguous()
+
+
 class _Linear(nn.Module):
     """Bias-free projection holder; key ``weight`` has shape ``[heads*out_channels, in_channels]``."""
 
@@ -168,13 +178,7 @@ class GATConv(nn.Module):
         g = self._graph(edge_index, x.size(0))
         self._check_inputs(x, g, residual)
         H, C = self.heads, self.out_channels
-        scale = shift = None
-        if batch_norm is not None:
-            inv = torch.rsqrt(batch_norm.running_var + batch_norm.eps)
-            w = batch_norm.weight if batch_norm.weight is not None else torch.ones_like(inv)
-            b = batch_norm.bias if batch_norm.bias is not None else torch.zeros_like(inv)
-            scale = (w * inv).contiguous()
-            shift = (b - batch_norm.running_mean * w * inv).contiguous()
+        scale, shift = fold_batch_norm(batch_norm)
         act = _abi.ACT_RELU if relu else _abi.ACT_NONE
         res = None if residual is None else residual.contiguous()
         W = self.lin_src.weight.contiguous()

@@ -617,3 +617,155 @@ class InputSpacePartition(DstRangePartition):
                 "includes": "per rank: H2D of own x rows + own edge list, all-gather of x over NVLink (both under the CSR/CSC "
                             "rebuild), fwd+bwd with the [N,H] logit exchange (" + str(getattr(self, "exchange", "nccl")) + "), "
                             "all-reduce of grads, D2H of grads"}
+
+
+def symmetric_buffer(shape, device):
+    """A zero-filled fp32 symmetric (peer-accessible) allocation: ``(this rank's tensor, _abi.Peers with its address on every
+    rank, the rendezvous handle)``.  The handle owns the mapping: keep it as long as the peers are used."""
+    import torch.distributed._symmetric_memory as symm
+    from . import _abi
+    t = symm.empty(shape, dtype=torch.float32, device=device)
+    h = symm.rendezvous(t, dist.group.WORLD)
+    p = _abi.Peers()
+    p.n_peers, p.rank = dist.get_world_size(), dist.get_rank()
+    for r, ptr in enumerate(h.buffer_ptrs):
+        p.ptr[r] = int(ptr)
+    p.multicast = int(getattr(h, "multicast_ptr", 0) or 0) or None
+    t.zero_()
+    return t, p, h
+
+
+class InputSpaceModelPartition(DstRangePartition):
+    """Inference of a whole ``GAT`` / ``TemporalGNN`` (eval mode) on a destination-range partition, every layer in the
+    input-space formulation (csrc/in_common.cuh) -- the cross-GPU form of ``model.eval()`` with ``gemm_algo=GEMM_INPUT`` on
+    every layer.
+
+    The model input ``x`` is replicated in padded position space; the hidden state ``h [n_pos, 64]`` lives in two buffers
+    that every rank holds whole.  Per layer each rank
+      1. computes the logits of its own rows and stores ``a_src`` into every rank's buffer (``in_logits_bcast``), then a
+         barrier and the max-reduce of ``max|input|`` (the fp16-pair scale);
+      2. aggregates the layer input over its destination rows (``in_fwd``, local);
+      3. runs the output GEMM with BatchNorm (running statistics), ReLU and the residual in its epilogue and stores each
+         finished row into the next hidden buffer on every rank (``in_out_bcast``), then a barrier.
+    Per layer and rank ~``N * (64 + 8) * 4`` bytes cross NVLink (each rank sends its rows to every other rank) and nothing is
+    projected twice.  The head runs on the own rows.  ``GNNFD_EXCHANGE=nccl``, or no symmetric memory, uses ``in_logits`` /
+    ``in_out`` and NCCL all-gathers instead, with bit-identical results.
+    """
+
+    H, HIDDEN = 8, 64
+
+    @staticmethod
+    def check_model(model):
+        """Refuse what this path does not compute, before anything is launched."""
+        from . import functional as Fn
+        from .models import GAT, TemporalGNN
+        if not isinstance(model, (GAT, TemporalGNN)):
+            raise TypeError(f"InputSpaceModelPartition runs GAT or TemporalGNN, not {type(model).__name__}")
+        if model.training:
+            raise RuntimeError("InputSpaceModelPartition is inference only: call model.eval() first "
+                               "(training across GPUs is not supported)")
+        if model.hidden_channels != InputSpaceModelPartition.HIDDEN:
+            raise NotImplementedError(f"InputSpaceModelPartition is built for hidden_channels=64, got {model.hidden_channels}")
+        for i, conv in enumerate(model.gat_layers):
+            if conv.heads != InputSpaceModelPartition.H:
+                raise NotImplementedError(f"InputSpaceModelPartition is built for 8 heads, layer {i} has {conv.heads}")
+            if not conv.add_self_loops:
+                raise NotImplementedError("InputSpaceModelPartition adds self-loops (local_edges): layer "
+                                          f"{i} has add_self_loops=False")
+            if not Fn.in_supported(conv.in_channels, conv.heads, conv.out_channels, conv.concat):
+                raise NotImplementedError(f"layer {i}: the input-space formulation needs in_channels <= 192, concat=False "
+                                          f"(got in_channels={conv.in_channels}, concat={conv.concat})")
+
+    def _setup_exchange(self):
+        import os
+        mode = os.environ.get("GNNFD_EXCHANGE", "auto")
+        shape = (self.n_pos, self.HIDDEN)
+        self.px = None
+        if self.world > 1 and mode != "nccl":
+            try:
+                px = PeerExchange(self.n_pos, self.device, mode, self.H)
+                bufs = [symmetric_buffer(shape, self.device) for _ in range(2)]
+                self.px = px
+            except Exception as ex:               # no symmetric memory on this box: NCCL collectives
+                if mode != "auto":
+                    raise
+                self.px_error = f"{type(ex).__name__}: {ex}"
+        if self.px is not None:
+            self.hidden = [b[0] for b in bufs]
+            self.hidden_peers = [b[1] for b in bufs]
+            self._handles = [b[2] for b in bufs]
+        else:
+            self.hidden = [torch.zeros(shape, dtype=torch.float32, device=self.device) for _ in range(2)]
+        self.exchange = self.px.mode if self.px is not None else ("nccl" if self.world > 1 else "none")
+
+    @torch.no_grad()
+    def forward(self, model, x_full, marks=None):
+        """``x_full``: the model input replicated in padded position space, ``[world*rows_padded, in_channels]`` with 16-byte
+        aligned zero-padded rows (``functional.in_pad_x`` layout).  ``marks``: optional per-layer lists of 4 CUDA events
+        (start, logits + exchange done, aggregation done, output GEMM + broadcast done).
+
+        Returns ``(logits, (lo, hi))`` for a GAT and ``((logits, hidden), (lo, hi))`` for a TemporalGNN (zero initial state):
+        the rows of the global nodes ``lo .. hi-1`` this rank owns."""
+        from . import _abi, fused
+        from . import functional as Fn
+        from .models import TemporalGNN
+        from .nn import fold_batch_norm
+        self.check_model(model)
+        if (not x_full.is_cuda or x_full.dtype != torch.float32 or x_full.dim() != 2
+                or tuple(x_full.shape) != (self.n_pos, model.in_channels)):
+            raise ValueError(f"x_full must be float32 CUDA [{self.n_pos},{model.in_channels}] in padded position space, "
+                             f"got {x_full.dtype} {tuple(x_full.shape)} on {x_full.device}")
+        if getattr(self, "hidden", None) is None:
+            self._setup_exchange()
+        P, n, dev, px = self.rows_padded, self.n_local, self.device, self.px
+        lo = self.rank * P
+        h_in = x_full
+        for i, conv in enumerate(model.gat_layers):
+            m = marks[i] if marks else None
+            if m: m[0].record()
+            K = h_in.size(1)
+            x_own = h_in[lo:lo + n]
+            W = conv.lin_src.weight.contiguous()
+            a_s, a_d = conv.att_src.reshape(-1).contiguous(), conv.att_dst.reshape(-1).contiguous()
+            prep = Fn._aligned_u8(Fn.in_sizes(n, K)[0], dev)
+            xmax = torch.zeros(16, dtype=torch.float32, device=dev)
+            if px is not None:
+                px.xmax.zero_()
+                a_dst = Fn.in_logits_bcast(x_own, W, a_s, a_d, prep, px.xmax, px.a_src_peers, lo, px.mode == "multicast")
+                px.barrier()
+                a_src_full = px.a_src
+                Fn.peer_reduce(px.xmax_peers, 0, 4, xmax, op="max")
+            else:
+                a_src_own, a_dst = Fn.in_logits(x_own, W, a_s, a_d, prep, xmax)
+                if self.world > 1:
+                    a_pad = torch.zeros(P, self.H, dtype=torch.float32, device=dev)
+                    a_pad[:n] = a_src_own
+                    a_src_full = torch.empty(self.n_pos, self.H, dtype=torch.float32, device=dev)
+                    dist.all_gather_into_tensor(a_src_full, a_pad)
+                    dist.all_reduce(xmax, op=dist.ReduceOp.MAX)
+                else:
+                    a_src_full = a_src_own
+            Fn.in_prepare(W, K, xmax, prep)
+            if m: m[1].record()
+            zimg, att = Fn.in_fwd(self.graph, h_in, a_src_full, a_dst, conv.negative_slope, prep)
+            if m: m[2].record()
+            bn = model.batch_norms[i] if model.use_batch_norm else None
+            scale, shift = fold_batch_norm(bn)
+            res = x_own.contiguous() if (model.residual and K == conv.out_channels) else None
+            h_out = self.hidden[i % 2]
+            if px is not None:
+                Fn.in_out_bcast(zimg, n, K, prep, conv.bias, self.hidden_peers[i % 2], lo,
+                                px.mode == "multicast" and self.hidden_peers[i % 2].multicast is not None, _abi.ACT_RELU,
+                                scale, shift, res)
+                px.barrier()       # every rank's rows have landed, and nobody reads the previous input any more
+            else:
+                Fn.in_out(zimg, n, K, prep, conv.bias, _abi.ACT_RELU, scale, shift, res, out=h_out[lo:lo + n])
+                if self.world > 1:
+                    dist.all_gather_into_tensor(h_out, h_out[lo:lo + P])
+            if m: m[3].record()
+            del zimg, att          # the next layer's image and attention reuse their memory (Z of K = 166: 5.25 KB per row)
+            h_in = h_out
+        h_own = h_in[lo:lo + n]
+        if isinstance(model, TemporalGNN):
+            return fused.gru_head(h_own, model.gru, model.out), (int(self.plan.start[self.rank]), int(self.plan.start[self.rank + 1]))
+        return model.out(h_own), (int(self.plan.start[self.rank]), int(self.plan.start[self.rank + 1]))

@@ -37,7 +37,7 @@
 extern "C" {
 #endif
 
-#define GNNFD_ABI_VERSION 19
+#define GNNFD_ABI_VERSION 20
 
 typedef void* gnnfd_stream_t; /* cudaStream_t */
 
@@ -372,6 +372,16 @@ typedef struct gnnfd_peers {
 int gnnfd_in_logits_bcast(const float* x, int64_t ldx, int64_t N, int64_t K, const float* W, const float* att_src,
                           const float* att_dst, const gnnfd_peers_t* a_src_all, int64_t row_offset, int use_multicast,
                           float* a_dst, float* xmax, void* prep, gnnfd_stream_t stream);
+/* gnnfd_in_out fused with the all-gather of the layer output: every finished 16-byte piece of output row r (r in [0,n)) is
+ * also stored into row row_offset + r of h_all [n_pos,C] ON EVERY RANK (use_multicast: one multimem.st, replicated by the
+ * switch; else one store per peer).  Same arithmetic as gnnfd_in_out, bit for bit; out (the own rows) may be NULL.  Checked
+ * before anything is launched: 1..GNNFD_MAX_PEERS peers, non-NULL 16-byte aligned peer addresses, a multicast address when
+ * use_multicast; n = 0 launches nothing.  With gnnfd_in_logits_bcast this runs a hidden GAT layer across GPUs exchanging
+ * only h [N,64] (256 B per node) and a_src [N,H] (32 B per node); partition.InputSpaceModelPartition drives it. */
+int gnnfd_in_out_bcast(const void* zimg, int64_t n, int64_t K, const void* prep, const float* bias, int act,
+                       const float* post_scale, const float* post_shift, const float* residual,
+                       const gnnfd_peers_t* h_all, int64_t row_offset, int use_multicast, float* out,
+                       gnnfd_stream_t stream);
 /* out[i] = reduce over ranks of buf_r[offset + i], i in [0,n)  (op 0: sum, 1: max).  use_multicast (sum only, offset and n
  * multiples of 4): multimem.ld_reduce -- the addition happens inside the NVSwitch; else peer loads summed in rank order
  * (deterministic).  The reduce-scatter of the partial da_src [n_pos,H]: every rank reduces ITS OWN row range. */
