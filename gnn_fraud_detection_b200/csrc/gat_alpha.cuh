@@ -89,7 +89,7 @@ __device__ __forceinline__ void alpha_stat_chunk(int beg, int n, const float (&a
 }
 
 // one warp per edge-balanced work item over rowptr; hub rows (above hub_threshold) are left to alpha_hub_*
-template <int H, bool PROJ, bool DROPOUT, bool PACK>
+template <int H, bool PROJ, bool DROPOUT>
 __device__ __forceinline__ void alpha_items_body(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
                                                  const float* __restrict__ a_src, const float* __restrict__ a_dst,
                                                  int r0, int r1, int hub_threshold, float slope, const AlphaOut& out,
@@ -106,10 +106,9 @@ __device__ __forceinline__ void alpha_items_body(const int32_t* __restrict__ row
     int row = 0, beg = 0, n = 0, k = 0, la = 0, lb = 0;
     bool first = false, last = false;
     while (true) {
-        const int kind = PACK ? cur.next_any(rowptr, lane, row, beg, n, first, last, k, la, lb, on_empty)
-                              : (cur.next(rowptr, row, beg, n, first, last, on_empty) ? 1 : 0);
+        const int kind = cur.next_any(rowptr, lane, row, beg, n, first, last, k, la, lb, on_empty);
         if (!kind) break;
-        if (PACK && kind == 2) {
+        if (kind == 2) {
             // pack of k whole rows: segmented scans over the lanes of each row (as fwd_phase_a_pack)
             const bool act = lane < n;
             const int e_id = beg + lane;

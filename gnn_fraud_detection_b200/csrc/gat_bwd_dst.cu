@@ -23,7 +23,6 @@
 
 #include <atomic>
 #include <climits>
-#include <cstdlib>
 
 namespace gnnfd {
 extern std::atomic<long long> g_launches;
@@ -54,9 +53,9 @@ __device__ __forceinline__ void load_g(float (&g)[GE::NS][GE::VW], int64_t i, co
 }
 
 
-// HUB = false: whole rows, results go to da_dst.  HUB = true: one (row, range) segment, the partial t of
-// the segment goes to part_t[chunk_id]; the second sweep is a separate kernel once every chunk's t is known.
-template <class GE, bool CONCAT, bool DROPOUT, bool HUB>
+// One (hub row, range) segment: the partial t of the segment goes to part_t[chunk_id]; the second sweep is a
+// separate kernel once every chunk's t is known.
+template <class GE, bool CONCAT, bool DROPOUT>
 __device__ __forceinline__ void bwd_dst_stream(ChunkCursor& cur, WarpRing<GE, bwd_extra<GE>()>& ring,
                                                const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
                                                const int32_t* __restrict__ perm, const int32_t* __restrict__ csr2csc,
@@ -66,15 +65,12 @@ __device__ __forceinline__ void bwd_dst_stream(ChunkCursor& cur, WarpRing<GE, bw
                                                const float* __restrict__ d_out, float slope,
                                                KeepMask keep, float keep_scale,
                                                float* __restrict__ alpha_used, float* __restrict__ dz, int64_t eg_ld,
-                                               float* __restrict__ da_dst, float* __restrict__ part_t, int chunk_id,
-                                               int lane)
+                                               float* __restrict__ part_t, int chunk_id, int lane)
 {
     constexpr int H = GE::H, NS = GE::NS, VW = GE::VW;
     float* dal_s = reinterpret_cast<float*>(ring.extra);
     int* bits_s = reinterpret_cast<int*>(ring.extra + 32 * H * 4);
-    auto on_empty = [&](int r) {
-        if (!HUB && lane < H) da_dst[int64_t(r) * H + lane] = 0.f;
-    };
+    auto on_empty = [](int) {};
     BwdChunk c0, c1;
     int b0 = 0;
     if (!cur.next(rowptr, c0.row, c0.beg, c0.n, c0.first, c0.last, on_empty)) return;
@@ -83,8 +79,7 @@ __device__ __forceinline__ void bwd_dst_stream(ChunkCursor& cur, WarpRing<GE, bw
     float g0[NS][VW], g1[NS][VW];
     load_g<GE, CONCAT>(g0, c0.row, d_out, lane);
     int issued0 = 0, issued1 = 0;
-    float trow[H];               // running t = sum alpha*d_alpha of the current (multi-chunk) row
-    int row_beg = c0.beg;        // first edge of the current row / segment
+    float trow[H];               // running t = sum alpha*d_alpha of the segment
 #pragma unroll
     for (int h = 0; h < H; ++h) trow[h] = 0.f;
     while (true) {
@@ -99,7 +94,6 @@ __device__ __forceinline__ void bwd_dst_stream(ChunkCursor& cur, WarpRing<GE, bw
             if (c1.first) load_g<GE, CONCAT>(g1, c1.row, d_out, lane);
         }
         if (c0.first) {
-            row_beg = c0.beg;
 #pragma unroll
             for (int h = 0; h < H; ++h) trow[h] = 0.f;
         }
@@ -142,45 +136,13 @@ __device__ __forceinline__ void bwd_dst_stream(ChunkCursor& cur, WarpRing<GE, bw
                 u[h] = live ? alpha[h] * dal[h] * ks : 0.f;
                 au[h] = alpha[h] * ks;
             }
-            if (!HUB && c0.first && c0.last) {
-                // the whole row is in registers: finish it here
-                float o[H], dad[H];
-#pragma unroll
-                for (int h = 0; h < H; ++h) {
-                    const float tt = warp_sum(u[h]);
-                    const float sl = (bits >> h) & 1 ? 1.f : slope;
-                    o[h] = live ? sl * (u[h] - alpha[h] * tt) : 0.f;
-                    dad[h] = warp_sum(o[h]);
-                }
-                if (live) {
-                    store_vecH<H>(alpha_used + pos * eg_ld, au);
-                    store_vecH<H>(dz + pos * eg_ld, o);
-                }
-                if (lane == 0) store_vecH<H>(da_dst + int64_t(c0.row) * H, dad);
-            } else {
-                if (live) {
-                    store_vecH<H>(alpha_used + pos * eg_ld, au);
-                    store_vecH<H>(dz + pos * eg_ld, u);       // parked until t is known
-                }
-#pragma unroll
-                for (int h = 0; h < H; ++h) trow[h] += warp_sum(u[h]);
-                if (c0.last) {
-                    if (HUB) {
-                        if (lane == 0) store_vecH<H>(part_t + int64_t(chunk_id) * H, trow);
-                    } else {
-                        __syncwarp();
-                        RowStat<H> r;
-                        load_row_stat<H>(r, c0.row, a_dst, rowmax, rowsum);
-                        float dad[H];
-#pragma unroll
-                        for (int h = 0; h < H; ++h) dad[h] = 0.f;
-                        dst_sweep2<GE>(r, row_beg, c0.beg + c0.n, col, csr2csc, a_src, slope, trow, lane, dz, eg_ld, dad);
-#pragma unroll
-                        for (int h = 0; h < H; ++h) dad[h] = warp_sum(dad[h]);
-                        if (lane == 0) store_vecH<H>(da_dst + int64_t(c0.row) * H, dad);
-                    }
-                }
+            if (live) {
+                store_vecH<H>(alpha_used + pos * eg_ld, au);
+                store_vecH<H>(dz + pos * eg_ld, u);       // parked until t is known
             }
+#pragma unroll
+            for (int h = 0; h < H; ++h) trow[h] += warp_sum(u[h]);
+            if (c0.last && lane == 0) store_vecH<H>(part_t + int64_t(chunk_id) * H, trow);
         }
         __syncwarp();
         if (!have1) break;
@@ -195,28 +157,6 @@ __device__ __forceinline__ void bwd_dst_stream(ChunkCursor& cur, WarpRing<GE, bw
         b0 ^= 1;
     }
 }
-
-template <class GE, bool CONCAT, bool DROPOUT>
-__global__ void __launch_bounds__(ST_THREADS, st_min_ctas<GE>())
-gat_bwd_dst_items(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col, const int32_t* __restrict__ perm,
-                  const int32_t* __restrict__ csr2csc, const typename GE::XT* __restrict__ xw, const float* __restrict__ a_src,
-                  const float* __restrict__ a_dst, const float* __restrict__ rowmax, const float* __restrict__ rowsum,
-                  const float* __restrict__ d_out, gnnfd_item_plan_t items, int hub_threshold, float slope,
-                  KeepMask keep, float keep_scale, float* __restrict__ alpha_used,
-                  float* __restrict__ dz, int64_t eg_ld, float* __restrict__ da_dst)
-{
-    extern __shared__ __align__(128) uint8_t smem[];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int item = blockIdx.x * ST_WARPS + warp;
-    if (item >= items.n_items) return;
-    WarpRing<GE, bwd_extra<GE>()> ring;
-    ring.init(smem + warp * StreamGeo<GE, bwd_extra<GE>()>::WARP_BYTES, lane);
-    ChunkCursor cur;
-    cur.start_rows(items.item_start[item], items.item_start[item + 1], hub_threshold);
-    bwd_dst_stream<GE, CONCAT, DROPOUT, false>(cur, ring, rowptr, col, perm, csr2csc, xw, a_src, a_dst, rowmax, rowsum, d_out, slope,
-                                               keep, keep_scale, alpha_used, dz, eg_ld, da_dst, nullptr, 0, lane);
-}
-
 
 template <class GE, bool CONCAT, bool DROPOUT>
 __device__ __forceinline__ void bwd_dst_stream_pack(ChunkCursor& cur, WarpRing<GE, bwd_extra<GE>()>& ring,
@@ -435,8 +375,8 @@ gat_bwd_dst_hub1(const int32_t* __restrict__ rowptr, const int32_t* __restrict__
     ring.init(smem + warp * StreamGeo<GE, bwd_extra<GE>()>::WARP_BYTES, lane);
     ChunkCursor cur;
     cur.start_segment(i, beg, end);
-    bwd_dst_stream<GE, CONCAT, DROPOUT, true>(cur, ring, rowptr, col, perm, csr2csc, xw, a_src, a_dst, rowmax, rowsum, d_out, slope,
-                                              keep, keep_scale, alpha_used, dz, eg_ld, nullptr, part_t, c, lane);
+    bwd_dst_stream<GE, CONCAT, DROPOUT>(cur, ring, rowptr, col, perm, csr2csc, xw, a_src, a_dst, rowmax, rowsum, d_out, slope,
+                                        keep, keep_scale, alpha_used, dz, eg_ld, part_t, c, lane);
 }
 
 template <class K>
@@ -467,30 +407,15 @@ static int launch_bwd_dst(const gnnfd_graph_t* g, const void* xw_, const float* 
     // two dense [E',H] arrays, or the halves of one interleaved [E',2H] buffer (dz == alpha_used + H)
     const int64_t eg_ld = (dz == alpha_used + GE::H) ? 2 * GE::H : GE::H;
     int rc = GNNFD_OK;
-#define GNNFD_BWD_ITEMS(CC, DD)                                                                                        \
-    rc = set_smem_bwd(gat_bwd_dst_items<GE, CC, DD>, SMEM);                                                            \
-    if (rc) return rc;                                                                                                 \
-    gat_bwd_dst_items<GE, CC, DD><<<grid, ST_THREADS, SMEM, st>>>(g->rowptr, g->col, g->perm, g->csr2csc, xw, a_src, a_dst, rowmax,  \
-                                                                  rowsum, d_out, g->items_dst, thr, slope, keep, ks,    \
-                                                                  alpha_used, dz, eg_ld, da_dst)
-    static const bool pack = [] {
-        const char* e = getenv("GNNFD_BWD_PACK");           // packs of whole short rows (gat_bwd_dst_items_pack); 0 disables
-        return e ? atoi(e) != 0 : true;
-    }();
+    // packs of whole short rows share one phase A
 #define GNNFD_BWD_ITEMS_PACK(CC, DD)                                                                                   \
     rc = set_smem_bwd(gat_bwd_dst_items_pack<GE, CC, DD>, SMEM);                                                       \
     if (rc) return rc;                                                                                                 \
     gat_bwd_dst_items_pack<GE, CC, DD><<<grid, ST_THREADS, SMEM, st>>>(g->rowptr, g->col, g->perm, g->csr2csc, xw, a_src, a_dst,    \
                                                                        rowmax, rowsum, d_out, g->items_dst, thr, slope, keep, \
                                                                        ks, alpha_used, dz, eg_ld, da_dst)
-    if (pack) {
-        if (concat) { if (drop) { GNNFD_BWD_ITEMS_PACK(true, true); } else { GNNFD_BWD_ITEMS_PACK(true, false); } }
-        else        { if (drop) { GNNFD_BWD_ITEMS_PACK(false, true); } else { GNNFD_BWD_ITEMS_PACK(false, false); } }
-    } else {
-        if (concat) { if (drop) { GNNFD_BWD_ITEMS(true, true); } else { GNNFD_BWD_ITEMS(true, false); } }
-        else        { if (drop) { GNNFD_BWD_ITEMS(false, true); } else { GNNFD_BWD_ITEMS(false, false); } }
-    }
-#undef GNNFD_BWD_ITEMS
+    if (concat) { if (drop) { GNNFD_BWD_ITEMS_PACK(true, true); } else { GNNFD_BWD_ITEMS_PACK(true, false); } }
+    else        { if (drop) { GNNFD_BWD_ITEMS_PACK(false, true); } else { GNNFD_BWD_ITEMS_PACK(false, false); } }
 #undef GNNFD_BWD_ITEMS_PACK
     g_launches += 1;
     if (g->hub_dst.n_hub > 0) {

@@ -18,19 +18,14 @@ int check_graph(const gnnfd_graph_t* g, bool need_csc, const char* who);
 bool gat_bwd_dst_srcmajor_applies(const gnnfd_graph_t* g, int concat);       // gat_bwd_dalpha.cu
 size_t gat_bwd_dst_srcmajor_ws_bytes(const gnnfd_graph_t* g, int H);
 
-#ifndef GNNFD_SRC_MINB
-#define GNNFD_SRC_MINB 4
-#endif
-#ifndef GNNFD_SRC_U
-#define GNNFD_SRC_U 4
-#endif
-constexpr int BWD_U = GNNFD_SRC_U;
-// The rows kernel at 8 x 128 channels (32 accumulators per lane): two CTAs per SM instead of GNNFD_SRC_MINB, and
+constexpr int SRC_MINB = 4;
+constexpr int BWD_U = 4;
+// The rows kernel at 8 x 128 channels (32 accumulators per lane): two CTAs per SM instead of SRC_MINB, and
 // with concat one dO row in flight per lane instead of BWD_U (each is 32 more registers), so that nothing spills.
 template <class GE>
 constexpr int src_minb()
 {
-    return GE::D > 512 ? 2 : GNNFD_SRC_MINB;
+    return GE::D > 512 ? 2 : SRC_MINB;
 }
 template <class GE, bool CONCAT>
 constexpr int src_unroll()

@@ -17,7 +17,6 @@
 
 #include <atomic>
 #include <climits>
-#include <cstdlib>
 
 namespace gnnfd {
 extern std::atomic<long long> g_launches;
@@ -222,27 +221,6 @@ __device__ __forceinline__ void fwd_stream(ChunkCursor& cur, WarpRing<GE>& ring,
         b0 ^= 1;
     }
 }
-
-template <class GE, bool CONCAT, bool DROPOUT>
-__global__ void __launch_bounds__(ST_THREADS, st_min_ctas<GE>())
-gat_fwd_items(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col, const int32_t* __restrict__ perm,
-              const typename GE::XT* __restrict__ xw, const float* __restrict__ a_src,
-              const float* __restrict__ a_dst, EpiParams ep, gnnfd_item_plan_t items,
-              int hub_threshold, float slope, KeepMask keep, float keep_scale,
-              float* __restrict__ out, float* __restrict__ rowmax, float* __restrict__ rowsum)
-{
-    extern __shared__ __align__(128) uint8_t smem[];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int item = blockIdx.x * ST_WARPS + warp;
-    if (item >= items.n_items) return;
-    WarpRing<GE> ring;
-    ring.init(smem + warp * StreamGeo<GE>::WARP_BYTES, lane);
-    ChunkCursor cur;
-    cur.start_rows(items.item_start[item], items.item_start[item + 1], hub_threshold);
-    RowEpilogue<GE, CONCAT> sink{ep, out, rowmax, rowsum};
-    fwd_stream<GE, DROPOUT>(cur, ring, sink, rowptr, col, perm, xw, a_src, a_dst, slope, keep, keep_scale, lane);
-}
-
 
 template <class GE, bool CONCAT, bool DROPOUT>
 __device__ __forceinline__ void fwd_stream_pack(ChunkCursor& cur, WarpRing<GE, 256>& ring, const RowEpilogue<GE, CONCAT>& sink,
@@ -516,31 +494,16 @@ static int launch_fwd(const gnnfd_graph_t* g, const void* xw_, const float* a_sr
     const int thr = g->hub_dst.n_hub > 0 ? g->hub_dst.threshold : INT_MAX;
     const unsigned grid = (unsigned)((g->items_dst.n_items + ST_WARPS - 1) / ST_WARPS);
     int rc = GNNFD_OK;
-#define GNNFD_FWD_ITEMS(CC, DD)                                                                                       \
-    rc = set_smem(gat_fwd_items<GE, CC, DD>, SMEM);                                                                   \
-    if (rc) return rc;                                                                                                \
-    gat_fwd_items<GE, CC, DD><<<grid, ST_THREADS, SMEM, st>>>(g->rowptr, g->col, g->perm, xw, a_src, a_dst, ep,         \
-                                                              g->items_dst, thr, slope, keep, ks, out, rowmax, rowsum)
-    // packs of whole short rows share one phase A (gat_fwd_items_pack): 2.2x on the Elliptic-size graph (2 edges per
-    // row), and still 11 % on the 200M-edge power-law graph, whose rows are mostly short.  GNNFD_FWD_PACK=0 disables it.
-    static const bool pack = [] {
-        const char* e = getenv("GNNFD_FWD_PACK");
-        return e ? atoi(e) != 0 : true;
-    }();
+    // packs of whole short rows share one phase A: 2.2x on the Elliptic-size graph (2 edges per row), and still 11 %
+    // on the 200M-edge power-law graph, whose rows are mostly short, against a kernel that streams row by row
     constexpr int SMEM_P = StreamGeo<GE, 256>::CTA_BYTES;
 #define GNNFD_FWD_ITEMS_PACK(CC, DD)                                                                                  \
     rc = set_smem(gat_fwd_items_pack<GE, CC, DD>, SMEM_P);                                                            \
     if (rc) return rc;                                                                                                \
     gat_fwd_items_pack<GE, CC, DD><<<grid, ST_THREADS, SMEM_P, st>>>(g->rowptr, g->col, g->perm, xw, a_src, a_dst, ep, \
                                                                      g->items_dst, thr, slope, keep, ks, out, rowmax, rowsum)
-    if (pack) {
-        if (concat) { if (drop) { GNNFD_FWD_ITEMS_PACK(true, true); } else { GNNFD_FWD_ITEMS_PACK(true, false); } }
-        else        { if (drop) { GNNFD_FWD_ITEMS_PACK(false, true); } else { GNNFD_FWD_ITEMS_PACK(false, false); } }
-    } else {
-        if (concat) { if (drop) { GNNFD_FWD_ITEMS(true, true); } else { GNNFD_FWD_ITEMS(true, false); } }
-        else        { if (drop) { GNNFD_FWD_ITEMS(false, true); } else { GNNFD_FWD_ITEMS(false, false); } }
-    }
-#undef GNNFD_FWD_ITEMS
+    if (concat) { if (drop) { GNNFD_FWD_ITEMS_PACK(true, true); } else { GNNFD_FWD_ITEMS_PACK(true, false); } }
+    else        { if (drop) { GNNFD_FWD_ITEMS_PACK(false, true); } else { GNNFD_FWD_ITEMS_PACK(false, false); } }
 #undef GNNFD_FWD_ITEMS_PACK
     g_launches += 1;
     if (g->hub_dst.n_hub > 0) {

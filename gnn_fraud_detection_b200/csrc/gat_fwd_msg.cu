@@ -73,7 +73,7 @@ gat_fwd_alpha_items(const int32_t* __restrict__ rowptr, const int32_t* __restric
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int item = blockIdx.x * ROW_WARPS + warp;
     if (item >= items.n_items) return;
-    alpha_items_body<H, true, DROPOUT, true>(rowptr, col, a_src, a_dst, items.item_start[item], items.item_start[item + 1],
+    alpha_items_body<H, true, DROPOUT>(rowptr, col, a_src, a_dst, items.item_start[item], items.item_start[item + 1],
                                              hub_threshold, slope, out, rowmax, rowsum, lane);
 }
 template <int H>

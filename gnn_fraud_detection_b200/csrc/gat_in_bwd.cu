@@ -12,20 +12,16 @@
 #include "in_common.cuh"
 #include "gat_phase_bwd.cuh"
 
-#ifndef GNNFD_IN_UNROLL_BWD
-#define GNNFD_IN_UNROLL_BWD 4
-#endif
 
 #include <atomic>
 #include <climits>
-#include <cstdlib>
 
 namespace gnnfd {
 extern std::atomic<long long> g_launches;
 int check_graph(const gnnfd_graph_t* g, bool need_csc, const char* who);
 
 namespace in {
-constexpr int IN_UNROLL_BWD = GNNFD_IN_UNROLL_BWD;
+constexpr int IN_UNROLL_BWD = 4;
 bool in_x_ok(const float* x, int64_t ldx, int KP);   // gat_in_fwd.cu
 
 
@@ -149,9 +145,9 @@ struct GdBuf {
     }
 };
 
-// HUB = false: whole rows (optionally packs of short rows), results go to da_dst.  HUB = true: one (row, range) segment,
-// the partial t of the segment goes to part_t[chunk_id]; the second sweep is a separate kernel.
-template <int N4, bool DROPOUT, bool PACK, bool HUB>
+// HUB = false: whole rows and packs of short rows, results go to da_dst.  HUB = true: one (row, range) segment, the
+// partial t of the segment goes to part_t[chunk_id]; the second sweep is a separate kernel.
+template <int N4, bool DROPOUT, bool HUB>
 __device__ __forceinline__ void in_bwd_stream(ChunkCursor& cur, BwdRing& ring, GdBuf<N4>& gdb, const int32_t* __restrict__ rowptr,
                                               const int32_t* __restrict__ perm, const int32_t* __restrict__ csr2csc,
                                               const float* __restrict__ alpha_g, const int32_t* __restrict__ jflag, float slope,
@@ -159,6 +155,7 @@ __device__ __forceinline__ void in_bwd_stream(ChunkCursor& cur, BwdRing& ring, G
                                               float* __restrict__ part_t, int chunk_id, int lane)
 {
     using RG = RowGeo<N4>;
+    constexpr bool PACK = !HUB;     // the row stream also hands out packs of short rows; a hub segment is part of one row
     const int h = lane >> 2, q = lane & 3, n4 = gdb.KP >> 2;
     float* dal_s = reinterpret_cast<float*>(ring.extra);
     int* bits_s = reinterpret_cast<int*>(ring.extra + 32 * H * 4);
@@ -344,12 +341,10 @@ __device__ __forceinline__ void gdbuf_init(GdBuf<N4>& gdb, BwdRing& ring, const 
     gdb.KP = KP;
 }
 
-#ifndef GNNFD_IN_BWD_CTAS
-#define GNNFD_IN_BWD_CTAS 4
-#endif
+constexpr int IN_BWD_CTAS = 4;
 
-template <int N4, bool DROPOUT, bool PACK>
-__global__ void __launch_bounds__(IN_THREADS, GNNFD_IN_BWD_CTAS)
+template <int N4, bool DROPOUT>
+__global__ void __launch_bounds__(IN_THREADS, IN_BWD_CTAS)
 gat_in_bwd_items(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ perm, const int32_t* __restrict__ csr2csc,
                  const float* __restrict__ x, int64_t ldx, int KP, const float* __restrict__ alpha,
                  const int32_t* __restrict__ jflag, const float* __restrict__ gd, gnnfd_item_plan_t items, int item_lo,
@@ -367,13 +362,13 @@ gat_in_bwd_items(const int32_t* __restrict__ rowptr, const int32_t* __restrict__
     gdbuf_init(gdb, ring, gd, F, KP);
     ChunkCursor cur;
     cur.start_rows(items.item_start[item], items.item_start[item + 1], hub_threshold);
-    in_bwd_stream<N4, DROPOUT, PACK, false>(cur, ring, gdb, rowptr, perm, csr2csc, alpha, jflag, slope, keep, keep_scale, dz, da_dst,
-                                            nullptr, 0, lane);
+    in_bwd_stream<N4, DROPOUT, false>(cur, ring, gdb, rowptr, perm, csr2csc, alpha, jflag, slope, keep, keep_scale, dz, da_dst,
+                                      nullptr, 0, lane);
 }
 
 // hub rows, step 1: one warp per chunk -- first sweep, partial t (rows outside [row_lo, row_hi) belong to another block)
 template <int N4, bool DROPOUT>
-__global__ void __launch_bounds__(IN_THREADS, GNNFD_IN_BWD_CTAS)
+__global__ void __launch_bounds__(IN_THREADS, IN_BWD_CTAS)
 gat_in_bwd_hub1(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ perm, const int32_t* __restrict__ csr2csc,
                 const float* __restrict__ x, int64_t ldx, int KP, const float* __restrict__ alpha,
                 const int32_t* __restrict__ jflag, const float* __restrict__ gd, gnnfd_hub_plan_t plan, int row_lo, int row_hi,
@@ -395,8 +390,8 @@ gat_in_bwd_hub1(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ 
     gdbuf_init(gdb, ring, gd, F, KP);
     ChunkCursor cur;
     cur.start_segment(i, beg, end);
-    in_bwd_stream<N4, DROPOUT, false, true>(cur, ring, gdb, rowptr, perm, csr2csc, alpha, jflag, slope, keep, keep_scale, dz, nullptr,
-                                            part_t, c, lane);
+    in_bwd_stream<N4, DROPOUT, true>(cur, ring, gdb, rowptr, perm, csr2csc, alpha, jflag, slope, keep, keep_scale, dz, nullptr,
+                                     part_t, c, lane);
 }
 
 // hub rows, step 2: second sweep of every chunk with the row's total t, partial da_dst
@@ -488,27 +483,22 @@ int gnnfd_in_bwd_edges(const gnnfd_graph_t* g, const float* x, int64_t ldx, int6
         part_dad = carve<float>(p, size_t(pl.n_chunk) * H);
         t_total = carve<float>(p, size_t(pl.n_hub) * H);
     }
-    static const bool pack = [] {
-        const char* e = getenv("GNNFD_BWD_PACK");
-        return e ? atoi(e) != 0 : true;
-    }();
     if ((phase & 1) && item_hi > item_lo) {
         const unsigned grid = (unsigned)((item_hi - item_lo + IN_WARPS - 1) / IN_WARPS);
         const unsigned gc = (unsigned)((pl.n_chunk + IN_WARPS - 1) / IN_WARPS);
-#define GNNFD_IN_BWD(NN, DD, PP)                                                                                       \
-    rc = in_set_smem_bwd(gat_in_bwd_items<NN, DD, PP>, smem);                                                          \
+#define GNNFD_IN_BWD(NN, DD)                                                                                           \
+    rc = in_set_smem_bwd(gat_in_bwd_items<NN, DD>, smem);                                                              \
     if (rc) return rc;                                                                                                 \
-    gat_in_bwd_items<NN, DD, PP><<<grid, IN_THREADS, smem, st>>>(g->rowptr, g->perm, g->csr2csc, x, ldx, d.KP, alpha, jflag, gd0, \
-                                                                 g->items_dst, (int)item_lo, (int)item_hi, thr, negative_slope,  \
-                                                                 keep, ks, dz, da_dst)
+    gat_in_bwd_items<NN, DD><<<grid, IN_THREADS, smem, st>>>(g->rowptr, g->perm, g->csr2csc, x, ldx, d.KP, alpha, jflag, gd0,     \
+                                                             g->items_dst, (int)item_lo, (int)item_hi, thr, negative_slope,      \
+                                                             keep, ks, dz, da_dst)
 #define GNNFD_IN_HUB1(NN, DD)                                                                                          \
     rc = in_set_smem_bwd(gat_in_bwd_hub1<NN, DD>, smem);                                                               \
     if (rc) return rc;                                                                                                 \
     gat_in_bwd_hub1<NN, DD><<<gc, IN_THREADS, smem, st>>>(g->rowptr, g->perm, g->csr2csc, x, ldx, d.KP, alpha, jflag, gd0, pl,   \
                                                           (int)row_lo, (int)row_hi, negative_slope, keep, ks, dz, part_t)
 #define GNNFD_IN_BWD_ALL(NN)                                                                                           \
-    if (pack) { if (drop) { GNNFD_IN_BWD(NN, true, true); } else { GNNFD_IN_BWD(NN, false, true); } }                  \
-    else      { if (drop) { GNNFD_IN_BWD(NN, true, false); } else { GNNFD_IN_BWD(NN, false, false); } }                \
+    if (drop) { GNNFD_IN_BWD(NN, true); } else { GNNFD_IN_BWD(NN, false); }                                            \
     g_launches += 1;                                                                                                   \
     if (pl.n_hub > 0) {                                                                                                \
         if (drop) { GNNFD_IN_HUB1(NN, true); } else { GNNFD_IN_HUB1(NN, false); }                                      \

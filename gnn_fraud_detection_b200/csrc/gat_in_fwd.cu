@@ -15,13 +15,8 @@
 #include "gat_stream.cuh"
 #include "gat_alpha.cuh"
 
-#ifndef GNNFD_IN_UNROLL_FWD
-#define GNNFD_IN_UNROLL_FWD 1     // the row epilogue (image write) sits inside the edge loop: unrolling it 4x thrashes the i-cache
-#endif
-
 #include <atomic>
 #include <climits>
-#include <cstdlib>
 
 namespace gnnfd {
 extern std::atomic<long long> g_launches;
@@ -29,7 +24,7 @@ int check_graph(const gnnfd_graph_t* g, bool need_csc, const char* who);
 int in_build_gd_image(const float* W, int K, void* prep, cudaStream_t st);   // in_gemm.cu
 
 namespace in {
-constexpr int IN_UNROLL_FWD = GNNFD_IN_UNROLL_FWD;
+constexpr int IN_UNROLL_FWD = 1;     // the row epilogue (image write) sits inside the edge loop: unrolling it 4x thrashes the i-cache
 
 // ---- u = W_h^T att  ([2H][KP]) --------------------------------------------------------------------------------------
 __global__ void in_u_kernel(const float* __restrict__ W, const float* __restrict__ att_src, const float* __restrict__ att_dst,
@@ -263,7 +258,6 @@ __device__ __forceinline__ void acc_zero(float2 (&acc)[NA])
 // edges without any softmax state: no logit gathers, no exp, no scans, no row statistics in their registers.
 // The kernels run the attention pass of gat_alpha.cuh (PROJ = false) at H = 8, without dropout: the feature passes apply it.
 // =====================================================================================================================
-template <bool PACK>
 __global__ void __launch_bounds__(IN_THREADS)
 in_alpha_items(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col, const float* __restrict__ a_src,
                const float* __restrict__ a_dst, gnnfd_item_plan_t items, int hub_threshold, float slope,
@@ -272,8 +266,8 @@ in_alpha_items(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ c
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int item = blockIdx.x * IN_WARPS + warp;
     if (item >= items.n_items) return;
-    alpha_items_body<H, false, false, PACK>(rowptr, col, a_src, a_dst, items.item_start[item], items.item_start[item + 1],
-                                            hub_threshold, slope, out, rowmax, rowsum, lane);
+    alpha_items_body<H, false, false>(rowptr, col, a_src, a_dst, items.item_start[item], items.item_start[item + 1],
+                                      hub_threshold, slope, out, rowmax, rowsum, lane);
 }
 
 // hub rows: (1) statistics of every 512-edge chunk, (2) one thread per (hub row, head) folds them in chunk order, (3) write sweep
@@ -339,8 +333,9 @@ __device__ __forceinline__ void stage_chunk(FeatChunk& c, const float* __restric
     __syncwarp();
 }
 
-// HUB: one (row, range) segment whose partial sum goes to the sink at the end; else whole rows, finished at the flags
-template <int N4, bool DROPOUT, bool PACK, bool HUB, class Sink>
+// HUB: one (row, range) segment whose partial sum goes to the sink at the end; else whole rows and packs of rows,
+// finished at the flags
+template <int N4, bool DROPOUT, bool HUB, class Sink>
 __device__ __forceinline__ void in_fwd_stream(ChunkCursor& cur, InRing& ring, const Sink& sink, const int32_t* __restrict__ rowptr,
                                               const int32_t* __restrict__ perm, int n4, const float* __restrict__ alpha,
                                               const int32_t* __restrict__ jflag, KeepMask keep, float keep_scale, int lane)
@@ -354,7 +349,7 @@ __device__ __forceinline__ void in_fwd_stream(ChunkCursor& cur, InRing& ring, co
     auto next = [&](FeatChunk& c) -> bool {
         bool first, last;
         int k, la, lb;
-        if (PACK) return cur.next_any(rowptr, lane, c.row, c.beg, c.n, first, last, k, la, lb, on_empty) != 0;
+        if (!HUB) return cur.next_any(rowptr, lane, c.row, c.beg, c.n, first, last, k, la, lb, on_empty) != 0;
         return cur.next(rowptr, c.row, c.beg, c.n, first, last, on_empty);
     };
     if (!next(c0)) return;
@@ -416,12 +411,10 @@ __device__ __forceinline__ void in_fwd_stream(ChunkCursor& cur, InRing& ring, co
 }
 
 constexpr int FWD_EXTRA = 0;
-#ifndef GNNFD_IN_FWD_CTAS
-#define GNNFD_IN_FWD_CTAS 5
-#endif
+constexpr int IN_FWD_CTAS = 5;
 
-template <int N4, bool DROPOUT, bool PACK>
-__global__ void __launch_bounds__(IN_THREADS, GNNFD_IN_FWD_CTAS)
+template <int N4, bool DROPOUT>
+__global__ void __launch_bounds__(IN_THREADS, IN_FWD_CTAS)
 gat_in_fwd_items(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ perm, const float* __restrict__ x, int64_t ldx,
                  const float* __restrict__ alpha, const int32_t* __restrict__ jflag, gnnfd_item_plan_t items, int hub_threshold,
                  KeepMask keep, float keep_scale, ZSink<N4> sink)
@@ -434,12 +427,12 @@ gat_in_fwd_items(const int32_t* __restrict__ rowptr, const int32_t* __restrict__
     ring.init(smem + warp * in_warp_bytes(sink.KP, FWD_EXTRA), x, ldx, sink.KP, lane);
     ChunkCursor cur;
     cur.start_rows(items.item_start[item], items.item_start[item + 1], hub_threshold);
-    in_fwd_stream<N4, DROPOUT, PACK, false>(cur, ring, sink, rowptr, perm, sink.KP >> 2, alpha, jflag, keep, keep_scale, lane);
+    in_fwd_stream<N4, DROPOUT, false>(cur, ring, sink, rowptr, perm, sink.KP >> 2, alpha, jflag, keep, keep_scale, lane);
 }
 
 // one warp per (hub row, chunk): partial accumulators
 template <int N4, bool DROPOUT>
-__global__ void __launch_bounds__(IN_THREADS, GNNFD_IN_FWD_CTAS)
+__global__ void __launch_bounds__(IN_THREADS, IN_FWD_CTAS)
 gat_in_fwd_hub_chunks(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ perm, const float* __restrict__ x, int64_t ldx,
                       int KP, const float* __restrict__ alpha, const int32_t* __restrict__ jflag, gnnfd_hub_plan_t plan,
                       KeepMask keep, float keep_scale, float* __restrict__ part_acc)
@@ -457,7 +450,7 @@ gat_in_fwd_hub_chunks(const int32_t* __restrict__ rowptr, const int32_t* __restr
     ChunkCursor cur;
     cur.start_segment(i, beg, end);
     ZPartialSink<N4> sink{part_acc, c};
-    in_fwd_stream<N4, DROPOUT, false, true>(cur, ring, sink, rowptr, perm, KP >> 2, alpha, jflag, keep, keep_scale, lane);
+    in_fwd_stream<N4, DROPOUT, true>(cur, ring, sink, rowptr, perm, KP >> 2, alpha, jflag, keep, keep_scale, lane);
 }
 
 // one CTA per hub row: warp w sums chunks w, w+8, ..., the eight warp sums are added in warp order -- a fixed order, so the
@@ -508,15 +501,8 @@ static int launch_in_alpha(const gnnfd_graph_t* g, const float* a_src, const flo
 {
     const int thr = g->hub_dst.n_hub > 0 ? g->hub_dst.threshold : INT_MAX;
     const unsigned grid = (unsigned)((g->items_dst.n_items + IN_WARPS - 1) / IN_WARPS);
-    static const bool pack = [] {
-        const char* e = getenv("GNNFD_FWD_PACK");
-        return e ? atoi(e) != 0 : true;
-    }();
     const AlphaOut out{alpha, jflag, nullptr, KeepMask(), 1.f};
-    if (pack)
-        in_alpha_items<true><<<grid, IN_THREADS, 0, st>>>(g->rowptr, g->col, a_src, a_dst, g->items_dst, thr, slope, out, rowmax, rowsum);
-    else
-        in_alpha_items<false><<<grid, IN_THREADS, 0, st>>>(g->rowptr, g->col, a_src, a_dst, g->items_dst, thr, slope, out, rowmax, rowsum);
+    in_alpha_items<<<grid, IN_THREADS, 0, st>>>(g->rowptr, g->col, a_src, a_dst, g->items_dst, thr, slope, out, rowmax, rowsum);
     g_launches += 1;
     if (g->hub_dst.n_hub > 0) {
         const gnnfd_hub_plan_t& pl = g->hub_dst;
@@ -546,18 +532,13 @@ static int launch_in_fwd(const gnnfd_graph_t* g, const float* x, int64_t ldx, co
     const int smem = IN_WARPS * in_warp_bytes(d.KP, FWD_EXTRA);
     const unsigned grid = (unsigned)((g->items_dst.n_items + IN_WARPS - 1) / IN_WARPS);
     ZSink<N4> sink{reinterpret_cast<uint8_t*>(zimg), scal, d.KP, d.NKB};
-    static const bool pack = [] {
-        const char* e = getenv("GNNFD_FWD_PACK");
-        return e ? atoi(e) != 0 : true;
-    }();
     int rc = GNNFD_OK;
-#define GNNFD_IN_FWD(DD, PP)                                                                                           \
-    rc = in_set_smem(gat_in_fwd_items<N4, DD, PP>, smem);                                                              \
+#define GNNFD_IN_FWD(DD)                                                                                               \
+    rc = in_set_smem(gat_in_fwd_items<N4, DD>, smem);                                                                  \
     if (rc) return rc;                                                                                                 \
-    gat_in_fwd_items<N4, DD, PP><<<grid, IN_THREADS, smem, st>>>(g->rowptr, g->perm, x, ldx, alpha, jflag, g->items_dst, thr, keep, \
-                                                                 ks, sink)
-    if (pack) { if (drop) { GNNFD_IN_FWD(true, true); } else { GNNFD_IN_FWD(false, true); } }
-    else      { if (drop) { GNNFD_IN_FWD(true, false); } else { GNNFD_IN_FWD(false, false); } }
+    gat_in_fwd_items<N4, DD><<<grid, IN_THREADS, smem, st>>>(g->rowptr, g->perm, x, ldx, alpha, jflag, g->items_dst, thr, keep, ks, \
+                                                             sink)
+    if (drop) { GNNFD_IN_FWD(true); } else { GNNFD_IN_FWD(false); }
 #undef GNNFD_IN_FWD
     g_launches += 1;
     if (g->hub_dst.n_hub > 0) {

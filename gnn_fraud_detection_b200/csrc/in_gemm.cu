@@ -563,10 +563,7 @@ namespace in {
 constexpr int G3_THREADS = 192;
 constexpr uint32_t G3_A = 2 * KBLOCK;              // 64 KB: two consecutive k-blocks (128 features), hi + lo each
 constexpr uint32_t G3_B = 2 * PLANE;               // 32 KB: dO tile, hi + lo planes
-#ifndef GNNFD_G3_FLUSH
-#define GNNFD_G3_FLUSH 4
-#endif
-constexpr int G3_FLUSH = GNNFD_G3_FLUSH;   // node tiles per accumulation chain (chain = G3_FLUSH x 8 k-steps x 3 MMAs)
+constexpr int G3_FLUSH = 4;   // node tiles per accumulation chain (chain = G3_FLUSH x 8 k-steps x 3 MMAs)
 constexpr int G3_STG_LD = 33;
 constexpr size_t G3_SMEM = 2 * size_t(G3_A) + 2 * size_t(G3_B) + 4 * 32 * G3_STG_LD * 4 + 1024;
 

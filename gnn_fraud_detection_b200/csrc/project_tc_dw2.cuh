@@ -1,9 +1,8 @@
 // Pipelined dW partials on the tensor cores:  P[slab][o][k] = sum_{n in slab} dxw[n][o] * x[n][k]   (3xTF32)
 //
-// Successor of dw_tc (project_tc.cu), which is bound by the load/store pipe that its two co-resident CTAs share:
-// every CTA there re-stages the same x tile for its own 128 output rows.  Here ONE persistent CTA per SM owns 256
-// output rows (two M=128 accumulators in TMEM that share the B = x operand), so the x tile is staged once per 256
-// rows, and the staging of node block i+1.. overlaps the MMAs of block i through a three-stage mbarrier ring:
+// Staging the operands is bound by the load/store pipe, so ONE persistent CTA per SM owns 256 output rows (two
+// M=128 accumulators in TMEM that share the B = x operand): the x tile is staged once per 256 rows rather than once
+// per 128, and the staging of node block i+1.. overlaps the MMAs of block i through a three-stage mbarrier ring:
 //   warps 0-7   producers: node group kq = warp/2 (4 nodes) of each 16-node stage; even warps stage the A operand
 //               (dxw rows, both o-tiles, float4), odd warps the B operand (x rows, float2 pairs when aligned);
 //               the global loads of the next stage are in flight while the current one is split and stored

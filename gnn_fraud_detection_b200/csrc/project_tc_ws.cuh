@@ -1,4 +1,5 @@
 // Persistent, warp-specialised tcgen05 GEMM:  C[M, NT*256] = A[M, Kd] * B^T  (3xTF32, fp32 accumulate in TMEM).
+// The projection backward's dx = dxw @ W; the forward runs the 2-SM variant (project_tc_ws2.cuh).
 //
 // One CTA per SM, 10 warps:
 //   warps 0-3  A producers: coalesced 128-byte row segments of x -> hi/lo split -> swizzled K-major smem stage
@@ -6,7 +7,7 @@
 //   warp  4    MMA issuer (one elected lane): waits only for FULL barriers, so the tcgen05.mma's of consecutive
 //              k-blocks queue back to back; tcgen05.commit releases the smem stage and, on a tile's last
 //              k-block, hands the TMEM accumulator to the epilogue
-//   warps 5-8  epilogue: tcgen05.ld of their TMEM lane quadrant, logit dot products, staged coalesced stores
+//   warps 5-8  epilogue: tcgen05.ld of their TMEM lane quadrant, staged coalesced stores of the first n_valid columns
 //   warp  9    B producer: cp.async.bulk of the prebuilt weight image of each k-block as soon as its stage drains
 // Two smem stages (A 2x32 KB, B 2x64 KB) and two TMEM accumulators (2 x 256 columns) keep all roles busy:
 // the epilogue of tile t overlaps the mainloop of tile t+1, the copies of k-block k+1 overlap the MMAs of k.
@@ -38,14 +39,10 @@ __device__ __forceinline__ void mbar_arrive(uint64_t* bar)
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 
-template <int EPI, bool OUT_BF16, bool FAST = false, int HC = 64>
 __global__ void __launch_bounds__(WS_THREADS, 1)
 gemm_tc_ws(const float* __restrict__ A, int64_t lda, int64_t M, int Kd, const float* __restrict__ b_img, int n_kb,
-           int n_col_tiles, float* __restrict__ Cf, __nv_bfloat16* __restrict__ Cb, int64_t ldc, int n_valid,
-           const float* __restrict__ att_src, const float* __restrict__ att_dst, float* __restrict__ a_src,
-           float* __restrict__ a_dst, int H)
+           int n_col_tiles, float* __restrict__ Cf, int64_t ldc, int n_valid)
 {
-    static_assert(HC == 32 || HC == 64 || HC == 128, "the logits epilogue covers heads of 32, 64 or 128 columns");
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     __shared__ uint64_t full_a[2], full_b[2], empty[2], acc_full[2], acc_empty[2];
@@ -182,10 +179,8 @@ gemm_tc_ws(const float* __restrict__ A, int64_t lda, int64_t M, int Kd, const fl
                         const uint64_t dah = make_desc(a_hi + ko, 16, 1024), dal = make_desc(a_lo + ko, 16, 1024);
                         const uint64_t dbh = make_desc(b_hi + ko, 16, 1024), dbl = make_desc(b_lo + ko, 16, 1024);
                         umma_tf32(d, dah, dbh, IDESC, (kb | ks) ? 1u : 0u);
-                        if (!FAST) {
-                            umma_tf32(d, dal, dbh, IDESC, 1u);
-                            umma_tf32(d, dah, dbl, IDESC, 1u);
-                        }
+                        umma_tf32(d, dal, dbh, IDESC, 1u);
+                        umma_tf32(d, dah, dbl, IDESC, 1u);
                     }
                     umma_commit(&empty[s]);                           // stage reusable once these MMAs retire
                     if (kb == n_kb - 1) umma_commit(&acc_full[buf]);  // ... and the tile is complete
@@ -207,9 +202,9 @@ gemm_tc_ws(const float* __restrict__ A, int64_t lda, int64_t M, int Kd, const fl
             if (u > 0) mbar_wait(&empty[s], uint32_t((u - 1) & 1));
             uint8_t* sB = smem + s * WS_STAGE + 2 * WS_A_PART;
             const float* img = b_img + (size_t(nt) * n_kb + kb) * 2 * (size_t(WS_BN) * BK);
-            if (elect_one()) {     // FAST needs only the hi half of the image
-                mbar_expect_tx(&full_b[s], (FAST ? 1 : 2) * WS_B_PART);
-                bulk_g2s(sB, img, (FAST ? 1 : 2) * WS_B_PART, &full_b[s]);
+            if (elect_one()) {
+                mbar_expect_tx(&full_b[s], 2 * WS_B_PART);
+                bulk_g2s(sB, img, 2 * WS_B_PART, &full_b[s]);
             }
             __syncwarp();
         };
@@ -225,32 +220,11 @@ gemm_tc_ws(const float* __restrict__ A, int64_t lda, int64_t M, int Kd, const fl
             const int buf = int(j & 1);
             mbar_wait(&acc_full[buf], uint32_t((j >> 1) & 1));
             tc_fence_after();
-            const int64_t row = m0 + quad * 32 + lane;
-            float ps = 0.f, pd = 0.f;
 #pragma unroll 1
             for (int ch = 0; ch < WS_BN / 32; ++ch) {
                 uint32_t v[32];
                 tmem_ld32(tmem_base + (uint32_t(quad * 32) << 16) + uint32_t(buf * WS_BN + ch * 32), v);
                 const int col0 = nt * WS_BN + ch * 32;
-                if (EPI == 1) {
-#pragma unroll
-                    for (int c = 0; c < 32; c += 4) {
-                        const float4 as4 = __ldg(reinterpret_cast<const float4*>(att_src + col0 + c));
-                        const float4 ad4 = __ldg(reinterpret_cast<const float4*>(att_dst + col0 + c));
-                        ps = fmaf(__uint_as_float(v[c]), as4.x, ps); pd = fmaf(__uint_as_float(v[c]), ad4.x, pd);
-                        ps = fmaf(__uint_as_float(v[c + 1]), as4.y, ps); pd = fmaf(__uint_as_float(v[c + 1]), ad4.y, pd);
-                        ps = fmaf(__uint_as_float(v[c + 2]), as4.z, ps); pd = fmaf(__uint_as_float(v[c + 2]), ad4.z, pd);
-                        ps = fmaf(__uint_as_float(v[c + 3]), as4.w, ps); pd = fmaf(__uint_as_float(v[c + 3]), ad4.w, pd);
-                    }
-                    if ((ch & (HC / 32 - 1)) == HC / 32 - 1) {      // HC/32 32-column chunks per head
-                        if (row < M) {
-                            const int h = col0 / HC;
-                            a_src[row * H + h] = ps;
-                            a_dst[row * H + h] = pd;
-                        }
-                        ps = pd = 0.f;
-                    }
-                }
                 // staged through smem so that every store instruction writes four full 128-byte lines (writing each
                 // thread's own row directly was measured 40 % slower: 16-byte fragments of 32 different lines)
                 __syncwarp();
@@ -266,24 +240,10 @@ gemm_tc_ws(const float* __restrict__ A, int64_t lda, int64_t M, int Kd, const fl
                     const int64_t gm = m0 + quad * 32 + r;
                     const float4 o = *reinterpret_cast<const float4*>(stg + r * WS_STG_LD + cq);
                     if (gm < M) {
-                        if (EPI == 1) {
-                            if (OUT_BF16) {
-                                __nv_bfloat162 lo2 = __floats2bfloat162_rn(o.x, o.y), hi2 = __floats2bfloat162_rn(o.z, o.w);
-                                uint2 pk;
-                                pk.x = *reinterpret_cast<uint32_t*>(&lo2);
-                                pk.y = *reinterpret_cast<uint32_t*>(&hi2);
-                                *reinterpret_cast<uint2*>(Cb + gm * ldc + col0 + cq) = pk;
-                            } else {
-                                *reinterpret_cast<float4*>(Cf + gm * ldc + col0 + cq) = o;
-                            }
-                        } else if (EPI == 2) {     // plain fp32 store, ldc and n_valid multiples of 4: one 16-byte store
-                            if (col0 + cq < n_valid) *reinterpret_cast<float4*>(Cf + gm * ldc + col0 + cq) = o;
-                        } else {
-                            const float ov[4] = {o.x, o.y, o.z, o.w};
+                        const float ov[4] = {o.x, o.y, o.z, o.w};
 #pragma unroll
-                            for (int k = 0; k < 4; ++k)
-                                if (col0 + cq + k < n_valid) Cf[gm * ldc + col0 + cq + k] = ov[k];
-                        }
+                        for (int k = 0; k < 4; ++k)
+                            if (col0 + cq + k < n_valid) Cf[gm * ldc + col0 + cq + k] = ov[k];
                     }
                 }
             }

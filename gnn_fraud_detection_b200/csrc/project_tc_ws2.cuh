@@ -95,10 +95,12 @@ __device__ __forceinline__ void umma2_commit_both(uint64_t* bar)
                  : "memory");
 }
 
-template <int EPI, bool OUT_BF16, bool FAST = false, int HC = 64>
+// The forward projection: stores xw (fp32, or bf16 with OUT_BF16) and the per-head logits of heads HC columns wide;
+// FAST runs one TF32 pass instead of the compensated three.
+template <bool OUT_BF16, bool FAST = false, int HC = 64>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(WS2_THREADS, 1)
 gemm_tc_ws2(const float* __restrict__ A, int64_t lda, int64_t M, int Kd, const float* __restrict__ b_img, int n_kb,
-            int n_col_tiles, float* __restrict__ Cf, __nv_bfloat16* __restrict__ Cb, int64_t ldc, int n_valid,
+            int n_col_tiles, float* __restrict__ Cf, __nv_bfloat16* __restrict__ Cb, int64_t ldc,
             const float* __restrict__ att_src, const float* __restrict__ att_dst, float* __restrict__ a_src,
             float* __restrict__ a_dst, int H)
 {
@@ -295,24 +297,22 @@ gemm_tc_ws2(const float* __restrict__ A, int64_t lda, int64_t M, int Kd, const f
                 uint32_t v[32];
                 tmem_ld32(tmem_base + (uint32_t(quad * 32) << 16) + uint32_t(buf * WS_BN + ch * 32), v);
                 const int col0 = nt * WS_BN + ch * 32;
-                if (EPI == 1) {
 #pragma unroll
-                    for (int c = 0; c < 32; c += 4) {
-                        const float4 as4 = __ldg(reinterpret_cast<const float4*>(att_src + col0 + c));
-                        const float4 ad4 = __ldg(reinterpret_cast<const float4*>(att_dst + col0 + c));
-                        ps = fmaf(__uint_as_float(v[c]), as4.x, ps); pd = fmaf(__uint_as_float(v[c]), ad4.x, pd);
-                        ps = fmaf(__uint_as_float(v[c + 1]), as4.y, ps); pd = fmaf(__uint_as_float(v[c + 1]), ad4.y, pd);
-                        ps = fmaf(__uint_as_float(v[c + 2]), as4.z, ps); pd = fmaf(__uint_as_float(v[c + 2]), ad4.z, pd);
-                        ps = fmaf(__uint_as_float(v[c + 3]), as4.w, ps); pd = fmaf(__uint_as_float(v[c + 3]), ad4.w, pd);
+                for (int c = 0; c < 32; c += 4) {
+                    const float4 as4 = __ldg(reinterpret_cast<const float4*>(att_src + col0 + c));
+                    const float4 ad4 = __ldg(reinterpret_cast<const float4*>(att_dst + col0 + c));
+                    ps = fmaf(__uint_as_float(v[c]), as4.x, ps); pd = fmaf(__uint_as_float(v[c]), ad4.x, pd);
+                    ps = fmaf(__uint_as_float(v[c + 1]), as4.y, ps); pd = fmaf(__uint_as_float(v[c + 1]), ad4.y, pd);
+                    ps = fmaf(__uint_as_float(v[c + 2]), as4.z, ps); pd = fmaf(__uint_as_float(v[c + 2]), ad4.z, pd);
+                    ps = fmaf(__uint_as_float(v[c + 3]), as4.w, ps); pd = fmaf(__uint_as_float(v[c + 3]), ad4.w, pd);
+                }
+                if ((ch & (HC / 32 - 1)) == HC / 32 - 1) {      // HC/32 32-column chunks per head
+                    if (row < M) {
+                        const int h = col0 / HC;
+                        a_src[row * H + h] = ps;
+                        a_dst[row * H + h] = pd;
                     }
-                    if ((ch & (HC / 32 - 1)) == HC / 32 - 1) {      // HC/32 32-column chunks per head
-                        if (row < M) {
-                            const int h = col0 / HC;
-                            a_src[row * H + h] = ps;
-                            a_dst[row * H + h] = pd;
-                        }
-                        ps = pd = 0.f;
-                    }
+                    ps = pd = 0.f;
                 }
                 __syncwarp();
 #pragma unroll
@@ -327,21 +327,14 @@ gemm_tc_ws2(const float* __restrict__ A, int64_t lda, int64_t M, int Kd, const f
                     const int64_t gm = m0 + quad * 32 + r;
                     const float4 o = *reinterpret_cast<const float4*>(stg + r * WS_STG_LD + cq);
                     if (gm < M) {
-                        if (EPI == 1) {
-                            if (OUT_BF16) {
-                                __nv_bfloat162 lo2 = __floats2bfloat162_rn(o.x, o.y), hi2 = __floats2bfloat162_rn(o.z, o.w);
-                                uint2 pk;
-                                pk.x = *reinterpret_cast<uint32_t*>(&lo2);
-                                pk.y = *reinterpret_cast<uint32_t*>(&hi2);
-                                *reinterpret_cast<uint2*>(Cb + gm * ldc + col0 + cq) = pk;
-                            } else {
-                                *reinterpret_cast<float4*>(Cf + gm * ldc + col0 + cq) = o;
-                            }
+                        if (OUT_BF16) {
+                            __nv_bfloat162 lo2 = __floats2bfloat162_rn(o.x, o.y), hi2 = __floats2bfloat162_rn(o.z, o.w);
+                            uint2 pk;
+                            pk.x = *reinterpret_cast<uint32_t*>(&lo2);
+                            pk.y = *reinterpret_cast<uint32_t*>(&hi2);
+                            *reinterpret_cast<uint2*>(Cb + gm * ldc + col0 + cq) = pk;
                         } else {
-                            const float ov[4] = {o.x, o.y, o.z, o.w};
-#pragma unroll
-                            for (int k = 0; k < 4; ++k)
-                                if (col0 + cq + k < n_valid) Cf[gm * ldc + col0 + cq + k] = ov[k];
+                            *reinterpret_cast<float4*>(Cf + gm * ldc + col0 + cq) = o;
                         }
                     }
                 }

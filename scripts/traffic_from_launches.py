@@ -7,7 +7,7 @@ STAGES = [   # (stage, regex over kernel names); first match wins
     ("project_fwd", r"in_wproj_image_kernel|in_proj_gemm<\(bool\)1>|in_proj_gemm<true>|in_proj_gemm<1>|build_b_images|gemm_tc_ws2|gemm_simt|wabsmax|in_w_absmax"),
     ("gat_fwd", r"gat_fwd_"),
     ("gat_bwd_dst_src", r"gat_bwd_dst|gat_bwd_src|gat_hub_chunk_sum"),
-    ("project_bwd", r"dw_tc|dax_partial|colsum_partial|reduce_slices|datt_from_g|dw_reduce|gemm_tc_ws<|transpose"),
+    ("project_bwd", r"dw_tc|dax_partial|colsum_partial|reduce_slices|datt_from_g|dw_reduce|gemm_tc_ws\b|transpose"),
     ("in_logits", r"in_u_kernel|in_logits_kernel|in_scales_kernel|in_wout_image|in_wgd_image"),
     ("in_fwd_edges", r"in_alpha_|gat_in_fwd_"),
     ("in_out_gemm", r"in_out_gemm"),
