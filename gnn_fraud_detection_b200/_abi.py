@@ -18,7 +18,7 @@ F32, BF16 = 0, 1
 ACT_NONE, ACT_RELU, ACT_ELU = 0, 1, 2
 GEMM_AUTO, GEMM_SIMT, GEMM_TC, GEMM_INPUT = 0, 1, 2, 3
 HUB_THRESHOLD, HUB_CHUNK = 512, 512
-ABI_VERSION = 20
+ABI_VERSION = 21
 
 _i32p = C.POINTER(C.c_int32)
 
@@ -87,7 +87,9 @@ SIGNATURES = {
     "gnnfd_project_bwd_workspace_bytes": (_i, [_i64, _i64, _i, _i, _i, _szp]),
     "gnnfd_project_bwd": (_i, [_vp, _i64, _vp, _vp, _vp, _i, _vp, _vp, _vp, _i64, _i64, _i, _i, _i, _i, _vp, _vp,
                                _vp, _vp, _vp, _i64, _vp, _sz, _vp]),
-    # input-space formulation of the first layer
+    "gnnfd_project_dx_workspace_bytes": (_i, [_i64, _i64, _i, _i, _szp]),
+    "gnnfd_project_dx": (_i, [_vp, _vp, _i64, _i64, _i, _i, _vp, _i64, _vp, _sz, _vp]),
+    # input-space formulation
     "gnnfd_in_supported": (_i, [_i64, _i, _i, _i]),
     "gnnfd_in_sizes": (_i, [_i64, _i64, _szp, _szp, _i64p, _i64p]),
     "gnnfd_in_pad_x": (_i, [_vp, _i64, _i64, _i64, _vp, _vp]),
@@ -103,7 +105,7 @@ SIGNATURES = {
     "gnnfd_in_bwd_gd": (_i, [_vp, _i64, _i64, _vp, _vp, _vp, _sz, _vp]),
     "gnnfd_in_bwd_edges_workspace_bytes": (_i, [_gp, _szp]),
     "gnnfd_in_bwd_edges": (_i, [_gp, _vp, _i64, _i64, _vp, _vp, _vp, _i64, _i64, _i64, _i64, _i64, _f, _vp, _f,
-                                _u64, _vp, _vp, _vp, _sz, _i, _vp]),
+                                _u64, _vp, _vp, _vp, _vp, _sz, _i, _vp]),
     "gnnfd_in_bwd_dasrc": (_i, [_gp, _vp, _vp, _vp]),
     "gnnfd_in_bwd_params_workspace_bytes": (_i, [_i64, _i64, _szp]),
     "gnnfd_in_bwd_params": (_i, [_vp, _vp, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz,

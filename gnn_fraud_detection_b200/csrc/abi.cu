@@ -10,6 +10,8 @@ int project_bwd_simt(const float* x, int64_t ldx, const float* W, const float* d
                      const float* da_src, const float* da_dst, const float* d_out, int64_t N, int64_t K, int H,
                      int C, int Co, float* dW, float* datt_src, float* datt_dst, float* dbias, float* dx,
                      int64_t lddx, void* ws, size_t ws_bytes, cudaStream_t st, bool skip_dw, bool skip_dx);
+void project_dx_simt(const float* dxw, const float* W, int64_t N, int64_t K, int D, int H, float* dx, int64_t lddx,
+                     cudaStream_t st);
 // tensor-core path (project_tc.cu)
 bool tc_supported(int64_t N, int64_t K, int H, int C);
 size_t tc_ws_bytes(int64_t N, int64_t K, int H, int C);
@@ -18,6 +20,7 @@ int project_fwd_tc(const float* x, int64_t ldx, const float* W, const float* att
                    size_t ws_bytes, cudaStream_t st);
 int project_bwd_dx_tc(const float* dxw, const float* W, int64_t N, int64_t K, int D, float* dx, int64_t lddx, void* ws,
                       size_t ws_bytes, cudaStream_t st);
+size_t dx_tc_ws_bytes(int64_t K, int D);
 int project_bwd_dw_tc(const float* dxw, const float* x, int64_t ldx, int64_t N, int64_t K, int D, float* dW, void* ws,
                       size_t ws_bytes, cudaStream_t st);
 bool dw_tc_supported(int64_t K, int D);
@@ -102,6 +105,31 @@ int gnnfd_project_bwd(const float* x, int64_t ldx, const float* W, const float* 
     }
     if (dx) rc = project_bwd_dx_tc(dxw, W, N, K, H * C, dx, lddx, tws, tws_bytes, st);
     return rc;
+}
+
+int gnnfd_project_dx_workspace_bytes(int64_t N, int64_t K, int H, int C, size_t* bytes)
+{
+    GNNFD_REQUIRE(bytes, GNNFD_ERR_ARG, "project_dx_workspace_bytes: bytes is NULL");
+    GNNFD_REQUIRE(N >= 0 && K > 0 && H > 0 && C > 0, GNNFD_ERR_ARG, "project_dx_workspace_bytes: bad shape");
+    *bytes = dx_tc_ws_bytes(K, H * C) + 256;
+    return GNNFD_OK;
+}
+
+int gnnfd_project_dx(const float* dxw, const float* W, int64_t N, int64_t K, int H, int C, float* dx, int64_t lddx, void* ws,
+                     size_t ws_bytes, gnnfd_stream_t stream)
+{
+    GNNFD_REQUIRE(N >= 0 && K > 0 && H > 0 && C > 0 && lddx >= K, GNNFD_ERR_ARG, "project_dx: bad shape");
+    GNNFD_REQUIRE(N == 0 || (dxw && W && dx), GNNFD_ERR_ARG, "project_dx: NULL tensor");
+    size_t need = 0;
+    gnnfd_project_dx_workspace_bytes(N, K, H, C, &need);
+    GNNFD_REQUIRE(ws && ws_bytes >= need, GNNFD_ERR_WORKSPACE, "project_dx: workspace %zu < %zu", ws_bytes, need);
+    if (N == 0) return GNNFD_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (pick_algo(GNNFD_GEMM_AUTO, N, K, H, C) == GNNFD_GEMM_TC)
+        return project_bwd_dx_tc(dxw, W, N, K, H * C, dx, lddx, ws, ws_bytes, st);
+    project_dx_simt(dxw, W, N, K, H * C, H, dx, lddx, st);
+    GNNFD_LAUNCH_CHECK();
+    return GNNFD_OK;
 }
 
 }  // extern "C"

@@ -49,18 +49,6 @@ __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc)
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(st_smem_u32(smem_dst)), "l"(gsrc) : "memory");
 }
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-// H floats to a 32-byte-aligned address: one 256-bit store for H = 8 (a whole sector per lane), else store_vecH
-template <int H>
-__device__ __forceinline__ void store_vecH_wide(float* __restrict__ p, const float (&v)[H])
-{
-    if constexpr (H == 8) {
-        asm volatile("st.global.v8.f32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(p), "f"(v[0]), "f"(v[1]),
-                     "f"(v[2]), "f"(v[3]), "f"(v[4]), "f"(v[5]), "f"(v[6]), "f"(v[7])
-                     : "memory");
-    } else {
-        store_vecH<H>(p, v);
-    }
-}
 // wait until at most n of this thread's commit groups are pending (n < DA_TASKS)
 __device__ __forceinline__ void cp_async_wait_pending(int n)
 {

@@ -50,6 +50,18 @@ __device__ __forceinline__ void store_vecH(float* __restrict__ p, const float (&
     for (int k = 0; k < H / 4; ++k)
         reinterpret_cast<float4*>(p)[k] = make_float4(v[4 * k], v[4 * k + 1], v[4 * k + 2], v[4 * k + 3]);
 }
+// H floats to a 32-byte-aligned address: one 256-bit store for H = 8 (a whole sector per lane), else store_vecH
+template <int H>
+__device__ __forceinline__ void store_vecH_wide(float* __restrict__ p, const float (&v)[H])
+{
+    if constexpr (H == 8) {
+        asm volatile("st.global.v8.f32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(p), "f"(v[0]), "f"(v[1]),
+                     "f"(v[2]), "f"(v[3]), "f"(v[4]), "f"(v[5]), "f"(v[6]), "f"(v[7])
+                     : "memory");
+    } else {
+        store_vecH<H>(p, v);
+    }
+}
 
 // one slot (VW elements) of a feature row, streamed past L1
 __device__ __forceinline__ void load_slot(const float* __restrict__ row, int q, int lane, float (&v)[4])

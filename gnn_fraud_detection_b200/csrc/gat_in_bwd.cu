@@ -1,9 +1,12 @@
-// Input-space backward of the first GAT layer, edge pass (see in_common.cuh for the algebra): the autograd mirror of
+// Input-space backward of the GAT layer, edge pass (see in_common.cuh for the algebra): the autograd mirror of
 // edge_update / softmax / aggregate (loss.backward() at src/train.py:142) without projected features:
 //     d_alpha[e,h] = Gd[i,h,:] . x[j,:]          Gd = dO W_r^T / H from gnnfd_in_bwd_gd (one 4*F-byte row per destination)
 //     u = alpha * d_alpha (dropout-scaled), t = sum_row u, dz = slope' * (u - alpha t), da_dst[i] = sum_row dz
 // dz is written in SOURCE-MAJOR order (slot csr2csc[e]) so that da_src = per-source sums (gnnfd_in_bwd_dasrc) reads it
-// contiguously.  No alpha_used / dxw: the weight gradient comes from the saved Z image (in_gemm.cu).
+// contiguously.  The weight gradient comes from the saved Z image (in_gemm.cu), so a first layer needs no alpha_used.
+// A hidden layer needs dx = dxw W, and dxw is what gnnfd_gat_bwd_src computes from (alpha_used, dz) slot records: the REC
+// variant (KP = 64) stores alpha_used = alpha * keep / (1-p) beside dz, as the 64-byte record [alpha_used | dz] at slot
+// csr2csc[e] that gnnfd_gat_bwd_dst writes (two 256-bit stores), and nothing else changes.
 // alpha (with the LeakyReLU region in its sign bit) and the row-end flags are what the forward's attention pass saved: the
 // staging of a chunk (lane = edge) is two coalesced loads, no logit gathers, no exp, no row statistics.
 // Same warp-stream structure as gat_bwd_dst.cu (work items, staging one chunk ahead, packs of short rows, hub rows in
@@ -70,7 +73,9 @@ __device__ __forceinline__ void stage_bwd_chunk(const BwdChunk& c, bool pack, co
     __syncwarp();
 }
 
-// second sweep of a long row: dz = slope' * (u - alpha * t); lane-local partial of da_dst
+// second sweep of a long row: dz = slope' * (u - alpha * t); lane-local partial of da_dst.  LD: floats per dz slot (H, or 2H
+// for records, whose alpha_used half phase C has already written)
+template <int LD>
 __device__ __forceinline__ void in_sweep2(int beg, int end, const int32_t* __restrict__ csr2csc, const float* __restrict__ alpha,
                                           float slope, const float (&t)[H], int lane, float* __restrict__ dz, float (&dad)[H])
 {
@@ -78,15 +83,26 @@ __device__ __forceinline__ void in_sweep2(int beg, int end, const int32_t* __res
         float a[H], u[H], o[H];
         const int64_t pos = csr2csc[e];          // edge gradients live in source-major order
         load_vecH<H>(alpha + int64_t(e) * H, a);
-        load_vecH<H>(dz + pos * H, u);
+        load_vecH<H>(dz + pos * LD, u);
 #pragma unroll
         for (int h = 0; h < H; ++h) {
             const float sl = (__float_as_uint(a[h]) >> 31) ? slope : 1.f;
             o[h] = sl * (u[h] - fabsf(a[h]) * t[h]);
             dad[h] += o[h];
         }
-        store_vecH<H>(dz + pos * H, o);
+        store_vecH<H>(dz + pos * LD, o);
     }
+}
+
+// phase C's store of one edge in record mode: the record [alpha_used | dz] at source-major slot pos, dz == record + H
+__device__ __forceinline__ void store_record(float* __restrict__ dz, int64_t pos, const float (&alpha)[H], int bits,
+                                             float keep_scale, const float (&o)[H])
+{
+    float au[H];
+#pragma unroll
+    for (int hh = 0; hh < H; ++hh) au[hh] = (bits >> (8 + hh)) & 1 ? alpha[hh] * keep_scale : 0.f;
+    store_vecH_wide<H>(dz + pos * 2 * H - H, au);
+    store_vecH_wide<H>(dz + pos * 2 * H, o);
 }
 
 // per-warp scratch beyond the ring: dal_s [32][H] floats, bits_s [2][32] ints, the Gd row buffer [F] floats
@@ -146,8 +162,8 @@ struct GdBuf {
 };
 
 // HUB = false: whole rows and packs of short rows, results go to da_dst.  HUB = true: one (row, range) segment, the
-// partial t of the segment goes to part_t[chunk_id]; the second sweep is a separate kernel.
-template <int N4, bool DROPOUT, bool HUB>
+// partial t of the segment goes to part_t[chunk_id]; the second sweep is a separate kernel.  REC: dz slots are records.
+template <int N4, bool DROPOUT, bool HUB, bool REC>
 __device__ __forceinline__ void in_bwd_stream(ChunkCursor& cur, BwdRing& ring, GdBuf<N4>& gdb, const int32_t* __restrict__ rowptr,
                                               const int32_t* __restrict__ perm, const int32_t* __restrict__ csr2csc,
                                               const float* __restrict__ alpha_g, const int32_t* __restrict__ jflag, float slope,
@@ -280,7 +296,10 @@ __device__ __forceinline__ void in_bwd_stream(ChunkCursor& cur, BwdRing& ring, G
                     o[hh] = live ? sl * (u[hh] - alpha[hh] * tt) : 0.f;
                     dad[hh] = seg_total(o[hh], sa, sb, lane);
                 }
-                if (live) store_vecH<H>(dz + pos * H, o);
+                if (live) {
+                    if constexpr (REC) store_record(dz, pos, alpha, bits, keep_scale, o);
+                    else store_vecH<H>(dz + pos * H, o);
+                }
                 const unsigned lastm = __ballot_sync(FULL, lastf);
                 if (lastf) {
                     const int64_t r = c0.row + __popc(lastm & ((1u << lane) - 1u));
@@ -295,10 +314,16 @@ __device__ __forceinline__ void in_bwd_stream(ChunkCursor& cur, BwdRing& ring, G
                     o[hh] = live ? sl * (u[hh] - alpha[hh] * tt) : 0.f;
                     dad[hh] = warp_sum(o[hh]);
                 }
-                if (live) store_vecH<H>(dz + pos * H, o);
+                if (live) {
+                    if constexpr (REC) store_record(dz, pos, alpha, bits, keep_scale, o);
+                    else store_vecH<H>(dz + pos * H, o);
+                }
                 if (lane == 0) store_vecH<H>(da_dst + int64_t(c0.row) * H, dad);
             } else {
-                if (live) store_vecH<H>(dz + pos * H, u);       // parked until t is known
+                if (live) {                                     // parked until t is known
+                    if constexpr (REC) store_record(dz, pos, alpha, bits, keep_scale, u);
+                    else store_vecH<H>(dz + pos * H, u);
+                }
 #pragma unroll
                 for (int hh = 0; hh < H; ++hh) trow[hh] += warp_sum(u[hh]);
                 if (c0.last) {
@@ -309,7 +334,7 @@ __device__ __forceinline__ void in_bwd_stream(ChunkCursor& cur, BwdRing& ring, G
                         float dad[H];
 #pragma unroll
                         for (int hh = 0; hh < H; ++hh) dad[hh] = 0.f;
-                        in_sweep2(row_beg, c0.beg + c0.n, csr2csc, alpha_g, slope, trow, lane, dz, dad);
+                        in_sweep2<REC ? 2 * H : H>(row_beg, c0.beg + c0.n, csr2csc, alpha_g, slope, trow, lane, dz, dad);
 #pragma unroll
                         for (int hh = 0; hh < H; ++hh) dad[hh] = warp_sum(dad[hh]);
                         if (lane == 0) store_vecH<H>(da_dst + int64_t(c0.row) * H, dad);
@@ -343,7 +368,7 @@ __device__ __forceinline__ void gdbuf_init(GdBuf<N4>& gdb, BwdRing& ring, const 
 
 constexpr int IN_BWD_CTAS = 4;
 
-template <int N4, bool DROPOUT>
+template <int N4, bool DROPOUT, bool REC>
 __global__ void __launch_bounds__(IN_THREADS, IN_BWD_CTAS)
 gat_in_bwd_items(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ perm, const int32_t* __restrict__ csr2csc,
                  const float* __restrict__ x, int64_t ldx, int KP, const float* __restrict__ alpha,
@@ -362,12 +387,12 @@ gat_in_bwd_items(const int32_t* __restrict__ rowptr, const int32_t* __restrict__
     gdbuf_init(gdb, ring, gd, F, KP);
     ChunkCursor cur;
     cur.start_rows(items.item_start[item], items.item_start[item + 1], hub_threshold);
-    in_bwd_stream<N4, DROPOUT, false>(cur, ring, gdb, rowptr, perm, csr2csc, alpha, jflag, slope, keep, keep_scale, dz, da_dst,
-                                      nullptr, 0, lane);
+    in_bwd_stream<N4, DROPOUT, false, REC>(cur, ring, gdb, rowptr, perm, csr2csc, alpha, jflag, slope, keep, keep_scale, dz,
+                                           da_dst, nullptr, 0, lane);
 }
 
 // hub rows, step 1: one warp per chunk -- first sweep, partial t (rows outside [row_lo, row_hi) belong to another block)
-template <int N4, bool DROPOUT>
+template <int N4, bool DROPOUT, bool REC>
 __global__ void __launch_bounds__(IN_THREADS, IN_BWD_CTAS)
 gat_in_bwd_hub1(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ perm, const int32_t* __restrict__ csr2csc,
                 const float* __restrict__ x, int64_t ldx, int KP, const float* __restrict__ alpha,
@@ -390,11 +415,12 @@ gat_in_bwd_hub1(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ 
     gdbuf_init(gdb, ring, gd, F, KP);
     ChunkCursor cur;
     cur.start_segment(i, beg, end);
-    in_bwd_stream<N4, DROPOUT, true>(cur, ring, gdb, rowptr, perm, csr2csc, alpha, jflag, slope, keep, keep_scale, dz, nullptr,
-                                     part_t, c, lane);
+    in_bwd_stream<N4, DROPOUT, true, REC>(cur, ring, gdb, rowptr, perm, csr2csc, alpha, jflag, slope, keep, keep_scale, dz,
+                                          nullptr, part_t, c, lane);
 }
 
 // hub rows, step 2: second sweep of every chunk with the row's total t, partial da_dst
+template <int LD>
 __global__ void __launch_bounds__(ROW_THREADS)
 gat_in_bwd_hub2(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ csr2csc, const float* __restrict__ alpha,
                 gnnfd_hub_plan_t plan, float slope, const float* __restrict__ t_total, float* __restrict__ dz,
@@ -411,7 +437,7 @@ gat_in_bwd_hub2(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ 
     load_vecH<H>(t_total + int64_t(slot) * H, t);      // the same total in every chunk of the row
 #pragma unroll
     for (int h = 0; h < H; ++h) dad[h] = 0.f;
-    in_sweep2(beg, end, csr2csc, alpha, slope, t, lane, dz, dad);
+    in_sweep2<LD>(beg, end, csr2csc, alpha, slope, t, lane, dz, dad);
 #pragma unroll
     for (int h = 0; h < H; ++h) dad[h] = warp_sum(dad[h]);
     if (lane == 0) store_vecH<H>(part_dad + int64_t(c) * H, dad);
@@ -442,12 +468,14 @@ int gnnfd_in_bwd_edges_workspace_bytes(const gnnfd_graph_t* g, size_t* bytes)
 /* dz [E',H] (source-major order) and da_dst [n_dst,H] for the destination rows of the work items [item_lo, item_hi)
  * (= rows [row_lo, row_hi), which must be the rows those items cover; pass 0, n_items, 0, n_dst for everything).
  * gd holds the Gd rows of [gd_row0, ...) with leading dimension F.  phase bit 0: process the row block (items + first
- * hub sweep); bit 1: finish the hub rows (second sweep; after the LAST block, with the same ws). */
+ * hub sweep); bit 1: finish the hub rows (second sweep; after the LAST block, with the same ws).
+ * alpha_used != NULL (padded K = 64 only): also alpha_used, as the interleaved [E',2H] records of gnnfd_gat_bwd_dst
+ * (dz == alpha_used + H, 32-byte aligned). */
 int gnnfd_in_bwd_edges(const gnnfd_graph_t* g, const float* x, int64_t ldx, int64_t K, const float* alpha,
                        const int32_t* jflag, const float* gd, int64_t gd_row0,
                        int64_t item_lo, int64_t item_hi, int64_t row_lo, int64_t row_hi, float negative_slope,
-                       const uint8_t* keep_mask, float p_drop, uint64_t dropout_seed, float* dz, float* da_dst, void* ws, size_t ws_bytes,
-                       int phase, gnnfd_stream_t stream)
+                       const uint8_t* keep_mask, float p_drop, uint64_t dropout_seed, float* alpha_used, float* dz, float* da_dst,
+                       void* ws, size_t ws_bytes, int phase, gnnfd_stream_t stream)
 {
     int rc = check_graph(g, true, "in_bwd_edges");
     if (rc) return rc;
@@ -464,6 +492,11 @@ int gnnfd_in_bwd_edges(const gnnfd_graph_t* g, const float* x, int64_t ldx, int6
     GNNFD_REQUIRE((reinterpret_cast<uintptr_t>(gd) & 15) == 0, GNNFD_ERR_ARG, "in_bwd_edges: gd must be 16-byte aligned");
     cudaStream_t st = (cudaStream_t)stream;
     const Dims d((int)K);
+    const bool rec = alpha_used != nullptr;
+    GNNFD_REQUIRE(!rec || d.KP == 64, GNNFD_ERR_UNSUPPORTED,
+                  "in_bwd_edges: alpha_used records are built for K <= 64 padded to 64 only (K = %lld)", (long long)K);
+    GNNFD_REQUIRE(!rec || g->n_edges == 0 || (dz == alpha_used + H && (reinterpret_cast<uintptr_t>(alpha_used) & 31) == 0),
+                  GNNFD_ERR_ARG, "in_bwd_edges: alpha_used / dz must be the halves of one 32-byte aligned [E',2H] buffer");
     const bool drop = p_drop > 0.f;              // explicit mask, or (mask == NULL) the counter-based RNG keyed on seed
     float ks = 1.f;
     const KeepMask keep = make_keep(keep_mask, p_drop, dropout_seed, &ks);
@@ -486,27 +519,28 @@ int gnnfd_in_bwd_edges(const gnnfd_graph_t* g, const float* x, int64_t ldx, int6
     if ((phase & 1) && item_hi > item_lo) {
         const unsigned grid = (unsigned)((item_hi - item_lo + IN_WARPS - 1) / IN_WARPS);
         const unsigned gc = (unsigned)((pl.n_chunk + IN_WARPS - 1) / IN_WARPS);
-#define GNNFD_IN_BWD(NN, DD)                                                                                           \
-    rc = in_set_smem_bwd(gat_in_bwd_items<NN, DD>, smem);                                                              \
+#define GNNFD_IN_BWD(NN, DD, RR)                                                                                       \
+    rc = in_set_smem_bwd(gat_in_bwd_items<NN, DD, RR>, smem);                                                          \
     if (rc) return rc;                                                                                                 \
-    gat_in_bwd_items<NN, DD><<<grid, IN_THREADS, smem, st>>>(g->rowptr, g->perm, g->csr2csc, x, ldx, d.KP, alpha, jflag, gd0,     \
-                                                             g->items_dst, (int)item_lo, (int)item_hi, thr, negative_slope,      \
-                                                             keep, ks, dz, da_dst)
-#define GNNFD_IN_HUB1(NN, DD)                                                                                          \
-    rc = in_set_smem_bwd(gat_in_bwd_hub1<NN, DD>, smem);                                                               \
+    gat_in_bwd_items<NN, DD, RR><<<grid, IN_THREADS, smem, st>>>(g->rowptr, g->perm, g->csr2csc, x, ldx, d.KP, alpha, jflag, gd0, \
+                                                                 g->items_dst, (int)item_lo, (int)item_hi, thr, negative_slope,  \
+                                                                 keep, ks, dz, da_dst)
+#define GNNFD_IN_HUB1(NN, DD, RR)                                                                                      \
+    rc = in_set_smem_bwd(gat_in_bwd_hub1<NN, DD, RR>, smem);                                                           \
     if (rc) return rc;                                                                                                 \
-    gat_in_bwd_hub1<NN, DD><<<gc, IN_THREADS, smem, st>>>(g->rowptr, g->perm, g->csr2csc, x, ldx, d.KP, alpha, jflag, gd0, pl,   \
-                                                          (int)row_lo, (int)row_hi, negative_slope, keep, ks, dz, part_t)
-#define GNNFD_IN_BWD_ALL(NN)                                                                                           \
-    if (drop) { GNNFD_IN_BWD(NN, true); } else { GNNFD_IN_BWD(NN, false); }                                            \
+    gat_in_bwd_hub1<NN, DD, RR><<<gc, IN_THREADS, smem, st>>>(g->rowptr, g->perm, g->csr2csc, x, ldx, d.KP, alpha, jflag, gd0, pl, \
+                                                              (int)row_lo, (int)row_hi, negative_slope, keep, ks, dz, part_t)
+#define GNNFD_IN_BWD_ALL(NN, RR)                                                                                       \
+    if (drop) { GNNFD_IN_BWD(NN, true, RR); } else { GNNFD_IN_BWD(NN, false, RR); }                                    \
     g_launches += 1;                                                                                                   \
     if (pl.n_hub > 0) {                                                                                                \
-        if (drop) { GNNFD_IN_HUB1(NN, true); } else { GNNFD_IN_HUB1(NN, false); }                                      \
+        if (drop) { GNNFD_IN_HUB1(NN, true, RR); } else { GNNFD_IN_HUB1(NN, false, RR); }                              \
         g_launches += 1;                                                                                               \
     }
-        if (d.KP == 168) { GNNFD_IN_BWD_ALL(42) }
-        else if (d.KP == 64) { GNNFD_IN_BWD_ALL(16) }
-        else { GNNFD_IN_BWD_ALL(0) }
+        if (d.KP == 168) { GNNFD_IN_BWD_ALL(42, false) }
+        else if (d.KP == 64 && rec) { GNNFD_IN_BWD_ALL(16, true) }
+        else if (d.KP == 64) { GNNFD_IN_BWD_ALL(16, false) }
+        else { GNNFD_IN_BWD_ALL(0, false) }
 #undef GNNFD_IN_BWD_ALL
 #undef GNNFD_IN_HUB1
 #undef GNNFD_IN_BWD
@@ -515,7 +549,11 @@ int gnnfd_in_bwd_edges(const gnnfd_graph_t* g, const float* x, int64_t ldx, int6
         const unsigned gh = (unsigned)((pl.n_hub + ROW_WARPS - 1) / ROW_WARPS);
         const unsigned gc2 = (unsigned)((pl.n_chunk + ROW_WARPS - 1) / ROW_WARPS);
         gat_hub_chunk_sum<H, false><<<gh, ROW_THREADS, 0, st>>>(pl, part_t, t_total);
-        gat_in_bwd_hub2<<<gc2, ROW_THREADS, 0, st>>>(g->rowptr, g->csr2csc, alpha, pl, negative_slope, t_total, dz, part_dad);
+        if (rec)
+            gat_in_bwd_hub2<2 * H><<<gc2, ROW_THREADS, 0, st>>>(g->rowptr, g->csr2csc, alpha, pl, negative_slope, t_total, dz,
+                                                                part_dad);
+        else
+            gat_in_bwd_hub2<H><<<gc2, ROW_THREADS, 0, st>>>(g->rowptr, g->csr2csc, alpha, pl, negative_slope, t_total, dz, part_dad);
         gat_hub_chunk_sum<H, true><<<gh, ROW_THREADS, 0, st>>>(pl, part_dad, da_dst);
         g_launches += 3;
     }

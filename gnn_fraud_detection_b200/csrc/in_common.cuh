@@ -1,4 +1,4 @@
-// Input-space formulation of the GAT layer (first layer: no gradient w.r.t. x, concat = False, H = 8, C = 64).
+// Input-space formulation of the GAT layer (concat = False, H = 8, C = 64; gradient w.r.t. x at K = 64 only).
 //
 // PyG's GATConv projects first (xw = x W^T, [N, H*C]) and aggregates 2 KB projected rows per edge.  When the input
 // width K is smaller than H*C (166 vs 512 for the reference's first layer, src/models/gat.py:39) the same layer is

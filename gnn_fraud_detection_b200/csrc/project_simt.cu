@@ -428,6 +428,16 @@ size_t project_bwd_ws_bytes(int64_t N, int64_t K, int H, int C)
            carve_bytes(size_t(col_slices(N)) * D, 4);
 }
 
+// dx[N,K] = dxw[N,D] @ W[D,K]
+void project_dx_simt(const float* dxw, const float* W, int64_t N, int64_t K, int D, int H, float* dx, int64_t lddx,
+                     cudaStream_t st)
+{
+    dim3 grid((unsigned)((N + GB_M - 1) / GB_M), (unsigned)((K + GB_N - 1) / GB_N));
+    gemm_simt<false, 0, false><<<grid, 256, 0, st>>>(dxw, D, W, K, 1, N, (int)K, D, dx, nullptr, lddx, nullptr,
+                                                     nullptr, nullptr, nullptr, H);
+    g_launches += 1;
+}
+
 int project_bwd_simt(const float* x, int64_t ldx, const float* W, const float* dxw, const void* xw, int xw_dtype,
                      const float* da_src, const float* da_dst, const float* d_out, int64_t N, int64_t K, int H,
                      int C, int Co, float* dW, float* datt_src, float* datt_dst, float* dbias, float* dx,
@@ -491,12 +501,7 @@ int project_bwd_simt(const float* x, int64_t ldx, const float* W, const float* d
         reduce_slices<<<(unsigned)((Co + 63) / 64), 64, 0, st>>>(Pc, Co, Sg, dbias);
         g_launches += 2;
     }
-    if (dx && !skip_dx) {
-        dim3 grid((unsigned)((N + GB_M - 1) / GB_M), (unsigned)((K + GB_N - 1) / GB_N));
-        gemm_simt<false, 0, false><<<grid, 256, 0, st>>>(dxw, D, W, K, 1, N, (int)K, D, dx, nullptr, lddx, nullptr,
-                                                         nullptr, nullptr, nullptr, H);
-        g_launches += 1;
-    }
+    if (dx && !skip_dx) project_dx_simt(dxw, W, N, K, D, H, dx, lddx, st);
     GNNFD_LAUNCH_CHECK();
     return GNNFD_OK;
 }

@@ -265,13 +265,18 @@ int project_fwd_tc(const float* x, int64_t ldx, const float* W, const float* att
 }
 
 // dx[N,K] = dxw[N,D] @ W[D,K]:  A = dxw (K-major in D), B rows = k (W^T), reduction over D
+constexpr int DX_BN = 256;   // TODO(perf): a BN=64/128 instantiation for the K=64 hidden layers
+size_t dx_tc_ws_bytes(int64_t K, int D)
+{
+    return size_t((K + DX_BN - 1) / DX_BN) * tc::kblocks(D) * 2 * (DX_BN * tc::BK) * sizeof(float) + 2048;
+}
 int project_bwd_dx_tc(const float* dxw, const float* W, int64_t N, int64_t K, int D, float* dx, int64_t lddx, void* ws,
                       size_t ws_bytes, cudaStream_t st)
 {
     if (N == 0) return GNNFD_OK;
-    constexpr int BN = 256;   // TODO(perf): a BN=64/128 instantiation for the K=64 hidden layers
+    constexpr int BN = DX_BN;
     const int n_kb = tc::kblocks(D), n_tiles = int((K + BN - 1) / BN);
-    const size_t need = size_t(n_tiles) * n_kb * 2 * (BN * tc::BK) * sizeof(float) + 2048;
+    const size_t need = dx_tc_ws_bytes(K, D);
     GNNFD_REQUIRE(ws && ws_bytes >= need, GNNFD_ERR_WORKSPACE, "project_bwd_dx_tc: workspace %zu < %zu", ws_bytes, need);
     float* img = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(ws) + 1023) & ~uintptr_t(1023));
     // B row r = input feature k, reduction index = output column o: element = W[o*K + k]

@@ -248,8 +248,21 @@ def project_bwd(x, W, dxw, xw, da_src, da_dst, d_out, H, C_, Co, need_dx, algo=_
     return dW, datt_src, datt_dst, dbias, dx
 
 
+def project_dx(dxw, W, H, C_):
+    """dx [N,K] = dxw [N,H*C] W: the dx GEMM of ``project_bwd`` alone (for a layer that has no xw)."""
+    L = _abi.lib()
+    N, K = dxw.size(0), W.size(1)
+    dx = torch.empty(N, K, dtype=torch.float32, device=dxw.device)
+    nb = C.c_size_t()
+    _abi.check(L.gnnfd_project_dx_workspace_bytes(N, K, H, C_, C.byref(nb)))
+    ws = _ws(nb.value, dxw.device)
+    _abi.check(L.gnnfd_project_dx(dxw.data_ptr(), W.data_ptr(), N, K, H, C_, dx.data_ptr(), K, ws.data_ptr(), ws.numel(),
+                                  _stream()))
+    return dx
+
+
 # ------------------------------------------------------------------------------------------------
-# input-space formulation of the first layer (include/gnnfd_b200.h section (5), csrc/in_common.cuh)
+# input-space formulation (include/gnnfd_b200.h section (5), csrc/in_common.cuh)
 # ------------------------------------------------------------------------------------------------
 def in_supported(K: int, H: int, C_: int, concat: bool) -> bool:
     return bool(_abi.lib().gnnfd_in_supported(int(K), int(H), int(C_), int(bool(concat))))
@@ -363,12 +376,19 @@ IN_GD_BLOCK_BYTES = 8 << 30     # upper bound of the Gd buffer of the backward e
 
 
 def in_bwd_edges(g: GraphCSR, x, att: "InAttention", d_out, prep, negative_slope, keep_mask=None, p_drop=0.0,
-                 n_blocks=None, seed=0):
-    """Gd GEMM + backward edge pass, in blocks of destination rows.  Returns dz [E',H] (source-major) and da_dst."""
+                 n_blocks=None, seed=0, records=False):
+    """Gd GEMM + backward edge pass, in blocks of destination rows.  Returns dz [E',H] (source-major) and da_dst.
+
+    ``records=True`` (K = 64): returns alpha_used, dz, da_dst, where alpha_used and dz are the halves of one interleaved
+    [E',2H] buffer, the slot records ``gat_bwd_src`` reads (what ``gat_bwd_dst`` returns on the projected path)."""
     L = _abi.lib()
     dev, K = x.device, x.size(1)
     F = in_sizes(g.n_dst, K)[2]
-    dz = torch.empty(g.n_edges, 8, dtype=torch.float32, device=dev)
+    if records:
+        eg = torch.empty(g.n_edges, 16, dtype=torch.float32, device=dev)
+        alpha_used, dz = eg[:, :8], eg[:, 8:]
+    else:
+        alpha_used, dz = None, torch.empty(g.n_edges, 8, dtype=torch.float32, device=dev)
     da_dst = torch.empty(g.n_dst, 8, dtype=torch.float32, device=dev)
     nb = C.c_size_t()
     _abi.check(L.gnnfd_in_bwd_edges_workspace_bytes(g.ref(), C.byref(nb)))
@@ -388,9 +408,10 @@ def in_bwd_edges(g: GraphCSR, x, att: "InAttention", d_out, prep, negative_slope
         phase = 1 | (2 if bi == len(blocks) - 1 else 0)
         _abi.check(L.gnnfd_in_bwd_edges(g.ref(), x.data_ptr(), x.stride(0), K, att.alpha.data_ptr(), att.jflag.data_ptr(),
                                         gd.data_ptr(), r_lo, i_lo, i_hi, r_lo, r_hi,
-                                        float(negative_slope), _abi.ptr(keep_mask), float(p_drop), int(seed), dz.data_ptr(),
-                                        da_dst.data_ptr(), ws.data_ptr(), ws.numel(), phase, _stream()))
-    return dz, da_dst
+                                        float(negative_slope), _abi.ptr(keep_mask), float(p_drop), int(seed),
+                                        _abi.ptr(alpha_used), dz.data_ptr(), da_dst.data_ptr(), ws.data_ptr(), ws.numel(),
+                                        phase, _stream()))
+    return (alpha_used, dz, da_dst) if records else (dz, da_dst)
 
 
 def in_dasrc(g: GraphCSR, dz, out=None):
@@ -437,7 +458,8 @@ def in_bwd_params_split(zimg, d_out, x, W, att_src, att_dst, prep, _phase=1, _da
 
 
 class GATConvInputSpaceFunction(torch.autograd.Function):
-    """First-layer GATConv (x needs no gradient, concat=False, H=8, C=64) in the input-space formulation."""
+    """GATConv (concat=False, H=8, C=64) in the input-space formulation.  The gradient w.r.t. x (a hidden layer, K=64) goes
+    through the projected path's source-major pass and dx GEMM: dx = dxw W with dxw from the (alpha_used, dz) records."""
 
     @staticmethod
     def forward(ctx, x, W, att_src, att_dst, bias, g: GraphCSR, negative_slope, keep_mask, p_drop, want_stats, seed=0):
@@ -476,15 +498,21 @@ class GATConvInputSpaceFunction(torch.autograd.Function):
         g = ctx.g
         if not g.has_csc:
             raise RuntimeError("backward needs the CSC twin; build the graph with build_csc=True")
-        if ctx.needs_input_grad[0]:
-            raise RuntimeError("the input-space formulation computes no gradient w.r.t. x (first layer only)")
         d_out = d_out.contiguous().float()
+        dx = None
         with torch.cuda.device(x.device):
             att = InAttention(alpha, jflag, rowmax, rowsum)
-            dz, da_dst = in_bwd_edges(g, x, att, d_out, prep, ctx.slope, keep_mask, ctx.p, seed=ctx.seed)
-            da_src = in_dasrc(g, dz)
-            dW, datt_src, datt_dst, dbias = in_bwd_params(zimg, d_out, x, W, a_s, a_d, da_src, da_dst, prep)
-        return (None, dW, datt_src.view(ctx.att_shape), datt_dst.view(ctx.att_shape), dbias if ctx.has_bias else None,
+            if ctx.needs_input_grad[0]:
+                alpha_used, dz, da_dst = in_bwd_edges(g, x, att, d_out, prep, ctx.slope, keep_mask, ctx.p, seed=ctx.seed,
+                                                      records=True)
+                dxw, da_src = gat_bwd_src(g, alpha_used, dz, d_out, a_s, a_d, da_dst, 8, 64, False)
+                dW, datt_src, datt_dst, dbias = in_bwd_params(zimg, d_out, x, W, a_s, a_d, da_src, da_dst, prep)
+                dx = project_dx(dxw, W, 8, 64)
+            else:
+                dz, da_dst = in_bwd_edges(g, x, att, d_out, prep, ctx.slope, keep_mask, ctx.p, seed=ctx.seed)
+                da_src = in_dasrc(g, dz)
+                dW, datt_src, datt_dst, dbias = in_bwd_params(zimg, d_out, x, W, a_s, a_d, da_src, da_dst, prep)
+        return (dx, dW, datt_src.view(ctx.att_shape), datt_dst.view(ctx.att_shape), dbias if ctx.has_bias else None,
                 None, None, None, None, None, None)
 
 
@@ -548,9 +576,10 @@ def gatconv(x, W, att_src, att_dst, bias, g: GraphCSR, heads, out_channels, conc
     """``p_drop > 0`` with ``keep_mask=None`` selects the in-kernel counter-based dropout RNG keyed on ``seed``."""
     if algo == _abi.GEMM_INPUT:
         need_dx = x.requires_grad and torch.is_grad_enabled()
-        if need_dx or xw_dtype != torch.float32 or not in_supported(x.size(1), heads, out_channels, concat) or p_drop > 0.9:
-            raise _abi.GnnfdError(-5, "input-space formulation: needs x without gradient, concat=False, heads=8, "
-                                      "out_channels=64, in_channels <= 192, fp32 features, dropout <= 0.9")
+        if ((need_dx and x.size(1) != 64) or xw_dtype != torch.float32 or not in_supported(x.size(1), heads, out_channels, concat)
+                or p_drop > 0.9):
+            raise _abi.GnnfdError(-5, "input-space formulation: needs concat=False, heads=8, out_channels=64, "
+                                      "in_channels <= 192 (exactly 64 when x needs a gradient), fp32 features, dropout <= 0.9")
         return GATConvInputSpaceFunction.apply(x, W, att_src, att_dst, bias, g, negative_slope, keep_mask, p_drop,
                                                want_stats, seed)
     return GATConvFunction.apply(x, W, att_src, att_dst, bias, g, heads, out_channels, concat, negative_slope,

@@ -37,7 +37,7 @@
 extern "C" {
 #endif
 
-#define GNNFD_ABI_VERSION 20
+#define GNNFD_ABI_VERSION 21
 
 typedef void* gnnfd_stream_t; /* cudaStream_t */
 
@@ -252,12 +252,19 @@ int gnnfd_project_bwd(const float* x, int64_t ldx, const float* W, const float* 
                       int64_t N, int64_t K, int H, int C, int Co, int algo, float* dW, float* datt_src,
                       float* datt_dst, float* dbias, float* dx, int64_t lddx, void* ws, size_t ws_bytes,
                       gnnfd_stream_t stream);
+/* dx [N,K] (leading dimension lddx) = dxw [N,H*C] W alone: the dx GEMM of gnnfd_project_bwd (GNNFD_GEMM_AUTO's choice of
+ * kernel), for callers that have dxw but no xw -- the input-space formulation of a hidden layer (5). */
+int gnnfd_project_dx_workspace_bytes(int64_t N, int64_t K, int H, int C, size_t* bytes);
+int gnnfd_project_dx(const float* dxw, const float* W, int64_t N, int64_t K, int H, int C, float* dx, int64_t lddx,
+                     void* ws, size_t ws_bytes, gnnfd_stream_t stream);
 
-/* ---- (5) input-space formulation of the FIRST layer (no gradient w.r.t. x, concat = 0, H = 8, C = 64, K <= 192) -------
+/* ---- (5) input-space formulation (concat = 0, H = 8, C = 64, K <= 192; gradient w.r.t. x at K = 64 only) -----------------
  * Same reference stages as (2)-(4) (GATConv.forward / backward at src/models/gat.py:39,80, src/train.py:142) evaluated
  * without projected features:  Z[i,h,:] = sum_e alpha[e,h] x[j,:] ;  out = Z W_r / H + bias ;  logits from x . (W_h^T att);
  * backward d_alpha[e,h] = Gd[i,h,:] . x[j,:] with Gd = dO W_r^T / H, dW from the saved Z.  The per-edge gather is K*4
  * bytes instead of H*C*4, and across GPUs (destination ranges, x replicated) only [N,H] logits / logit gradients travel.
+ * A first layer needs no dx.  A hidden layer (K = 64) gets it as the projected path does: gnnfd_in_bwd_edges also writes the
+ * alpha_used / dz records, gnnfd_gat_bwd_src turns them into dxw and da_src, and gnnfd_project_dx computes dx = dxw W.
  * Z lives in HBM as the fp16-pair tensor-core image described in csrc/in_common.cuh (opaque to the caller).
  *   prep  : per-call constants + weight images, gnnfd_in_sizes().prep_bytes, 1024-byte aligned, built by
  *           gnnfd_in_logits (u) + gnnfd_in_prepare (scales, images); valid until W / att / max|x| change
@@ -300,12 +307,16 @@ int gnnfd_in_bwd_edges_workspace_bytes(const gnnfd_graph_t* g, size_t* bytes);
 /* dz [E',H] (source-major order, row csr2csc[e]) and da_dst [n_dst,H] for the destination rows covered by the work items
  * [item_lo, item_hi) = rows [row_lo, row_hi) (0, n_items, 0, n_dst for everything); gd holds the Gd rows from gd_row0 on.
  * phase bit 0: process the block; bit 1: finish the hub rows (after the last block, same ws).  Needs the CSC twin.
- * alpha / jflag: what gnnfd_in_fwd saved (the backward gathers no logits and recomputes no softmax). */
+ * alpha / jflag: what gnnfd_in_fwd saved (the backward gathers no logits and recomputes no softmax).
+ * alpha_used: NULL, or (K <= 64, padded to 64) the first half of ONE 32-byte aligned interleaved [E',2H] buffer with
+ * dz == alpha_used + H, which then receives the (alpha_used, dz) records gnnfd_gat_bwd_src reads, as gnnfd_gat_bwd_dst
+ * writes them; dz and da_dst are the same either way. */
 int gnnfd_in_bwd_edges(const gnnfd_graph_t* g, const float* x, int64_t ldx, int64_t K, const float* alpha,
                        const int32_t* jflag, const float* gd,
                        int64_t gd_row0, int64_t item_lo, int64_t item_hi, int64_t row_lo, int64_t row_hi,
                        float negative_slope, const uint8_t* keep_mask, float p_drop, uint64_t dropout_seed,
-                       float* dz, float* da_dst, void* ws, size_t ws_bytes, int phase, gnnfd_stream_t stream);
+                       float* alpha_used, float* dz, float* da_dst, void* ws, size_t ws_bytes, int phase,
+                       gnnfd_stream_t stream);
 /* da_src [n_src,H] = per-source sums of dz (over g's CSC). */
 int gnnfd_in_bwd_dasrc(const gnnfd_graph_t* g, const float* dz, float* da_src, gnnfd_stream_t stream);
 int gnnfd_in_bwd_params_workspace_bytes(int64_t n, int64_t K, size_t* bytes);
