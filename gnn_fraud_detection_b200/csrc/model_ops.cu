@@ -474,14 +474,19 @@ bce_partial_kernel(const float* __restrict__ logits, const int64_t* __restrict__
         float g = 0.f;
         if (yi != -1) {
             const float xv = logits[i], yf = float(yi);
-            // softplus(v) = max(v,0) + log1p(exp(-|v|))
-            const float l1p = log1pf(__expf(-fabsf(xv)));
+            // softplus(v) = max(v,0) + log1p(exp(-|v|)); the accurate expf: a well-classified node's loss IS the log1p term,
+            // and __expf's error grows with |v| (about 25 ulp at |v| = 20) and flushes results below 2^-126 to zero
+            const float l1p = log1pf(expf(-fabsf(xv)));
             const float sp_pos = fmaxf(xv, 0.f) + l1p, sp_neg = fmaxf(-xv, 0.f) + l1p;
             s[0] += double(pos_weight * yf * sp_neg + (1.f - yf) * sp_pos);
             s[1] += 1.0;
             const float sg = 1.f / (1.f + __expf(-xv));
             g = sg * (pos_weight * yf + 1.f - yf) - pos_weight * yf;
-            const bool pred = xv >= 0.f, pos = yi == 1;
+            // the reference's predicate is torch.sigmoid(logit) >= 0.5 in fp32, which torch on CUDA evaluates as
+            // 1 / (1 + expf(-x)) with IEEE add and divide: it holds for small negative logits too (down to -1.6525915e-7
+            // with CUDA's expf; CPU torch's differs, -1.7881391e-7), so `xv >= 0` would miscount those.  Same arithmetic,
+            // same answer, bit for bit.
+            const bool pred = __fdiv_rn(1.f, __fadd_rn(1.f, expf(-xv))) >= 0.5f, pos = yi == 1;
             s[2] += (pred && pos); s[3] += (pred && !pos); s[4] += (!pred && !pos); s[5] += (!pred && pos);
         }
         g_unnorm[i] = g;

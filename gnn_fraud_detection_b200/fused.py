@@ -53,6 +53,9 @@ class _BNReluDropRes(torch.autograd.Function):
                     cnt = torch.tensor([count], dtype=torch.float64, device=dev)
                     dist.all_reduce(cnt, group=group)
                     count = float(cnt.item())
+            if count == 1.0:
+                # as nn.BatchNorm1d: one row has no batch variance (the output would silently be relu(beta))
+                raise ValueError(f"Expected more than 1 value per channel when training, got input size {[1, Cc]}")
             mean = torch.empty(Cc, dtype=torch.float32, device=dev)
             invstd = torch.empty(Cc, dtype=torch.float32, device=dev)
             _abi.check(L.gnnfd_bn_finalize(sums.data_ptr(), count, Cc, float(eps), float(momentum), _abi.ptr(running_mean),

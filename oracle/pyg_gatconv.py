@@ -131,11 +131,14 @@ def temporal_subgraph_oracle(x, edge_index, time_steps, t):
 # ----------------------------------------------------------------------------------------------
 def gatconv_forward(x, edge_index, W, att_src, att_dst, bias, heads: int, out_channels: int,
                     concat: bool = False, negative_slope: float = 0.2, add_self_loops: bool = True,
-                    dropout_mask: Optional[torch.Tensor] = None, p: float = 0.0):
+                    dropout_mask: Optional[torch.Tensor] = None, p: float = 0.0,
+                    dropout_scale: Optional[float] = None):
     """One GATConv forward in PyG 2.0-2.4 semantics.  dtype-generic (fp32 / fp64).
 
     ``dropout_mask`` is an optional ``[E',H]`` keep-mask in ``edge_index'`` order, applied as
-    ``alpha * mask / (1-p)`` (``F.dropout`` semantics with an injected mask).
+    ``alpha * mask / (1-p)`` (``F.dropout`` semantics with an injected mask).  ``dropout_scale`` replaces
+    ``1/(1-p)``: the CUDA kernels' counter-based generator scales its survivors by the exact keep
+    probability of its 16-bit threshold (``functional.dropout_mask`` returns it).
     Returns ``out, (edge_index', alpha [E',H])``.
     """
     N, H, C = x.size(0), heads, out_channels
@@ -153,7 +156,10 @@ def gatconv_forward(x, edge_index, W, att_src, att_dst, bias, heads: int, out_ch
     alpha = pexp / s[dst]
     alpha_used = alpha
     if dropout_mask is not None:
-        alpha_used = alpha * dropout_mask.to(alpha.dtype) / (1.0 - p)
+        if dropout_scale is None:
+            alpha_used = alpha * dropout_mask.to(alpha.dtype) / (1.0 - p)
+        else:
+            alpha_used = alpha * dropout_mask.to(alpha.dtype) * dropout_scale
     msg = alpha_used[:, :, None] * xw[src]
     out = torch.zeros(N, H, C, dtype=x.dtype).index_add_(0, dst, msg)
     out = out.reshape(N, H * C) if concat else out.mean(1)
@@ -250,7 +256,7 @@ class OracleGATConv(nn.Module):
         if self.bias is not None:
             nn.init.zeros_(self.bias)
 
-    def forward(self, x, edge_index, return_attention_weights=None, dropout_mask=None):
+    def forward(self, x, edge_index, return_attention_weights=None, dropout_mask=None, dropout_scale=None):
         mask = dropout_mask
         p = self.dropout if self.training else 0.0
         if mask is None and self.training and self.dropout > 0:
@@ -258,7 +264,7 @@ class OracleGATConv(nn.Module):
             mask = torch.rand(n_edges, self.heads) >= self.dropout
         out, (ei, alpha) = gatconv_forward(
             x, edge_index, self.lin_src.weight, self.att_src, self.att_dst, self.bias, self.heads,
-            self.out_channels, self.concat, self.negative_slope, self.add_self_loops, mask, p)
+            self.out_channels, self.concat, self.negative_slope, self.add_self_loops, mask, p, dropout_scale)
         if return_attention_weights:
             return out, (ei, alpha)
         return out
@@ -280,19 +286,29 @@ class OracleGAT(nn.Module):
             nn.BatchNorm1d(hidden_channels) for _ in widths) if use_batch_norm else None
         self.out = nn.Linear(hidden_channels, out_channels)
 
-    def _stack(self, x, edge_index):
+    def _stack(self, x, edge_index, att_masks=None, feat_masks=None, dropout_scale=None):
+        """``att_masks`` / ``feat_masks``: optional per-layer keep-masks, ``[E',8]`` in ``edge_index'`` order for the
+        attention coefficients and ``[N,hidden]`` for the features after the ReLU, applied as ``mask * dropout_scale``
+        (default ``1/(1-p)``) in place of fresh random draws.  Given masks apply whatever the module's mode is."""
         h = x
         for i, gat in enumerate(self.gat_layers):
-            h_new = gat(h, edge_index)
+            if att_masks is None:
+                h_new = gat(h, edge_index)
+            else:
+                h_new = gat(h, edge_index, dropout_mask=att_masks[i], dropout_scale=dropout_scale)
             if self.use_batch_norm:
                 h_new = self.batch_norms[i](h_new)
             h_new = F.relu(h_new)
-            h_new = F.dropout(h_new, p=self.dropout, training=self.training)
+            if feat_masks is None:
+                h_new = F.dropout(h_new, p=self.dropout, training=self.training)
+            else:
+                scale = 1.0 / (1.0 - self.dropout) if dropout_scale is None else dropout_scale
+                h_new = h_new * feat_masks[i].to(h_new.dtype) * scale
             h = h + h_new if (self.residual and h.size(-1) == h_new.size(-1)) else h_new
         return h
 
-    def forward(self, x, edge_index, batch=None):
-        return self.out(self._stack(x, edge_index))
+    def forward(self, x, edge_index, batch=None, att_masks=None, feat_masks=None, dropout_scale=None):
+        return self.out(self._stack(x, edge_index, att_masks, feat_masks, dropout_scale))
 
     def predict(self, x, edge_index, batch=None, apply_sigmoid=True):
         out = self.forward(x, edge_index, batch)
@@ -308,10 +324,11 @@ class OracleTemporalGNN(OracleGAT):
                          use_batch_norm)
         self.gru = nn.GRUCell(hidden_channels, hidden_channels)
 
-    def forward(self, x, edge_index, batch=None, hidden_state=None):
+    def forward(self, x, edge_index, batch=None, hidden_state=None, att_masks=None, feat_masks=None,
+                dropout_scale=None):
         if hidden_state is None:
             hidden_state = torch.zeros(x.size(0), self.hidden_channels, device=x.device)
-        h = self._stack(x, edge_index)
+        h = self._stack(x, edge_index, att_masks, feat_masks, dropout_scale)
         hidden_state = self.gru(h, hidden_state)
         return self.out(hidden_state), hidden_state
 

@@ -7,6 +7,7 @@ import os
 import numpy as np
 import pytest
 import torch
+import torch.nn.functional as F
 
 from oracle import build_c
 from oracle import pyg_gatconv as O
@@ -267,3 +268,74 @@ def test_forward_matches_a_pure_python_loop_restatement(concat):
             exp_out.append([sum(heads[h][c] for h in range(H)) / H + bl[c] for c in range(Cc)])
     assert torch.allclose(alpha, torch.tensor(exp_alpha, dtype=torch.float64), atol=1e-13)
     assert torch.allclose(out, torch.tensor(exp_out, dtype=torch.float64), atol=1e-12)
+
+
+def _model_masks(model, x, ei, gen, p):
+    n_edges = O.rewrite_self_loops(ei, x.size(0)).size(1)
+    L, hid = len(model.gat_layers), model.hidden_channels
+    att = [torch.rand(n_edges, 8, generator=gen) >= p for _ in range(L)]
+    feat = [torch.rand(x.size(0), hid, generator=gen) >= p for _ in range(L)]
+    return att, feat
+
+
+@pytest.mark.parametrize("cls", [O.OracleGAT, O.OracleTemporalGNN])
+def test_models_with_all_ones_masks_and_unit_scale_equal_the_dropout_free_model(cls):
+    x, ei, _ = synth.elliptic_synth(num_nodes=300, num_edges=400, num_feats=12, seed=0)
+    x = x.double()
+    torch.manual_seed(0)
+    m = cls(12, 64, 1, num_layers=3, dropout=0.3).double().train()
+    m0 = cls(12, 64, 1, num_layers=3, dropout=0.0).double().train()
+    m0.load_state_dict(m.state_dict(), strict=True)
+    ones_a = [torch.ones(O.rewrite_self_loops(ei, x.size(0)).size(1), 8, dtype=torch.bool)] * 3
+    ones_f = [torch.ones(x.size(0), 64, dtype=torch.bool)] * 3
+    kw = {"hidden_state": torch.zeros(x.size(0), 64, dtype=torch.float64)} if cls is O.OracleTemporalGNN else {}
+    r = m(x, ei, att_masks=ones_a, feat_masks=ones_f, dropout_scale=1.0, **kw)
+    r0 = m0(x, ei, **kw)
+    out, out0 = (r[0], r0[0]) if isinstance(r, tuple) else (r, r0)
+    assert torch.equal(out, out0)
+    out.square().sum().backward()
+    out0.square().sum().backward()
+    for (n, pa), (_, pb) in zip(m.named_parameters(), m0.named_parameters()):
+        assert torch.equal(pa.grad, pb.grad), n
+
+
+@pytest.mark.parametrize("cls", [O.OracleGAT, O.OracleTemporalGNN])
+@pytest.mark.parametrize("p", [0.2, 0.5])
+def test_models_with_injected_masks_equal_a_loop_restatement_with_f_dropout(cls, p):
+    """The oracle's explicit-mask path against the reference's layer loop (src/models/gat.py:78-96) written out with the
+    same masks: attention dropout through ``gatconv_forward`` (``mask / (1-p)``) and feature dropout through ``F.dropout``
+    itself, under a seed whose draws are the injected feature masks."""
+    x, ei, _ = synth.elliptic_synth(num_nodes=300, num_edges=400, num_feats=12, seed=1)
+    x = x.double()
+    torch.manual_seed(0)
+    m = cls(12, 64, 1, num_layers=3, dropout=p).double().train()
+    att, _ = _model_masks(m, x, ei, torch.Generator().manual_seed(5), p)
+    # the feature masks F.dropout draws for [N,64] under seeds 100 + i
+    feat = []
+    for i in range(3):
+        torch.manual_seed(100 + i)
+        feat.append(F.dropout(torch.ones(x.size(0), 64, dtype=torch.float64), p=p, training=True) != 0)
+    kw = {"hidden_state": torch.zeros(x.size(0), 64, dtype=torch.float64)} if cls is O.OracleTemporalGNN else {}
+    r = m(x, ei, att_masks=att, feat_masks=feat, **kw)
+    got = r[0] if isinstance(r, tuple) else r
+
+    h = x
+    for i, conv in enumerate(m.gat_layers):
+        z, _ = O.gatconv_forward(h, ei, conv.lin_src.weight, conv.att_src, conv.att_dst, conv.bias, 8, 64,
+                                 dropout_mask=att[i], p=p)
+        bn = m.batch_norms[i]
+        z = F.relu(F.batch_norm(z, None, None, bn.weight, bn.bias, training=True, eps=bn.eps))
+        torch.manual_seed(100 + i)
+        z = F.dropout(z, p=p, training=True)
+        h = h + z if h.size(-1) == z.size(-1) else z
+    if cls is O.OracleTemporalGNN:
+        h = m.gru(h, torch.zeros(x.size(0), 64, dtype=torch.float64))
+    want = m.out(h)
+    assert float((got - want).detach().abs().max()) <= 1e-12 * float(want.detach().abs().max())
+    # an explicit scale replaces 1/(1-p) in both places: the same masks at scale s equal masks at 1/(1-p), rescaled layer
+    # by layer -- checked on the first layer's output, where nothing else intervenes
+    s = 1.0 / (1.0 - p) * (1 + 1e-3)
+    conv = m.gat_layers[0]
+    a = conv(x, ei, dropout_mask=att[0], dropout_scale=s) - conv.bias
+    b = conv(x, ei, dropout_mask=att[0]) - conv.bias
+    assert torch.allclose(a, b * (1 + 1e-3), rtol=1e-12, atol=1e-15)
