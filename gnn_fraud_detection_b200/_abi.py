@@ -18,7 +18,7 @@ F32, BF16 = 0, 1
 ACT_NONE, ACT_RELU, ACT_ELU = 0, 1, 2
 GEMM_AUTO, GEMM_SIMT, GEMM_TC, GEMM_INPUT = 0, 1, 2, 3
 HUB_THRESHOLD, HUB_CHUNK = 512, 512
-ABI_VERSION = 21
+ABI_VERSION = 22
 
 _i32p = C.POINTER(C.c_int32)
 
@@ -115,6 +115,8 @@ SIGNATURES = {
     "gnnfd_bn_sums": (_i, [_vp, _i64, _i, _vp, _vp, _sz, _vp]),
     "gnnfd_bn_finalize": (_i, [_vp, C.c_double, _i, _f, _f, _vp, _vp, _vp, _vp, _vp]),
     "gnnfd_bn_relu_drop_res_fwd": (_i, [_vp, _i64, _i, _vp, _vp, _vp, _vp, _f, _u64, _i64, _vp, _vp, _vp]),
+    "gnnfd_bn_relu_drop_res_fwd_bcast": (_i, [_vp, _i64, _i, _vp, _vp, _vp, _vp, _f, _u64, _i64, _vp, C.POINTER(Peers), _i64, _i,
+                                             _vp, _vp]),
     "gnnfd_bn_bwd_sums": (_i, [_vp, _vp, _i64, _i, _vp, _vp, _vp, _vp, _f, _u64, _i64, _vp, _vp, _sz, _vp]),
     "gnnfd_bn_bwd_apply": (_i, [_vp, _vp, _i64, _i, _vp, _vp, _vp, _vp, _f, _u64, _i64, _vp, C.c_double, _vp, _vp, _vp, _vp]),
     "gnnfd_gru_head_fwd": (_i, [_vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),

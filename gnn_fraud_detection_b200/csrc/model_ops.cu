@@ -12,7 +12,7 @@
 //        mean over labelled nodes, its gradient, and the confusion counters of src/train.py:146-149 -- no host sync.
 // Column reductions over nodes use per-block partials in double, summed in block order: deterministic, and accurate enough
 // that the batch variance needs no second pass.
-#include "gat_common.cuh"
+#include "in_common.cuh"
 
 #include <atomic>
 
@@ -94,11 +94,15 @@ __global__ void bn_finalize_kernel(const double* __restrict__ sums, double count
     }
 }
 
-// out = residual + dropout(relu((z - mean) * invstd * gamma + beta))
+// out = residual + dropout(relu((z - mean) * invstd * gamma + beta)).  PM (in::PeerRows::mode): 0 = out only (the
+// single-GPU kernel); 1 / 2 = each finished 16-byte piece also goes to element (row_off * C + i) of the symmetric buffer
+// on every rank (one store per peer / one multimem.st), and out may be NULL.
+template <int PM>
 __global__ void __launch_bounds__(256)
 bn_apply_fwd_kernel(const float* __restrict__ z, int64_t total, int C, const float* __restrict__ mean,
                     const float* __restrict__ invstd, const float* __restrict__ gamma, const float* __restrict__ beta,
-                    KeepMask km, float keep_scale, int64_t elem_base, const float* __restrict__ residual, float* __restrict__ out)
+                    KeepMask km, float keep_scale, int64_t elem_base, const float* __restrict__ residual, float* __restrict__ out,
+                    in::PeerRows peers)
 {
     for (int64_t i = (blockIdx.x * int64_t(blockDim.x) + threadIdx.x) * 4; i < total; i += int64_t(gridDim.x) * blockDim.x * 4) {
         const int c = int(i % C);
@@ -113,7 +117,12 @@ bn_apply_fwd_kernel(const float* __restrict__ z, int64_t total, int C, const flo
             if (km.thr || km.mask) y = (km.bits(elem_base + i + k, 1) & 1u) ? y * keep_scale : 0.f;
             rr[k] += y;
         }
-        *reinterpret_cast<float4*>(out + i) = make_float4(rr[0], rr[1], rr[2], rr[3]);
+        const float4 o4 = make_float4(rr[0], rr[1], rr[2], rr[3]);
+        if (PM == 0 || out) *reinterpret_cast<float4*>(out + i) = o4;
+        if (PM == 1)
+            for (int g = 0; g < peers.n; ++g) *reinterpret_cast<float4*>(peers.ptr[g] + peers.row_off * C + i) = o4;
+        else if (PM == 2)
+            in::multimem_st_v4(peers.mc + peers.row_off * C + i, o4);
     }
 }
 // dz = gamma * invstd * (dy - s1/count - zhat * s2/count),  dy = d_out * keep * relu'
@@ -585,8 +594,44 @@ int gnnfd_bn_relu_drop_res_fwd(const float* z, int64_t N, int C, const float* me
     const int64_t total = N * C;
     int64_t blocks = (total / 4 + 255) / 256;
     if (blocks > int64_t(sm_count()) * 16) blocks = int64_t(sm_count()) * 16;
-    bn_apply_fwd_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(z, total, C, mean, invstd, gamma, beta, km, ks,
-                                                                         row_base * C, residual, out);
+    bn_apply_fwd_kernel<0><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(z, total, C, mean, invstd, gamma, beta, km, ks,
+                                                                            row_base * C, residual, out, in::PeerRows{});
+    g_launches += 1;
+    GNNFD_LAUNCH_CHECK();
+    return GNNFD_OK;
+}
+
+/* gnnfd_bn_relu_drop_res_fwd fused with the all-gather of its rows: every finished 16-byte piece of row r also goes to row
+ * (row_offset + r) of h_all [n_pos, C] on every rank (one multimem.st, or one store per peer).  out (own rows) may be NULL. */
+int gnnfd_bn_relu_drop_res_fwd_bcast(const float* z, int64_t N, int C, const float* mean, const float* invstd,
+                                     const float* gamma, const float* beta, float p_drop, uint64_t dropout_seed,
+                                     int64_t row_base, const float* residual, const gnnfd_peers_t* h_all,
+                                     int64_t row_offset, int use_multicast, float* out, gnnfd_stream_t stream)
+{
+    GNNFD_REQUIRE(C >= 4 && C % 4 == 0 && N >= 0 && p_drop >= 0.f && p_drop < 1.f, GNNFD_ERR_ARG,
+                  "bn_relu_drop_res_fwd_bcast: bad argument");
+    in::PeerRows peers;
+    const int rc = in::peer_rows_from(h_all, row_offset, use_multicast, "bn_relu_drop_res_fwd_bcast", peers);
+    if (rc) return rc;
+    GNNFD_REQUIRE(!use_multicast || (reinterpret_cast<uintptr_t>(h_all->multicast) & 15) == 0, GNNFD_ERR_ARG,
+                  "bn_relu_drop_res_fwd_bcast: the multicast address must be 16-byte aligned");
+    if (N == 0) return GNNFD_OK;
+    GNNFD_REQUIRE(z && mean && invstd, GNNFD_ERR_ARG, "bn_relu_drop_res_fwd_bcast: NULL tensor");
+    GNNFD_REQUIRE((reinterpret_cast<uintptr_t>(z) & 15) == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0 &&
+                  (reinterpret_cast<uintptr_t>(residual) & 15) == 0, GNNFD_ERR_ARG,
+                  "bn_relu_drop_res_fwd_bcast: z, residual and out must be 16-byte aligned");
+    float ks = 1.f;
+    const KeepMask km = make_keep(nullptr, p_drop, dropout_seed, &ks);
+    const int64_t total = N * C;
+    int64_t blocks = (total / 4 + 255) / 256;
+    if (blocks > int64_t(sm_count()) * 16) blocks = int64_t(sm_count()) * 16;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (use_multicast)
+        bn_apply_fwd_kernel<2><<<(unsigned)blocks, 256, 0, st>>>(z, total, C, mean, invstd, gamma, beta, km, ks, row_base * C,
+                                                                residual, out, peers);
+    else
+        bn_apply_fwd_kernel<1><<<(unsigned)blocks, 256, 0, st>>>(z, total, C, mean, invstd, gamma, beta, km, ks, row_base * C,
+                                                                residual, out, peers);
     g_launches += 1;
     GNNFD_LAUNCH_CHECK();
     return GNNFD_OK;

@@ -214,12 +214,15 @@ def gat_bwd_dst(g: GraphCSR, xw, a_src, a_dst, rowmax, rowsum, d_out, H, C_, neg
     return alpha_used, dz, da_dst
 
 
-def gat_bwd_src(g: GraphCSR, alpha_used, dz, d_out, att_src, att_dst, da_dst_full, H, C_, concat):
-    """src-major pass over g's CSC: dxw [n_src,H*C] and da_src [n_src,H]."""
+def gat_bwd_src(g: GraphCSR, alpha_used, dz, d_out, att_src, att_dst, da_dst_full, H, C_, concat, da_src_out=None):
+    """src-major pass over g's CSC: dxw [n_src,H*C] and da_src [n_src,H] (written into ``da_src_out`` if given)."""
     L = _abi.lib()
     dev = alpha_used.device
     dxw = torch.empty(g.n_src, H * C_, dtype=torch.float32, device=dev)
-    da_src = torch.empty(g.n_src, H, dtype=torch.float32, device=dev)
+    if da_src_out is not None and (tuple(da_src_out.shape) != (g.n_src, H) or da_src_out.dtype != torch.float32
+                                   or not da_src_out.is_contiguous() or da_src_out.device != dev):
+        raise ValueError(f"da_src_out must be a contiguous float32 [{g.n_src},{H}] tensor on {dev}")
+    da_src = da_src_out if da_src_out is not None else torch.empty(g.n_src, H, dtype=torch.float32, device=dev)
     nb = C.c_size_t()
     _abi.check(L.gnnfd_gat_bwd_workspace_bytes(g.ref(), H, C_, C.byref(nb)))
     ws = _ws(nb.value, dev)
@@ -248,16 +251,19 @@ def project_bwd(x, W, dxw, xw, da_src, da_dst, d_out, H, C_, Co, need_dx, algo=_
     return dW, datt_src, datt_dst, dbias, dx
 
 
-def project_dx(dxw, W, H, C_):
-    """dx [N,K] = dxw [N,H*C] W: the dx GEMM of ``project_bwd`` alone (for a layer that has no xw)."""
+def project_dx(dxw, W, H, C_, out=None):
+    """dx [N,K] = dxw [N,H*C] W: the dx GEMM of ``project_bwd`` alone (for a layer that has no xw).  ``out``: an [N,K] view
+    with unit column stride to write into (e.g. a symmetric buffer the ranks reduce from)."""
     L = _abi.lib()
     N, K = dxw.size(0), W.size(1)
-    dx = torch.empty(N, K, dtype=torch.float32, device=dxw.device)
+    if out is not None and (tuple(out.shape) != (N, K) or out.stride(1) != 1 or out.dtype != torch.float32):
+        raise ValueError(f"out must be float32 [{N},{K}] with unit column stride")
+    dx = out if out is not None else torch.empty(N, K, dtype=torch.float32, device=dxw.device)
     nb = C.c_size_t()
     _abi.check(L.gnnfd_project_dx_workspace_bytes(N, K, H, C_, C.byref(nb)))
     ws = _ws(nb.value, dxw.device)
-    _abi.check(L.gnnfd_project_dx(dxw.data_ptr(), W.data_ptr(), N, K, H, C_, dx.data_ptr(), K, ws.data_ptr(), ws.numel(),
-                                  _stream()))
+    _abi.check(L.gnnfd_project_dx(dxw.data_ptr(), W.data_ptr(), N, K, H, C_, dx.data_ptr(), dx.stride(0), ws.data_ptr(),
+                                  ws.numel(), _stream()))
     return dx
 
 

@@ -35,7 +35,7 @@ def _draw_seed() -> int:
 class _BNReluDropRes(torch.autograd.Function):
     @staticmethod
     def forward(ctx, z, gamma, beta, residual, running_mean, running_var, eps, momentum, p_drop, seed, row_base, group,
-                global_rows):
+                global_rows, bcast):
         L = _abi.lib()
         z = z.contiguous()
         N, Cc = z.shape
@@ -62,9 +62,16 @@ class _BNReluDropRes(torch.autograd.Function):
                                            _abi.ptr(running_var), mean.data_ptr(), invstd.data_ptr(), _stream()))
             out = torch.empty_like(z)
             res = None if residual is None else residual.contiguous()
-            _abi.check(L.gnnfd_bn_relu_drop_res_fwd(z.data_ptr(), N, Cc, mean.data_ptr(), invstd.data_ptr(), _abi.ptr(gamma),
-                                                    _abi.ptr(beta), float(p_drop), int(seed), int(row_base), _abi.ptr(res),
-                                                    out.data_ptr(), _stream()))
+            if bcast is None:
+                _abi.check(L.gnnfd_bn_relu_drop_res_fwd(z.data_ptr(), N, Cc, mean.data_ptr(), invstd.data_ptr(),
+                                                        _abi.ptr(gamma), _abi.ptr(beta), float(p_drop), int(seed),
+                                                        int(row_base), _abi.ptr(res), out.data_ptr(), _stream()))
+            else:
+                peers, row_offset, use_multicast = bcast
+                _abi.check(L.gnnfd_bn_relu_drop_res_fwd_bcast(z.data_ptr(), N, Cc, mean.data_ptr(), invstd.data_ptr(),
+                                                              _abi.ptr(gamma), _abi.ptr(beta), float(p_drop), int(seed),
+                                                              int(row_base), _abi.ptr(res), C.byref(peers), int(row_offset),
+                                                              int(use_multicast), out.data_ptr(), _stream()))
         ctx.save_for_backward(z, mean, invstd, gamma, beta)
         ctx.p, ctx.seed, ctx.row_base, ctx.group, ctx.count = p_drop, seed, row_base, group, count
         ctx.has_res = residual is not None
@@ -92,17 +99,21 @@ class _BNReluDropRes(torch.autograd.Function):
                                             _abi.ptr(gamma), _abi.ptr(beta), float(ctx.p), int(ctx.seed), int(ctx.row_base),
                                             sums.data_ptr(), float(ctx.count), dz.data_ptr(), _abi.ptr(dgamma), _abi.ptr(dbeta),
                                             _stream()))
-        return dz, dgamma, dbeta, (d_out if ctx.has_res else None), None, None, None, None, None, None, None, None, None
+        return (dz, dgamma, dbeta, (d_out if ctx.has_res else None), None, None, None, None, None, None, None, None, None,
+                None)
 
 
 def bn_relu_dropout_residual(z: torch.Tensor, bn: nn.BatchNorm1d, p_drop: float = 0.0,
                              residual: Optional[torch.Tensor] = None, seed: Optional[int] = None, row_base: int = 0,
-                             group=None, global_rows: Optional[int] = None) -> torch.Tensor:
+                             group=None, global_rows: Optional[int] = None, bcast=None) -> torch.Tensor:
     """``residual + dropout(relu(bn(z)))`` with ``bn`` in TRAINING mode (batch statistics, running buffers updated).
 
     ``group``: a process group whose ranks hold disjoint rows of one batch -- the statistics are then those of the whole
     batch and ``row_base`` is this rank's first global row (it keys the dropout generator); ``global_rows`` = the batch size
-    over all ranks, if known (saves a collective and a host synchronisation: required under CUDA-graph capture)."""
+    over all ranks, if known (saves a collective and a host synchronisation: required under CUDA-graph capture).
+    ``bcast = (peers, row_offset, use_multicast)``: the finished rows also go to rows ``row_offset ..`` of the symmetric
+    ``[n_pos, C]`` buffer described by ``peers`` (``_abi.Peers``) on EVERY rank (``gnnfd_bn_relu_drop_res_fwd_bcast``); the
+    caller puts a cross-GPU barrier between this and the first read of that buffer."""
     if not z.is_cuda or z.dtype != torch.float32 or z.dim() != 2:
         raise RuntimeError("bn_relu_dropout_residual needs a float32 CUDA tensor [N,C] (no CPU fallback)")
     if not bn.training:
@@ -116,7 +127,7 @@ def bn_relu_dropout_residual(z: torch.Tensor, bn: nn.BatchNorm1d, p_drop: float 
     if p_drop > 0.0 and seed is None:
         seed = _draw_seed()
     out = _BNReluDropRes.apply(z, bn.weight, bn.bias, residual, bn.running_mean, bn.running_var, bn.eps, bn.momentum,
-                               float(p_drop), int(seed or 0), int(row_base), group, global_rows)
+                               float(p_drop), int(seed or 0), int(row_base), group, global_rows, bcast)
     if bn.num_batches_tracked is not None:
         bn.num_batches_tracked.add_(1)
     return out

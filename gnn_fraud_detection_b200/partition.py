@@ -438,6 +438,36 @@ class PeerExchange:
         self.handles[0].barrier()
 
 
+def exchange_logits(part, px, x_own, W, a_s, a_d, prep, xmax):
+    """The logits of this rank's rows ``x_own`` and their exchange, for one input-space layer on a destination-range
+    partition.  Returns ``(a_src of every position [n_pos,H], a_dst of the own rows)`` and leaves max|input| over all ranks in
+    ``xmax`` (the fp16-pair scale ``in_prepare`` needs).
+
+    With a ``PeerExchange`` the logits kernel stores its rows into ``px.a_src`` ON EVERY RANK (NVLink stores / one multicast
+    store), then a barrier and the max-reduce of ``xmax``; otherwise the own rows, zero-padded to ``rows_padded``, are
+    all-gathered with NCCL."""
+    from . import functional as Fn
+    lo = part.rank * part.rows_padded
+    if px is not None:
+        px.xmax.zero_()
+        a_dst = Fn.in_logits_bcast(x_own, W, a_s, a_d, prep, px.xmax, px.a_src_peers, lo, px.mode == "multicast")
+        px.barrier()
+        Fn.peer_reduce(px.xmax_peers, 0, 4, xmax, op="max")
+        return px.a_src, a_dst
+    xmax.zero_()
+    a_src_own, a_dst = Fn.in_logits(x_own, W, a_s, a_d, prep, xmax)
+    if part.world == 1:
+        return a_src_own, a_dst
+    if a_src_own.size(0) < part.rows_padded:
+        a_pad = torch.zeros(part.rows_padded, a_src_own.size(1), dtype=torch.float32, device=a_src_own.device)
+        a_pad[:a_src_own.size(0)] = a_src_own
+        a_src_own = a_pad
+    a_src_full = torch.empty(part.n_pos, a_src_own.size(1), dtype=torch.float32, device=a_src_own.device)
+    dist.all_gather_into_tensor(a_src_full, a_src_own)
+    dist.all_reduce(xmax, op=dist.ReduceOp.MAX)
+    return a_src_full, a_dst
+
+
 class InputSpacePartition(DstRangePartition):
     """Destination-range partition of the FIRST layer in the input-space formulation (csrc/in_common.cuh).
 
@@ -495,27 +525,13 @@ class InputSpacePartition(DstRangePartition):
         if marks: marks[0].record()
         # forward: logits of the own rows, gathered from every rank; softmax / aggregation / output GEMM are local
         x_own = x_full[lo:lo + P]
-        if px is not None:
-            # fused: the logits kernel stores its rows into a_src_full ON EVERY RANK (NVLink stores / one multicast store)
-            px.xmax.zero_()
-            a_dst_own = Fn.in_logits_bcast(x_own, W, a_s, a_d, prep, px.xmax, px.a_src_peers, lo, px.mode == "multicast")
-            px.barrier()
-            a_src_full = px.a_src
-            Fn.peer_reduce(px.xmax_peers, 0, 4, xmax, op="max")
-        elif self.world > 1 and self.redundant_logits:
+        if self.world > 1 and self.redundant_logits:
             # every rank holds all of x: 32 B of logits per node can also be recomputed locally instead of gathered
             xmax.zero_()
             a_src_full, a_dst_full = Fn.in_logits(x_full, W, a_s, a_d, prep, xmax)
             a_dst_own = a_dst_full[lo:lo + P]
         else:
-            xmax.zero_()
-            a_src_own, a_dst_own = Fn.in_logits(x_own, W, a_s, a_d, prep, xmax)
-            if self.world > 1:
-                a_src_full = torch.empty(self.n_pos, H, dtype=torch.float32, device=dev)
-                dist.all_gather_into_tensor(a_src_full, a_src_own)
-                dist.all_reduce(xmax, op=dist.ReduceOp.MAX)
-            else:
-                a_src_full = a_src_own
+            a_src_full, a_dst_own = exchange_logits(self, px, x_own, W, a_s, a_d, prep, xmax)
         Fn.in_prepare(W, K, xmax, prep)
         if marks: marks[1].record()
         zimg, att = Fn.in_fwd(g, x_full, a_src_full, a_dst_own, 0.2, prep)
@@ -655,15 +671,19 @@ class InputSpaceModelPartition(DstRangePartition):
     H, HIDDEN = 8, 64
 
     @staticmethod
-    def check_model(model):
-        """Refuse what this path does not compute, before anything is launched."""
+    def check_model(model, training=False):
+        """Refuse what this path does not compute, before anything is launched.  ``training``: checked for
+        ``InputSpaceModelTrainStep`` (train mode required) instead of ``forward`` (eval mode required)."""
         from . import functional as Fn
         from .models import GAT, TemporalGNN
         if not isinstance(model, (GAT, TemporalGNN)):
             raise TypeError(f"InputSpaceModelPartition runs GAT or TemporalGNN, not {type(model).__name__}")
-        if model.training:
-            raise RuntimeError("InputSpaceModelPartition is inference only: call model.eval() first "
-                               "(training across GPUs is not supported)")
+        if model.training and not training:
+            raise RuntimeError("InputSpaceModelPartition.forward is inference only: call model.eval() first "
+                               "(InputSpaceModelTrainStep trains across GPUs)")
+        if training and not model.training:
+            raise RuntimeError("InputSpaceModelTrainStep trains the model: call model.train() first "
+                               "(InputSpaceModelPartition.forward scores it)")
         if model.hidden_channels != InputSpaceModelPartition.HIDDEN:
             raise NotImplementedError(f"InputSpaceModelPartition is built for hidden_channels=64, got {model.hidden_channels}")
         for i, conv in enumerate(model.gat_layers):
@@ -677,26 +697,29 @@ class InputSpaceModelPartition(DstRangePartition):
                                           f"(got in_channels={conv.in_channels}, concat={conv.concat})")
 
     def _setup_exchange(self):
+        self.px, self.hidden, self.hidden_peers, self._handles, self.exchange = self.hidden_buffers(2)
+
+    def hidden_buffers(self, count):
+        """``count`` ``[n_pos, 64]`` buffers every rank holds whole, and the exchange that fills them:
+        ``(PeerExchange or None, tensors, peer tables or None, rendezvous handles, exchange name)``.  Symmetric memory unless
+        ``GNNFD_EXCHANGE=nccl`` or the box has none (then zero-filled plain tensors for the NCCL collectives)."""
         import os
         mode = os.environ.get("GNNFD_EXCHANGE", "auto")
         shape = (self.n_pos, self.HIDDEN)
-        self.px = None
+        px = None
         if self.world > 1 and mode != "nccl":
             try:
-                px = PeerExchange(self.n_pos, self.device, mode, self.H)
-                bufs = [symmetric_buffer(shape, self.device) for _ in range(2)]
-                self.px = px
+                px_try = PeerExchange(self.n_pos, self.device, mode, self.H)
+                bufs = [symmetric_buffer(shape, self.device) for _ in range(count)]
+                px = px_try
             except Exception as ex:               # no symmetric memory on this box: NCCL collectives
                 if mode != "auto":
                     raise
                 self.px_error = f"{type(ex).__name__}: {ex}"
-        if self.px is not None:
-            self.hidden = [b[0] for b in bufs]
-            self.hidden_peers = [b[1] for b in bufs]
-            self._handles = [b[2] for b in bufs]
-        else:
-            self.hidden = [torch.zeros(shape, dtype=torch.float32, device=self.device) for _ in range(2)]
-        self.exchange = self.px.mode if self.px is not None else ("nccl" if self.world > 1 else "none")
+        exchange = px.mode if px is not None else ("nccl" if self.world > 1 else "none")
+        if px is not None:
+            return px, [b[0] for b in bufs], [b[1] for b in bufs], [b[2] for b in bufs], exchange
+        return None, [torch.zeros(shape, dtype=torch.float32, device=self.device) for _ in range(count)], None, [], exchange
 
     @torch.no_grad()
     def forward(self, model, x_full, marks=None):
@@ -729,22 +752,7 @@ class InputSpaceModelPartition(DstRangePartition):
             a_s, a_d = conv.att_src.reshape(-1).contiguous(), conv.att_dst.reshape(-1).contiguous()
             prep = Fn._aligned_u8(Fn.in_sizes(n, K)[0], dev)
             xmax = torch.zeros(16, dtype=torch.float32, device=dev)
-            if px is not None:
-                px.xmax.zero_()
-                a_dst = Fn.in_logits_bcast(x_own, W, a_s, a_d, prep, px.xmax, px.a_src_peers, lo, px.mode == "multicast")
-                px.barrier()
-                a_src_full = px.a_src
-                Fn.peer_reduce(px.xmax_peers, 0, 4, xmax, op="max")
-            else:
-                a_src_own, a_dst = Fn.in_logits(x_own, W, a_s, a_d, prep, xmax)
-                if self.world > 1:
-                    a_pad = torch.zeros(P, self.H, dtype=torch.float32, device=dev)
-                    a_pad[:n] = a_src_own
-                    a_src_full = torch.empty(self.n_pos, self.H, dtype=torch.float32, device=dev)
-                    dist.all_gather_into_tensor(a_src_full, a_pad)
-                    dist.all_reduce(xmax, op=dist.ReduceOp.MAX)
-                else:
-                    a_src_full = a_src_own
+            a_src_full, a_dst = exchange_logits(self, px, x_own, W, a_s, a_d, prep, xmax)
             Fn.in_prepare(W, K, xmax, prep)
             if m: m[1].record()
             zimg, att = Fn.in_fwd(self.graph, h_in, a_src_full, a_dst, conv.negative_slope, prep)
@@ -769,3 +777,264 @@ class InputSpaceModelPartition(DstRangePartition):
         if isinstance(model, TemporalGNN):
             return fused.gru_head(h_own, model.gru, model.out), (int(self.plan.start[self.rank]), int(self.plan.start[self.rank + 1]))
         return model.out(h_own), (int(self.plan.start[self.rank]), int(self.plan.start[self.rank + 1]))
+
+
+def _splitmix64(x: int) -> int:
+    x = (x + 0x9E3779B97F4A7C15) & 0xFFFFFFFFFFFFFFFF
+    x = ((x ^ (x >> 30)) * 0xBF58476D1CE4E5B9) & 0xFFFFFFFFFFFFFFFF
+    x = ((x ^ (x >> 27)) * 0x94D049BB133111EB) & 0xFFFFFFFFFFFFFFFF
+    return x ^ (x >> 31)
+
+
+class _RankLayer(torch.autograd.Function):
+    """One GATConv layer in the input-space formulation on this rank's destination rows.
+
+    forward ``(x_own, W, att_src, att_dst, bias)`` -> ``z [n_local, 64]`` (no activation); ``x_full``, the layer input of every
+    position, is read as data.  ``x_own`` (its own rows) is the differentiable input: backward returns ``d x_own`` = the sum
+    over ranks of every rank's ``dx`` partial over all ``n_pos`` source positions, reduced to the owner -- each partial is
+    written by the dx GEMM straight into this rank's symmetric buffer and pulled by the owners (``gnnfd_peer_reduce``), or
+    reduce-scattered with NCCL."""
+
+    @staticmethod
+    def forward(ctx, x_own, W, att_src, att_dst, bias, step, x_full, slope, p_drop, seed, marks):
+        from . import functional as Fn
+        part, px = step.part, step.px
+        n, K, dev = part.n_local, x_full.size(1), x_full.device
+        W = W.contiguous()
+        a_s, a_d = att_src.reshape(-1).contiguous(), att_dst.reshape(-1).contiguous()
+        if marks: marks[0].record()
+        prep = Fn._aligned_u8(Fn.in_sizes(n, K)[0], dev)
+        xmax = torch.zeros(16, dtype=torch.float32, device=dev)
+        a_src_full, a_dst = exchange_logits(part, px, x_own, W, a_s, a_d, prep, xmax)
+        Fn.in_prepare(W, K, xmax, prep)
+        if marks: marks[1].record()
+        zimg, att = Fn.in_fwd(part.graph, x_full, a_src_full, a_dst, slope, prep, None, p_drop, seed)
+        if marks: marks[2].record()
+        z = Fn.in_out(zimg, n, K, prep, bias)
+        ctx.save_for_backward(x_own, W, a_s, a_d, att.alpha, att.jflag, att.rowmax, att.rowsum, zimg, prep)
+        ctx.step, ctx.x_full, ctx.slope, ctx.p, ctx.seed, ctx.marks = step, x_full, slope, p_drop, seed, marks
+        ctx.att_shape, ctx.has_bias = att_src.shape, bias is not None
+        return z
+
+    @staticmethod
+    def backward(ctx, d_out):
+        from . import functional as Fn
+        x_own, W, a_s, a_d, alpha, jflag, rowmax, rowsum, zimg, prep = ctx.saved_tensors
+        step, marks = ctx.step, ctx.marks
+        part, px = step.part, step.px
+        g, n, P, H, dev = part.graph, part.n_local, part.rows_padded, 8, x_own.device
+        lo = part.rank * P
+        d_out = d_out.contiguous()
+        att = Fn.InAttention(alpha, jflag, rowmax, rowsum)
+        need_dx = ctx.needs_input_grad[0]
+        if marks: marks[4].record()
+        da_out = px.da_part if px is not None else None
+        if need_dx:
+            alpha_used, dz, da_dst = Fn.in_bwd_edges(g, ctx.x_full, att, d_out, prep, ctx.slope, None, ctx.p, seed=ctx.seed,
+                                                     records=True)
+            if marks: marks[5].record()
+            da_dst_full = torch.zeros(part.n_pos, H, dtype=torch.float32, device=dev)
+            da_dst_full[lo:lo + n] = da_dst
+            # dxw_part [n_pos, H*C] and da_src_part: linear in this rank's edges, so their sums over ranks are the layer's
+            dxw, da_part = Fn.gat_bwd_src(g, alpha_used, dz, d_out, a_s, a_d, da_dst_full, H, 64, False, da_src_out=da_out)
+        else:
+            dz, da_dst = Fn.in_bwd_edges(g, ctx.x_full, att, d_out, prep, ctx.slope, None, ctx.p, seed=ctx.seed)
+            if marks: marks[5].record()
+            da_part = Fn.in_dasrc(g, dz, out=da_out)
+        if marks: marks[6].record()
+        if px is not None:
+            # the da_src exchange runs on the side stream under the tensor-core part of the weight gradient (dO^T Z)
+            da_src = torch.empty(P, H, dtype=torch.float32, device=dev)
+            main = torch.cuda.current_stream()
+            px.side.wait_stream(main)
+            with torch.cuda.stream(px.side):
+                px.barrier()
+                Fn.peer_reduce(px.da_peers, lo * H, P * H, da_src, op="sum", use_multicast=px.mode == "multicast")
+            finish = Fn.in_bwd_params_split(zimg, d_out, x_own, W, a_s, a_d, prep)
+            main.wait_stream(px.side)
+            dW, datt_s, datt_d, dbias = finish(da_src[:n], da_dst)
+        else:
+            if part.world > 1:
+                da_src = torch.empty(P, H, dtype=torch.float32, device=dev)
+                dist.reduce_scatter_tensor(da_src, da_part)
+            else:
+                da_src = da_part
+            dW, datt_s, datt_d, dbias = Fn.in_bwd_params(zimg, d_out, x_own, W, a_s, a_d, da_src[:n], da_dst, prep)
+        if marks: marks[7].record()
+        dx = None
+        if need_dx:
+            if px is not None:
+                # every rank passed the da_src barrier above only after its previous layer's dx pulls: the buffer is free
+                Fn.project_dx(dxw, W, H, 64, out=step.dx_buf)
+                px.barrier()
+                dh = torch.empty(P, 64, dtype=torch.float32, device=dev)
+                Fn.peer_reduce(step.dx_peers, lo * 64, P * 64, dh, op="sum",
+                               use_multicast=px.mode == "multicast" and step.dx_peers.multicast is not None)
+            else:
+                dx_part = Fn.project_dx(dxw, W, H, 64)
+                if part.world > 1:
+                    dh = torch.empty(P, 64, dtype=torch.float32, device=dev)
+                    dist.reduce_scatter_tensor(dh, dx_part)
+                else:
+                    dh = dx_part
+            dx = dh[:n]
+        if marks: marks[8].record()
+        return (dx, dW, datt_s.view(ctx.att_shape), datt_d.view(ctx.att_shape), dbias if ctx.has_bias else None,
+                None, None, None, None, None, None)
+
+
+class InputSpaceModelTrainStep:
+    """Training of a whole ``GAT`` / ``TemporalGNN`` on a destination-range partition (``InputSpaceModelPartition``), every
+    layer in the input-space formulation -- the cross-GPU form of one full-batch step of the single-GPU model with
+    ``gemm_algo=GEMM_INPUT`` on every layer, ``fused.masked_bce_with_logits`` and Adam.
+
+    ``x_full``: the model input replicated in padded position space (as ``InputSpaceModelPartition.forward`` takes it);
+    ``y``: the global labels ``[N]`` (-1 = unlabelled), of which each rank uses its own rows.  The parameters and buffers are
+    broadcast from rank 0 at construction.  ``step()`` runs the forward, the loss of the own rows weighted by this rank's
+    share of the labelled nodes (the global mean over labelled nodes), ``backward``, one all-reduce of the flat parameter
+    gradients (the BatchNorm affine gradients come out of the tail's backward already summed) and Adam, identical on every
+    rank.  Per layer each rank
+      forward   gathers the logits of its rows to every rank (``exchange_logits``), aggregates over its destination rows,
+                runs the output GEMM, then BatchNorm with the batch statistics of all ranks (one all-reduce of the column sums),
+                ReLU, feature dropout and the residual; the finished rows are stored into the next layer's input buffer on
+                every rank (``gnnfd_bn_relu_drop_res_fwd_bcast``), then a barrier;
+      backward  runs the edge pass and the source-major pass over its edges, reduces ``da_src`` to the owners, and -- for a
+                hidden layer -- writes its ``dx`` partial over all ``n_pos`` positions (the dx GEMM) into a symmetric buffer
+                that each owner reduces over its row range (``gnnfd_peer_reduce``): 256 B per node instead of 2 KB of
+                ``dxw``.  The dx GEMM and ``dxw_part`` (2 KB per node, transient) cover every position on every rank: they do
+                not shrink with the number of ranks.
+    Every hidden layer keeps its own input buffer (the backward gathers from it), so ``num_layers - 1`` hidden buffers and
+    one dx buffer are allocated once.  ``GNNFD_EXCHANGE=nccl``, or no symmetric memory, uses NCCL all-gathers and
+    reduce-scatters instead.
+
+    Dropout: the seeds of step ``s`` and layer ``l`` are ``dropout_seeds(seed, s, l)``, the same on every rank with no
+    collective.  Feature dropout is keyed on global rows, so its masks equal the single-GPU model's.  Attention dropout is
+    keyed on the position in this rank's local ``edge_index'`` (``DstRangePlan.local_edges``: the original order, then the
+    self-loops): the masks have the single-GPU distribution, and at one rank the single-GPU bits, but not the same bits when
+    there is more than one rank.
+    """
+
+    def __init__(self, part: InputSpaceModelPartition, model, x_full: torch.Tensor, y: torch.Tensor, pos_weight: float = 50.0,
+                 lr: float = 1e-3, weight_decay: float = 5e-4, seed: int = 0):
+        from . import fused
+        from .models import TemporalGNN
+        InputSpaceModelPartition.check_model(model, training=True)
+        if not model.use_batch_norm:
+            raise NotImplementedError("InputSpaceModelTrainStep needs use_batch_norm=True: the hidden rows are broadcast by the "
+                                      "BatchNorm tail")
+        if not model.fused_tail:
+            raise NotImplementedError("InputSpaceModelTrainStep runs the fused BatchNorm tail: fused_tail=False is not supported")
+        if not 0.0 <= model.dropout <= 0.9:
+            raise NotImplementedError(f"the input-space formulation supports dropout <= 0.9, got {model.dropout}")
+        self.is_tgn = isinstance(model, TemporalGNN)
+        if self.is_tgn and not (model.fused_head and fused.gru_head_supported(model.gru, model.out)):
+            raise NotImplementedError("InputSpaceModelTrainStep runs the TemporalGNN head as fused.gru_head")
+        if (not x_full.is_cuda or x_full.dtype != torch.float32 or x_full.dim() != 2
+                or tuple(x_full.shape) != (part.n_pos, model.in_channels)):
+            raise ValueError(f"x_full must be float32 CUDA [{part.n_pos},{model.in_channels}] in padded position space, "
+                             f"got {x_full.dtype} {tuple(x_full.shape)} on {x_full.device}")
+        N = part.plan.num_nodes
+        if y.dim() != 1 or y.numel() != N or y.device != x_full.device:
+            raise ValueError(f"y must be the global labels [{N}] on {x_full.device}, got {tuple(y.shape)} on {y.device}")
+        self.part, self.model, self.x_full, self.pos_weight, self.seed = part, model, x_full, float(pos_weight), int(seed)
+        self.lo, self.hi = int(part.plan.start[part.rank]), int(part.plan.start[part.rank + 1])
+        self.y_own = y[self.lo:self.hi].long().contiguous()
+        dev, world = x_full.device, part.world
+        if world > 1:
+            state = [t for t in list(model.parameters()) + list(model.buffers()) if t.dtype == torch.float32]
+            flat = torch.cat([t.detach().reshape(-1) for t in state])
+            dist.broadcast(flat, src=0)
+            k = 0
+            with torch.no_grad():
+                for t in state:
+                    t.copy_(flat[k:k + t.numel()].view_as(t))
+                    k += t.numel()
+        n_lab = torch.tensor([float((self.y_own != -1).sum())], dtype=torch.float64, device=dev)
+        own_lab = float(n_lab.item())
+        if world > 1:
+            dist.all_reduce(n_lab)
+        self.w_lab = own_lab / max(float(n_lab.item()), 1.0)        # this rank's share of the labelled nodes
+        self.params = list(model.parameters())
+        # the BatchNorm tails' backward all-reduces its column sums: dgamma / dbeta are already the whole batch's on every rank
+        bn_params = {id(q) for bn in model.batch_norms for q in bn.parameters()}
+        self.reduced = [q for q in self.params if id(q) not in bn_params]
+        self.optimizer = torch.optim.Adam(self.params, lr=lr, weight_decay=weight_decay)
+        L = model.num_layers
+        self.px, bufs, peers, self._handles, self.exchange = part.hidden_buffers(L if L > 1 else 0)
+        self.hidden, self.dx_buf = bufs[:L - 1], (bufs[L - 1] if L > 1 else None)
+        self.hidden_peers = peers[:L - 1] if peers else None
+        self.dx_peers = peers[L - 1] if (peers and L > 1) else None
+        self.totals = torch.zeros(8, dtype=torch.float64, device=dev)
+        self.steps = 0
+
+    @staticmethod
+    def dropout_seeds(seed: int, step: int, layer: int):
+        """(attention seed, feature seed) of ``layer`` in step ``step``: host arithmetic, the same on every rank."""
+        base = _splitmix64(_splitmix64(_splitmix64(int(seed) & 0xFFFFFFFFFFFFFFFF) ^ int(step)) ^ int(layer))
+        return _splitmix64(base ^ 1) >> 2, _splitmix64(base ^ 2) >> 2
+
+    def step(self, marks=None):
+        """One optimizer step.  Returns device tensors ``(loss, stats)``: the global loss (mean over all labelled nodes) and
+        this rank's counters.  ``marks``: optional per-layer lists of 9 CUDA events -- forward: start, logits + exchange done,
+        aggregation done, output GEMM + BatchNorm + broadcast done; backward: start, edge pass done, source pass done,
+        parameter gradients (with the da_src exchange) done, dx GEMM + reduce done -- and one more list of 2 (head start,
+        optimizer done)."""
+        from . import fused
+        model, part, px = self.model, self.part, self.px
+        model.train()
+        n, P, world = part.n_local, part.rows_padded, part.world
+        lo = part.rank * P
+        group = dist.group.WORLD if world > 1 else None
+        self.optimizer.zero_grad(set_to_none=True)
+        x_own, h_full = self.x_full[lo:lo + n], self.x_full
+        L = len(model.gat_layers)
+        for i, conv in enumerate(model.gat_layers):
+            m = marks[i] if marks else None
+            s_att, s_feat = self.dropout_seeds(self.seed, self.steps, i)
+            z = _RankLayer.apply(x_own, conv.lin_src.weight, conv.att_src, conv.att_dst, conv.bias, self, h_full,
+                                 conv.negative_slope, conv.dropout, s_att, m)
+            res = x_own.contiguous() if (model.residual and x_own.size(1) == z.size(1)) else None
+            bcast = None
+            if i < L - 1 and px is not None:
+                bcast = (self.hidden_peers[i], lo, px.mode == "multicast" and self.hidden_peers[i].multicast is not None)
+            h = fused.bn_relu_dropout_residual(z, model.batch_norms[i], model.dropout, res, seed=s_feat, row_base=self.lo,
+                                               group=group, global_rows=part.plan.num_nodes, bcast=bcast)
+            if i < L - 1:
+                h_full = self.hidden[i]
+                if px is not None:
+                    px.barrier()       # every rank's rows have landed
+                else:
+                    h_full[lo:lo + n].copy_(h.detach())
+                    if world > 1:
+                        dist.all_gather_into_tensor(h_full, h_full[lo:lo + P])
+            if m: m[3].record()
+            x_own = h
+        if marks: marks[L][0].record()
+        logits = fused.gru_head(x_own, model.gru, model.out)[0] if self.is_tgn else model.out(x_own)
+        self.logits = logits.detach()       # the own rows' logits of this step (before the update)
+        loss, stats = fused.masked_bce_with_logits(logits, self.y_own, self.pos_weight)
+        (loss * self.w_lab).backward()
+        loss = loss.detach() * self.w_lab
+        if world > 1:
+            flat = torch.cat([p.grad.reshape(-1) for p in self.reduced] + [loss.reshape(1)])
+            dist.all_reduce(flat)      # also the step-end rendezvous that keeps a fast rank out of the next step's buffers
+            k = 0
+            for p in self.reduced:
+                p.grad.copy_(flat[k:k + p.numel()].view_as(p))
+                k += p.numel()
+            loss = flat[k]
+        self.optimizer.step()
+        if marks: marks[L][1].record()
+        self.totals.add_(stats)
+        self.steps += 1
+        return loss, stats
+
+    def metrics(self, reset: bool = True):
+        """As ``DeviceTrainStep.metrics``, with the counters summed over the ranks (one all-reduce, one synchronisation)."""
+        from .train_step import metrics_from_totals
+        t = self.totals.clone()
+        if self.part.world > 1:
+            dist.all_reduce(t)
+        if reset:
+            self.totals.zero_()
+        return metrics_from_totals(t.tolist())

@@ -92,13 +92,19 @@ class DeviceTrainStep:
         t = self.totals.tolist()
         if reset:
             self.totals.zero_()
-        n = max(t[1], 1.0)
-        tp, fp, tn, fn = t[2], t[3], t[4], t[5]
-        prec = tp / (tp + fp) if tp + fp else 0.0
-        rec = tp / (tp + fn) if tp + fn else 0.0
-        return {"loss": t[0] / n, "labelled": t[1], "tp": tp, "fp": fp, "tn": tn, "fn": fn, "accuracy": (tp + tn) / n,
-                "precision": prec, "recall": rec, "f1": 2 * prec * rec / (prec + rec) if prec + rec else 0.0}
+        return metrics_from_totals(t)
 
     def close(self):
         _abi.lib().gnnfd_set_dropout_seed_source(None)
         self.graph = None
+
+
+def metrics_from_totals(t) -> Dict[str, float]:
+    """The counters of ``masked_bce_with_logits`` summed over steps (``[sum of losses, labelled, TP, FP, TN, FN, ..]``) ->
+    mean loss per labelled node and the confusion-matrix metrics."""
+    n = max(t[1], 1.0)
+    tp, fp, tn, fn = t[2], t[3], t[4], t[5]
+    prec = tp / (tp + fp) if tp + fp else 0.0
+    rec = tp / (tp + fn) if tp + fn else 0.0
+    return {"loss": t[0] / n, "labelled": t[1], "tp": tp, "fp": fp, "tn": tn, "fn": fn, "accuracy": (tp + tn) / n,
+            "precision": prec, "recall": rec, "f1": 2 * prec * rec / (prec + rec) if prec + rec else 0.0}

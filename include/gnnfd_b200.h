@@ -37,7 +37,7 @@
 extern "C" {
 #endif
 
-#define GNNFD_ABI_VERSION 21
+#define GNNFD_ABI_VERSION 22
 
 typedef void* gnnfd_stream_t; /* cudaStream_t */
 
@@ -369,7 +369,10 @@ int gnnfd_bce_masked(const float* logits, const int64_t* y, int64_t N, float pos
  * addresses (its own included, ptr[rank]) plus, where the allocation has one, the NVSwitch multicast address.  The kernels
  * store / load straight through NVLink -- no staging buffer, no collective call; the caller separates a producing kernel
  * from the consuming one with a cross-GPU barrier (any: a signal-pad barrier of the symmetric allocation, a 1-element
- * all-reduce).  Host side: partition.PeerExchange (torch symmetric memory). */
+ * all-reduce).  Host side: partition.PeerExchange (torch symmetric memory).  Scoring a whole model across GPUs
+ * (partition.InputSpaceModelPartition) uses gnnfd_in_logits_bcast, gnnfd_in_out_bcast and gnnfd_peer_reduce; training it
+ * (partition.InputSpaceModelTrainStep) uses gnnfd_in_logits_bcast, gnnfd_bn_relu_drop_res_fwd_bcast (the hidden rows, finished
+ * after the batch statistics) and gnnfd_peer_reduce (da_src and the dx partials, reduced by their owners). */
 #define GNNFD_MAX_PEERS 16
 typedef struct gnnfd_peers {
     int32_t n_peers;               /* G */
@@ -393,6 +396,16 @@ int gnnfd_in_out_bcast(const void* zimg, int64_t n, int64_t K, const void* prep,
                        const float* post_scale, const float* post_shift, const float* residual,
                        const gnnfd_peers_t* h_all, int64_t row_offset, int use_multicast, float* out,
                        gnnfd_stream_t stream);
+/* gnnfd_bn_relu_drop_res_fwd (section 6) fused with the all-gather of its rows: same arithmetic and dropout key
+ * (dropout_seed, (row_base + n) * C + c), bit for bit; every finished 16-byte piece of row r (r in [0,N)) is also stored into
+ * row row_offset + r of h_all [n_pos,C] ON EVERY RANK (use_multicast: one multimem.st; else one store per peer).  out (the own
+ * rows) may be NULL.  Same refusals as gnnfd_in_out_bcast, before anything is launched.  In training the batch statistics
+ * exist only after the output GEMM, so this -- not gnnfd_in_out_bcast -- is where a hidden row is finished and broadcast;
+ * partition.InputSpaceModelTrainStep drives it. */
+int gnnfd_bn_relu_drop_res_fwd_bcast(const float* z, int64_t N, int C, const float* mean, const float* invstd,
+                                     const float* gamma, const float* beta, float p_drop, uint64_t dropout_seed,
+                                     int64_t row_base, const float* residual, const gnnfd_peers_t* h_all,
+                                     int64_t row_offset, int use_multicast, float* out, gnnfd_stream_t stream);
 /* out[i] = reduce over ranks of buf_r[offset + i], i in [0,n)  (op 0: sum, 1: max).  use_multicast (sum only, offset and n
  * multiples of 4): multimem.ld_reduce -- the addition happens inside the NVSwitch; else peer loads summed in rank order
  * (deterministic).  The reduce-scatter of the partial da_src [n_pos,H]: every rank reduces ITS OWN row range. */
